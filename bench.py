@@ -24,6 +24,8 @@ One "step" = one pass of the whole hot path over one batch of stereo pairs.
   cpu_baseline : the reference's OpenCV call sequence (cv2) on the box's host cores on a bounded
            sample of the same workload (rank 0, N=1 only).
   --impl reference : the same CPU path as its own arm.
+  --dump-outputs DIR : after the timed steps, what the timed path returned for its last step is written as DIR/<name>.npy
+           (see dump_outputs); the inputs are seeded, so two builds run with the same arguments can be compared file by file.
   --workload c5_1024_sharded : BASELINE config 5 as written -- ONE global batch of 1024 pairs of 1920x1200 / N=10000
            partitioned frame-wise with front_end_b200.shard.shard_range over the N ranks ("scaling": "strong").
 
@@ -154,6 +156,47 @@ class ClockSampler:
         reasons = [n for i, n in enumerate(names) if any(r[4 + i].lower().startswith("active") for r in rows)]
         return {"sm_mhz": sm[len(sm) // 2], "sm_max_mhz": float(rows[0][2]), "reasons": reasons, "samples": len(rows),
                 "power_w_max": max(float(r[3]) for r in rows)}
+
+
+DUMP_BUDGET = 64_000_000       # bytes of --dump-outputs files
+
+
+def dump_outputs(path, res, cap, tracks=None, seed=0):
+    """Writes the batch results of one step (FrontEnd.batch_download's dict; `tracks` = window_batch's (tracks, n_tracks) for
+    the window workload) as float32 / float64 .npy files under `path`, at most DUMP_BUDGET bytes in all.  The counts of every
+    pair are written in full; keypoints, descriptors and match lists for a sample of pairs fixed by `seed` and the batch shape,
+    as many as the budget holds.  Each image's / pair's list is zero-padded to `cap` rows, so the file shapes do not depend on
+    the results.  Returns {name: array}."""
+    n_kps = np.minimum(res["n_kps"], cap)
+    P = len(res["n_a"])
+    dw = res["desc"].shape[-1]
+    per_pair = 2 * cap * (7 + dw) * 4 + 2 * cap * 4 * 8 + (cap * 4 * 8 if tracks is not None else 0)
+    pool = P - 1 if tracks is not None else P            # window tracks exist for the P - 1 consecutive frame pairs
+    fixed = (4 * P + 2 * pool) * 8 + 16 * 1024            # counts, pair indices, .npy headers
+    S = int(min(pool, max(DUMP_BUDGET - fixed, 0) // per_pair))
+    pairs = np.sort(np.random.default_rng(seed).choice(pool, S, replace=False))
+    imgs = np.stack([2 * pairs, 2 * pairs + 1], 1).reshape(-1)
+    rows = np.arange(cap)
+
+    def records(a, n, dtype):        # structured (..., cap) slab -> (..., cap, fields), rows past each count zeroed
+        v = np.stack([a[k].astype(dtype) for k in a.dtype.names], -1)
+        return np.where((rows[None, :] < n[:, None])[..., None], v, 0).astype(dtype)
+
+    out = {"n_kps": res["n_kps"].astype(np.float64), "n_a": res["n_a"].astype(np.float64),
+           "n_b": res["n_b"].astype(np.float64), "pairs": pairs.astype(np.float64),
+           "kps": records(res["kps"][imgs, :cap], n_kps[imgs], np.float32).reshape(S, 2, cap, 7),
+           "desc": np.where((rows[None, :] < n_kps[imgs][:, None])[..., None], res["desc"][imgs, :cap], 0)
+                     .astype(np.float32).reshape(S, 2, cap, dw)}
+    for k, n in (("matches_a", "n_a"), ("matches_b", "n_b")):
+        out[k] = records(res[k][pairs, :cap], np.minimum(res[n][pairs], cap), np.float64)
+    if tracks is not None:
+        t, nt = tracks
+        out["n_tracks"] = nt[:pool].astype(np.float64)
+        out["tracks"] = records(t[pairs, :cap], np.minimum(nt[pairs], cap), np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+    return out
 
 
 # ---- CPU arm: the reference's OpenCV call sequence ----------------------------------------------------------
@@ -306,7 +349,10 @@ def main():
     ap.add_argument("--cpu-pairs", type=int, default=0, help="pairs in the bounded CPU-baseline sample")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--e2e-workers", type=int, default=3, help="host threads (one fe_ctx each) issuing the e2e steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computes; the reference arm keeps only counts")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -442,6 +488,8 @@ def main():
     res = f.batch_download(out)
     n_kps = res["n_kps"].copy()
     n_a, n_b = res["n_a"].copy(), res["n_b"].copy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, cap, wout)
 
     # ---- cross-rank verification: one probe batch every rank runs, digests all-gathered over NCCL ------------------
     results_agree = None

@@ -45,6 +45,51 @@ def test_reference_arm_other_ranks_print_nothing():
     assert p.returncode == 0 and p.stdout.strip() == ""
 
 
+def test_dump_outputs_is_bounded_padded_and_repeatable(tmp_path):
+    """--dump-outputs: float files only, within the budget at the largest batch shape, rows past each count zeroed, the counts
+    and the sampled pairs' lists equal to what the batch held, the same files from the same results."""
+    import numpy as np
+    import bench
+    from front_end_b200 import KPOINT, MATCH
+    P, cap = 96, 8192
+    rng = np.random.default_rng(3)
+    res = dict(kps=np.zeros((2 * P, cap), KPOINT), desc=rng.integers(0, 256, (2 * P, cap, 32), dtype=np.uint8),
+               n_kps=rng.integers(0, cap + 100, 2 * P).astype(np.int32), matches_a=np.zeros((P, cap), MATCH),
+               n_a=rng.integers(0, cap, P).astype(np.int32), matches_b=np.zeros((P, cap), MATCH), n_b=rng.integers(0, cap, P).astype(np.int32))
+    for k in KPOINT.names:
+        res["kps"][k] = rng.integers(-1, 2000, (2 * P, cap))
+    for k in ("matches_a", "matches_b"):
+        for f in MATCH.names:
+            res[k][f] = rng.integers(0, cap, (P, cap))
+    tracks = (np.zeros((P, cap), MATCH), rng.integers(0, cap, P).astype(np.int32))
+    tracks[0]["trainIdx"] = rng.integers(0, cap, (P, cap))
+    a = bench.dump_outputs(str(tmp_path / "a"), res, cap, tracks)
+    b = bench.dump_outputs(str(tmp_path / "b"), res, cap, tracks)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(k + ".npy" for k in a) and sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64_000_000
+    for f in files:
+        x = np.load(tmp_path / "a" / f)
+        assert x.dtype in (np.float32, np.float64) and np.array_equal(x, np.load(tmp_path / "b" / f)), f
+    pairs = a["pairs"].astype(int)
+    assert len(pairs) >= 8 and len(set(pairs)) == len(pairs) and pairs.max() < P - 1
+    assert np.array_equal(a["n_kps"], res["n_kps"]) and np.array_equal(a["n_b"], res["n_b"])
+    for s, p in enumerate(pairs):
+        for e in range(2):
+            m = min(int(res["n_kps"][2 * p + e]), cap)
+            assert np.array_equal(a["desc"][s, e, :m], res["desc"][2 * p + e, :m]) and not a["desc"][s, e, m:].any()
+            assert np.array_equal(a["kps"][s, e, :m, 5], res["kps"]["octave"][2 * p + e, :m]) and not a["kps"][s, e, m:].any()
+        m = int(res["n_a"][p])
+        assert np.array_equal(a["matches_a"][s, :m, 1], res["matches_a"]["trainIdx"][p, :m]) and not a["matches_a"][s, m:].any()
+        m = int(tracks[1][p])
+        assert np.array_equal(a["tracks"][s, :m, 1], tracks[0]["trainIdx"][p, :m]) and not a["tracks"][s, m:].any()
+
+
+def test_dump_outputs_needs_the_gpu_arm():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", "x"],
+                       capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert p.returncode == 2 and "--dump-outputs" in p.stderr
+
+
 def test_reference_arm_surf_workload_is_bounded_and_says_what_it_scaled():
     """BASELINE config 3 on the CPU: the numpy SURF restatement is timed on a keypoint sample and scaled (a full pair would take
     ~25 s); the line says so."""

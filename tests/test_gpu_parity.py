@@ -1355,10 +1355,12 @@ def test_orb_parameter_table_vs_cv2_golden(FE, tag):
 @pytest.mark.gpu
 def test_bench_gpu_arm_line_has_the_contract_keys(tmp_path):
     """bench.py's own arm on a small batch: ONE JSON line carrying the contract's keys (metric / value / e2e with real copy
-    bytes / roofline / clocks / gpu_launches) and, with FE_BENCH_PHASED=1, both copy schedules."""
+    bytes / roofline / clocks / gpu_launches) and, with FE_BENCH_PHASED=1, both copy schedules.  --dump-outputs writes the
+    last timed step's results as float arrays that agree with the line's counts."""
     import json, os, subprocess, sys
     env = dict(os.environ, FE_BENCH_PHASED="1")
-    p = subprocess.run([sys.executable, os.path.join(ROOT_DIR, "bench.py"), "--steps", "2", "--warmup", "3", "--pairs", "8", "--no-cpu"],
+    p = subprocess.run([sys.executable, os.path.join(ROOT_DIR, "bench.py"), "--steps", "2", "--warmup", "3", "--pairs", "8", "--no-cpu",
+                        "--dump-outputs", str(tmp_path / "dump")],
                        capture_output=True, text=True, timeout=900, cwd=ROOT_DIR, env=env)
     assert p.returncode == 0, p.stderr[-2000:]
     lines = [l for l in p.stdout.strip().splitlines() if l.strip()]
@@ -1376,3 +1378,11 @@ def test_bench_gpu_arm_line_has_the_contract_keys(tmp_path):
     assert r["bound"] in ("hbm", "tensor") and r["unit"] in ("GB/s", "TFLOP/s") and abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-9
     assert set(d["e2e_schedules"]) == {"overlapped", "phased"} and e["schedule"] in ("overlapped", "phased")
     assert d["clocks"]["sm_mhz"] > 0 and isinstance(d["clocks"]["reasons"], list)
+    dump = {f[:-4]: np.load(tmp_path / "dump" / f) for f in os.listdir(tmp_path / "dump")}
+    assert all(v.dtype in (np.float32, np.float64) for v in dump.values())
+    assert dump["n_kps"].mean() == d["counts"]["keypoints_per_image_mean"] and dump["n_a"].mean() == d["counts"]["ratio_matches_per_pair_mean"]
+    assert dump["n_b"].mean() == d["counts"]["crosscheck_matches_per_pair_mean"] and dump["pairs"].tolist() == list(range(8))
+    for e in range(16):
+        m = int(dump["n_kps"][e])
+        k = dump["kps"][e // 2, e % 2]
+        assert m > 1000 and np.all((k[:m, 0] > 0) & (k[:m, 0] < 1280) & (k[:m, 1] > 0) & (k[:m, 1] < 720)) and not k[m:].any()

@@ -1,16 +1,84 @@
-"""Pin the numpy oracle against (a) the committed cv2-generated golden vectors and (b) cv2 itself
-when importable.  CPU only.  Bar: bit-exact keypoints / responses / angles / descriptor bits /
-match indices and distances."""
+"""Pin the numpy oracle against (a) the committed cv2-generated golden vectors and (b) cv2's answers on
+fresh inputs that this module builds (stored in golden/cv2_pins.npz by golden/make_golden_cv2_pins.py,
+which calls the builders below).  CPU only.  Bar: bit-exact keypoints / responses / angles / descriptor
+bits / match indices and distances."""
 import numpy as np
 import pytest
 
 from conftest import golden
 from oracle import fast, match, orb, synth
 
-try:
-    import cv2
-except Exception:  # pragma: no cover
-    cv2 = None
+CV2_PINS = "cv2_pins"
+
+
+def fresh_seed_pair():
+    return synth.stereo_pair(300, 420, 12345)
+
+
+def surf_primitive_inputs():
+    """An image, square windows SURF resizes to 21 x 21 and (y, x) for fastAtan2."""
+    rng = np.random.default_rng(0)
+    img = rng.integers(0, 256, (60, 80), dtype=np.uint8)
+    windows = []
+    # 19: FAST keypoints (size 7); 86: ORB keypoints (size 31); multiples of 21 take OpenCV's integer-decimation path
+    # (ResizeAreaFast; 42 = every size-15 Fast-Hessian keypoint, 126 = size 45); the rest the general area table
+    for S in (19, 86, 33, 24, 21, 20, 12, 57, 42, 63, 84, 105, 126, 147, 168, 189, 210, 231, 252, 43, 41, 125, 127):
+        for rep in range(6):
+            w = rng.integers(0, 256, (S, S), dtype=np.uint8)
+            if rep & 1:     # few grey levels: many box sums land exactly on a rounding tie
+                w = (w // 64 * 64 + rng.integers(0, 3, (S, S))).astype(np.uint8)
+            windows.append(w)
+    y = rng.standard_normal(2000).astype(np.float32) * 50
+    x = rng.standard_normal(2000).astype(np.float32) * 50
+    return img, windows, y, x
+
+
+def subpix_inputs(img):
+    """A small border-heavy crop, points for cornerSubPix and centres for getRectSubPix (13 x 13, partly outside)."""
+    rng = np.random.default_rng(11)
+    small = np.ascontiguousarray(img[40:100, 60:130])
+    pts = np.stack([rng.uniform(0, 69.99, 60), rng.uniform(0, 59.99, 60)], 1).astype(np.float32)
+    centres = [(float(np.float32(rng.uniform(-8, 78))), float(np.float32(rng.uniform(-8, 68)))) for _ in range(40)]
+    return small, pts, centres
+
+
+def harris_fresh_image():
+    return synth.stereo_pair(200, 260, 77)[1]
+
+
+def resize_inputs():
+    rng = np.random.default_rng(0)
+    out = []
+    for (h, w) in ((240, 320), (123, 457), (37, 41)):
+        img = rng.integers(0, 256, (h, w), dtype=np.uint8)
+        out.append((img, int(np.rint(w / 1.2)), int(np.rint(h / 1.2))))
+    return out
+
+
+def wide_row_inputs():
+    """64-byte rows clustered around 40 prototypes with planted exact duplicates, ragged counts, and the masks (epipolar band,
+    window box, none) they are matched under."""
+    rng = np.random.default_rng(11)
+    base = rng.integers(0, 256, (40, 64), dtype=np.uint8)
+    def rows(n):
+        d = base[rng.integers(0, 40, n)].copy()                       # clusters: near-duplicates of 40 prototypes
+        flips = rng.integers(0, 512, (n, 24))
+        for i in range(n):
+            for b in flips[i, :rng.integers(0, 24)]:
+                d[i, b >> 3] ^= 1 << (b & 7)
+        return d
+    ql, tr = rows(301), rows(277)
+    tr[5], tr[9], tr[100] = tr[200], tr[200], ql[17]                  # exact duplicates and an exact hit
+    qx, qy = rng.uniform(0, 320, 301).astype(np.float32), np.sort(rng.integers(0, 240, 301)).astype(np.float32)
+    tx, ty = rng.uniform(0, 320, 277).astype(np.float32), np.sort(rng.integers(0, 240, 277)).astype(np.float32)
+    return ql, tr, (match.epipolar_mask(qy, ty, 2.0), match.window_mask(qx, qy, tx, ty, 100, 60), None)
+
+
+def _assert_knn(g, p, idx, dd, cnt):
+    """The oracle's knn2 against cv2's knnMatch rows, stored as per-row counts and the first `count` train indices / distances."""
+    assert np.array_equal(cnt, g[p + "_knn_cnt"])
+    valid = np.arange(2)[None, :] < cnt[:, None]
+    assert np.array_equal(idx[valid], g[p + "_knn_idx"][valid]) and np.array_equal(dd[valid], g[p + "_knn_dist"][valid])
 
 
 @pytest.mark.parametrize("ps", [16, 12, 8])
@@ -101,59 +169,38 @@ def test_setpoint_controller():
     assert thr.tolist() == [[6, 10, 10], [6, 10, 10]]
 
 
-@pytest.mark.skipif(cv2 is None, reason="cv2 not importable")
 def test_live_cv2_pin_fresh_seed():
-    """The reference's call sequence through cv2 on a seed that is not in the fixtures."""
-    L, R = synth.stereo_pair(300, 420, 12345)
-    o = cv2.ORB_create(nfeatures=800, scaleFactor=1.2, nlevels=1, edgeThreshold=31, firstLevel=0, WTA_K=2,
-                       scoreType=cv2.ORB_FAST_SCORE, patchSize=31, fastThreshold=15)
+    """The reference's call sequence through cv2 (ORB detectAndCompute, masked knnMatch, crossCheck match) on a seed that is
+    not in the other fixtures."""
+    g = golden(CV2_PINS)
     out = []
-    for img in (L, R):
-        kps, desc = o.detectAndCompute(img, None)
-        x = np.array([k.pt[0] for k in kps], np.float32)
-        y = np.array([k.pt[1] for k in kps], np.float32)
-        a = np.array([k.angle for k in kps], np.float32)
-        order = np.lexsort((x, y))
+    for eye, img in zip("lr", fresh_seed_pair()):
         r = orb.orb_detect_and_compute(img, 800, 15)
-        assert np.array_equal(r["x"], x[order]) and np.array_equal(r["y"], y[order])
-        assert np.array_equal(r["angle"], a[order]) and np.array_equal(r["desc"], desc[order])
+        p = "fresh_%s_" % eye
+        assert np.array_equal(r["x"], g[p + "x"]) and np.array_equal(r["y"], g[p + "y"])
+        assert np.array_equal(r["angle"], g[p + "angle"]) and np.array_equal(r["desc"], g[p + "desc"])
         out.append(r)
     l, r = out
     D = match.hamming_matrix(l["desc"], r["desc"])
-    mask = match.epipolar_mask(l["y"], r["y"], 2.0)
-    res = cv2.BFMatcher(cv2.NORM_HAMMING, False).knnMatch(l["desc"], r["desc"], 2, mask.astype(np.uint8))
-    idx, dd, cnt = match.knn2(D, mask)
-    for i, row in enumerate(res):
-        assert len(row) == cnt[i]
-        for j, m in enumerate(row):
-            assert m.trainIdx == idx[i, j] and m.distance == dd[i, j]
-    mc = cv2.BFMatcher(cv2.NORM_HAMMING, True).match(l["desc"], r["desc"])
+    _assert_knn(g, "fresh", *match.knn2(D, match.epipolar_mask(l["y"], r["y"], 2.0)))
     q, t, d = match.cross_check(D)
-    assert [m.queryIdx for m in mc] == q.tolist() and [m.trainIdx for m in mc] == t.tolist()
+    assert np.array_equal(q, g["fresh_cc_q"]) and np.array_equal(t, g["fresh_cc_t"]) and np.array_equal(d, g["fresh_cc_d"])
 
 
-@pytest.mark.skipif(cv2 is None, reason="cv2 not importable")
 def test_surf_primitives_pinned_against_cv2():
     """No SURF binary exists here; pin every primitive src/surf.cpp delegates to OpenCV."""
     from oracle import surf
-    rng = np.random.default_rng(0)
-    img = rng.integers(0, 256, (60, 80), dtype=np.uint8)
-    assert np.array_equal(surf.integral_i32(img), cv2.integral(img, sdepth=cv2.CV_32S))
-    assert np.allclose(surf.G_ORI, cv2.getGaussianKernel(13, 2.5, cv2.CV_32F).ravel(), rtol=2e-7, atol=0)
+    g = golden(CV2_PINS)
+    img, windows, y, x = surf_primitive_inputs()
+    assert np.array_equal(surf.integral_i32(img), g["surf_integral"])
+    assert np.allclose(surf.G_ORI, g["surf_gauss13"], rtol=2e-7, atol=0)
     # the reference's own CUDA tables (src/cuda/surf.cu:537,699-721) for the two Gaussians
     assert abs(float(surf.G_ORI[6]) ** 2 - 0.02592208795249462) < 1e-8
     assert abs(float(surf.DW[9, 9]) - 0.01435048412531614) < 1e-8 and abs(float(surf.DW[0, 0]) - 3.695352233989979e-06) < 1e-11
-    # 19: FAST keypoints (size 7); 86: ORB keypoints (size 31); multiples of 21 take OpenCV's integer-decimation path
-    # (ResizeAreaFast; 42 = every size-15 Fast-Hessian keypoint, 126 = size 45); the rest the general area table
-    for S in (19, 86, 33, 24, 21, 20, 12, 57, 42, 63, 84, 105, 126, 147, 168, 189, 210, 231, 252, 43, 41, 125, 127):
-        for rep in range(6):
-            w = rng.integers(0, 256, (S, S), dtype=np.uint8)
-            if rep & 1:     # few grey levels: many box sums land exactly on a rounding tie
-                w = (w // 64 * 64 + rng.integers(0, 3, (S, S))).astype(np.uint8)
-            assert np.array_equal(surf.resize_area_21(w), cv2.resize(w, (21, 21), interpolation=cv2.INTER_AREA)), S
-    y = rng.standard_normal(2000).astype(np.float32) * 50
-    x = rng.standard_normal(2000).astype(np.float32) * 50
-    assert np.array_equal(orb.fast_atan2_deg(y, x), np.array([cv2.fastAtan2(float(a), float(b)) for a, b in zip(y, x)], np.float32))
+    assert len(windows) == len(g["surf_resize21"])
+    for w, want in zip(windows, g["surf_resize21"]):
+        assert np.array_equal(surf.resize_area_21(w), want), w.shape[0]
+    assert np.array_equal(orb.fast_atan2_deg(y, x), g["surf_atan2"])
 
 
 def test_surf_oracle_properties():
@@ -176,24 +223,19 @@ def test_surf_oracle_properties():
 
 def test_cornersubpix_pinned_against_cv2():
     """oracle/subpix.py restates cv::cornerSubPix + getRectSubPix; pinned bit-for-bit on the committed cv2 fixture
-    (400 points incl. every border) and, when cv2 is importable, on fresh points of a small image (border-heavy)."""
+    (400 points incl. every border) and on cv2's answers for fresh points of a small image (border-heavy)."""
     from oracle import subpix
     g = golden("grid_subpix_480x360")
     img = g["img_f0_l"]
     sel = np.r_[0:160:4, 160:400:12]
     got = subpix.corner_subpix(img, g["subpix_in"][sel])
     assert np.array_equal(got, g["subpix_out"][sel])
-    if cv2 is not None:
-        rng = np.random.default_rng(11)
-        small = np.ascontiguousarray(img[40:100, 60:130])
-        pts = np.stack([rng.uniform(0, 69.99, 60), rng.uniform(0, 59.99, 60)], 1).astype(np.float32)
-        want = cv2.cornerSubPix(small, pts.copy().reshape(-1, 1, 2), (5, 5), (-1, -1),
-                                (cv2.TERM_CRITERIA_EPS | cv2.TERM_CRITERIA_COUNT, 40, 0.001)).reshape(-1, 2)
-        assert np.array_equal(subpix.corner_subpix(small, pts), want)
-        for k in range(40):
-            c = (float(np.float32(rng.uniform(-8, 78))), float(np.float32(rng.uniform(-8, 68))))
-            assert np.array_equal(subpix.rect_subpix_8u32f(small, 13, 13, c[0], c[1]),
-                                  cv2.getRectSubPix(small, (13, 13), c, patchType=cv2.CV_32F))
+    c2 = golden(CV2_PINS)
+    small, pts, centres = subpix_inputs(img)
+    assert np.array_equal(subpix.corner_subpix(small, pts), c2["subpix_small_out"])
+    assert len(centres) == len(c2["subpix_rect"])
+    for c, want in zip(centres, c2["subpix_rect"]):
+        assert np.array_equal(subpix.rect_subpix_8u32f(small, 13, 13, c[0], c[1]), want)
 
 
 @pytest.mark.parametrize("variant", ["cpp", "py"])
@@ -257,23 +299,17 @@ def test_orb_harris_score_golden(tag):
         keys = ("x", "y", "octave", "size", "angle", "response", "desc")
     for k in keys:
         assert np.array_equal(np.asarray(r[k]).astype(g["%s_l_%s" % (tag, k)].dtype), g["%s_l_%s" % (tag, k)]), k
-    if cv2 is not None and tag == "a":
-        img2 = synth.stereo_pair(200, 260, 77)[1]
-        o = cv2.ORB_create(nfeatures=150, nlevels=1, scoreType=cv2.ORB_HARRIS_SCORE, fastThreshold=12)
-        kps = o.detect(img2, None)
-        r2 = orb.orb_detect_and_compute(img2, 150, 12, harris=True)
+    if tag == "a":
+        c2 = golden(CV2_PINS)
+        r2 = orb.orb_detect_and_compute(harris_fresh_image(), 150, 12, harris=True)
         got = {(int(x), int(y)): v for x, y, v in zip(r2["x"], r2["y"], r2["response"])}
-        assert got == {(int(k.pt[0]), int(k.pt[1])): np.float32(k.response) for k in kps}
+        assert got == {(int(x), int(y)): v for x, y, v in zip(c2["harris_x"], c2["harris_y"], c2["harris_response"])}
 
 
 def test_resize_linear_exact_pinned():
-    if cv2 is None:
-        pytest.skip("cv2 not importable")
-    rng = np.random.default_rng(0)
-    for (h, w) in ((240, 320), (123, 457), (37, 41)):
-        img = rng.integers(0, 256, (h, w), dtype=np.uint8)
-        dw, dh = int(np.rint(w / 1.2)), int(np.rint(h / 1.2))
-        assert np.array_equal(orb.resize_linear_exact(img, dw, dh), cv2.resize(img, (dw, dh), interpolation=cv2.INTER_LINEAR_EXACT))
+    g = golden(CV2_PINS)
+    for i, (img, dw, dh) in enumerate(resize_inputs()):
+        assert np.array_equal(orb.resize_linear_exact(img, dw, dh), g["resize_linear_exact_%d" % i])
 
 
 @pytest.mark.parametrize("k", [3, 4])
@@ -392,35 +428,18 @@ def test_freak_oracle_pattern_and_direct_means():
     assert abs(float(a[0]) - 90.0) < 15.0
 
 
-@pytest.mark.skipif(cv2 is None, reason="cv2 not importable")
 def test_wide_row_matcher_pinned_against_cv2():
     """64-byte rows (BRIEF-64, FREAK): the oracle's BFMatcher restatement -- what the 512-bit GPU kernels are compared with --
     against cv2.BFMatcher(NORM_HAMMING) itself: masked kNN-2 (epipolar band and window box), the unmasked kNN-2 and crossCheck,
     on clustered rows with planted exact duplicates (first minimum wins) and ragged counts."""
-    rng = np.random.default_rng(11)
-    base = rng.integers(0, 256, (40, 64), dtype=np.uint8)
-    def rows(n):
-        d = base[rng.integers(0, 40, n)].copy()                       # clusters: near-duplicates of 40 prototypes
-        flips = rng.integers(0, 512, (n, 24))
-        for i in range(n):
-            for b in flips[i, :rng.integers(0, 24)]:
-                d[i, b >> 3] ^= 1 << (b & 7)
-        return d
-    ql, tr = rows(301), rows(277)
-    tr[5], tr[9], tr[100] = tr[200], tr[200], ql[17]                  # exact duplicates and an exact hit
-    qx, qy = rng.uniform(0, 320, 301).astype(np.float32), np.sort(rng.integers(0, 240, 301)).astype(np.float32)
-    tx, ty = rng.uniform(0, 320, 277).astype(np.float32), np.sort(rng.integers(0, 240, 277)).astype(np.float32)
+    g = golden(CV2_PINS)
+    ql, tr, masks = wide_row_inputs()
     D = match.hamming_matrix(ql, tr)
     assert D.max() <= 512 and D[17, 100] == 0
-    for mask in (match.epipolar_mask(qy, ty, 2.0), match.window_mask(qx, qy, tx, ty, 100, 60), None):
-        res = cv2.BFMatcher(cv2.NORM_HAMMING, False).knnMatch(ql, tr, 2, None if mask is None else mask.astype(np.uint8))
+    for i, mask in enumerate(masks):
         idx, dd, cnt = match.knn2(D, mask)
-        assert len(res) == len(ql)
-        for i, row in enumerate(res):
-            assert len(row) == cnt[i]
-            for j, m in enumerate(row):
-                assert m.trainIdx == idx[i, j] and m.distance == dd[i, j]
-    mc = cv2.BFMatcher(cv2.NORM_HAMMING, True).match(ql, tr)
+        assert len(cnt) == len(ql)
+        _assert_knn(g, "wide%d" % i, idx, dd, cnt)
     q, t, d = match.cross_check(D)
-    assert len(mc) > 20 and [m.queryIdx for m in mc] == q.tolist() and [m.trainIdx for m in mc] == t.tolist()
-    assert [m.distance for m in mc] == d.tolist()
+    assert len(g["wide_cc_q"]) > 20 and np.array_equal(q, g["wide_cc_q"]) and np.array_equal(t, g["wide_cc_t"])
+    assert np.array_equal(d, g["wide_cc_d"])

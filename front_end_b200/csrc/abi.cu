@@ -229,6 +229,13 @@ int run_detect_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, b
     { StageTimer t(c, ST_FAST, st, timed); t.done(launch_fast(g, p, b, st)); }
     { StageTimer t(c, ST_SELECT, st, timed); t.done(launch_select(g, p, b, st)); }
     if (harris) { StageTimer t(c, ST_SELECT, st, timed); t.done(launch_harris_select(g, n_final, b, st)); }
+    // default ORB geometry: orientation and rBRIEF in one pass over image tiles, after the blur (which needs no keypoints)
+    if (describe && c->cfg.orientation && c->patch_size == 31 && c->cfg.edge_threshold >= 19 && c->wta_k == 2 && !harris) {
+        { StageTimer t(c, ST_BLUR, st, timed); t.done(launch_blur(g, b, st)); }
+        { StageTimer t(c, ST_BRIEF, st, timed); t.done(launch_describe_tile(g, p, b, (float)c->patch_size, st)); }
+        FE_CUDA(c, cudaGetLastError());
+        return FE_OK;
+    }
     { StageTimer t(c, ST_ORIENT, st, timed);
       t.done(launch_orient_pack(g, p, b, c->cfg.orientation != 0, c->cfg.orientation ? (float)c->patch_size : 7.f, general_half(c), st)); }
     if (harris) { StageTimer t(c, ST_ORIENT, st, timed); t.done(launch_harris_store(g, b, st)); }

@@ -193,6 +193,9 @@ int launch_select(const Geom &g, const DetectParams &p, const Buffers &b, cudaSt
 int launch_orient_pack(const Geom &g, const DetectParams &p, const Buffers &b, bool orientation,
                        float kp_size, int half_patch, cudaStream_t s);
 int launch_blur(const Geom &g, const Buffers &b, cudaStream_t s);
+// orientation + wire keypoints + rBRIEF-256 of the default ORB geometry (31-px patch, edgeThreshold >= 19, WTA_K 2, FAST score)
+// per image tile, from b.img and b.blur: writes what launch_orient_pack and launch_brief write
+int launch_describe_tile(const Geom &g, const DetectParams &p, const Buffers &b, float kp_size, cudaStream_t s);
 // cv::ORB HARRIS_SCORE (harris.cu): score the selected FAST corners, keep the n_features best (ties kept, raster order);
 // then, after the keypoints are packed, store the score as their response
 int launch_harris_select(const Geom &g, int n_features, const Buffers &b, cudaStream_t s);

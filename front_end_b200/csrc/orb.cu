@@ -562,6 +562,257 @@ rbrief_kernel(const uint8_t *__restrict__ blur, Geom g, const uint32_t *__restri
     }
 }
 
+// ---- orientation + rBRIEF per image tile ---------------------------------------------------------------------------------
+// Detect-and-describe of the default geometry (31-px patch, edgeThreshold >= 19, WTA_K 2, FAST score, one level): one CTA
+// per (image, DT_ROWS x DT_COLS tile of keypoint centres).  The CTA stages the raw and the blurred tile with a 19-px halo in
+// shared memory once and describes every keypoint of the tile from there.  orient_pack_kernel + rbrief_kernel instead re-read
+// each keypoint's neighbourhood from global memory: at ~5 200 keypoints per 1280 x 720 image that is ~15x the image, the
+// tiles stage ~2x it (halo included).  Keypoints are in raster order (kp_key ascending y << 16 | x per image), so those of the
+// tile's rows are one index range, found by binary search.  Moments, angle, (cos, sin) and the 256 tests are computed by the
+// same arithmetic as orient_pack_kernel and rbrief_kernel: the outputs are bit-identical.
+constexpr int DT_ROWS = 64, DT_COLS = 256;          // 64 x 128 and 32 x 256 tiles measured slower (more CTAs and halo)
+constexpr int DT_TROWS = DT_ROWS + 2 * BR_R;                // staged rows y0 - 19 .. y0 + DT_ROWS + 18
+// staged columns x0 - 32 .. x0 + DT_COLS + 31: 16-byte aligned (x0 is), they cover the reach -19 .. +20 of a keypoint (the
+// orientation's 9th word ends at x + 20; those bytes weigh 0 but are read)
+constexpr int DT_XL = 32;
+constexpr int DT_VECS = (DT_COLS + 2 * DT_XL) / 16;         // 16-byte vectors per staged row
+// raw-tile row pitch in words: 105 == 9 mod 32, so the 32 consecutive (row, word) slots of a 31 x 9-word patch read by a warp
+// fall on 32 distinct banks; blurred-tile row pitch 336 bytes: 16-byte rows, and 84 words == -12 mod 32 spreads the rotated
+// samples over the banks as rbrief_kernel's 12-word patch rows do
+constexpr int DT_RAW_W = 105;
+constexpr int DT_BLUR_B = 336;
+constexpr int DT_WARPS = 8, DT_THREADS = DT_WARPS * 32;
+constexpr int DT_CHUNK = 2 * DT_THREADS;                               // indices of the tile's row band examined per pass
+constexpr int DT_STAGE = (2 * DT_TROWS * DT_VECS + DT_THREADS - 1) / DT_THREADS;   // 16-byte loads per thread
+constexpr int DT_SMEM = DT_TROWS * DT_BLUR_B + DT_TROWS * DT_RAW_W * 4;             // dynamic: the two tiles
+static_assert(DT_COLS % 16 == 0 && DT_XL % 16 == 0 && DT_XL >= BR_R, "staged columns must start 16-byte aligned");
+static_assert(DT_VECS * 16 <= DT_BLUR_B && DT_VECS * 4 <= DT_RAW_W && DT_BLUR_B % 16 == 0, "staged row fits the tile row");
+static_assert(DT_COLS + 2 * DT_XL - DT_XL >= DT_COLS + 21, "right halo reaches x + 20");
+static_assert(DT_RAW_W % 32 == 9 && (DT_BLUR_B / 4) % 32 == 20, "bank spread of the tile rows");
+
+// orient_pack_kernel's dp4a weight tables (u, membership mask) for the 4 alignments, built at compile time: read through L1 by
+// every CTA instead of rebuilt in shared memory
+struct OriTables { uint32_t u[4][288], m[4][288]; };
+constexpr OriTables make_ori_tables() {
+    constexpr int umax[16] = {15, 15, 15, 15, 14, 14, 14, 13, 13, 12, 11, 10, 9, 8, 6, 3};
+    OriTables t{};
+    for (int off = 0; off < 4; ++off)
+        for (int slot = 0; slot < ORI_SLOTS; ++slot) {
+            const int r = slot / ORI_WORDS, w = slot - r * ORI_WORDS;
+            const int v = r - 15, d = umax[v < 0 ? -v : v];
+            for (int b = 0; b < 4; ++b) {
+                const int u = 4 * w + b - off - 15;
+                if (u >= -d && u <= d) { t.u[off][slot] |= (uint32_t)(u & 0xFF) << (8 * b); t.m[off][slot] |= 1u << (8 * b); }
+            }
+        }
+    return t;
+}
+__device__ const OriTables d_ori_tab = make_ori_tables();
+
+// first index in [0, n) whose key is >= target (n if none): 32-way search, one key per lane per round
+__device__ __forceinline__ int warp_lower_bound(const uint32_t *__restrict__ keys, int n, uint32_t target, int lane) {
+    int lo = 0, hi = n;
+    while (lo < hi) {
+        const int step = (hi - lo + 31) >> 5, i = lo + lane * step;
+        const uint32_t m = __ballot_sync(0xffffffffu, i >= hi || keys[i] >= target);
+        const int f = m ? __ffs(m) - 1 : 32;          // keys[lo + (f - 1) step] < target <= keys[lo + f step]
+        if (f == 0) break;
+        hi = min(lo + f * step, hi);
+        lo += (f - 1) * step + 1;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(DT_THREADS, 2)
+orb_describe_tile_kernel(const uint8_t *__restrict__ img, const uint8_t *__restrict__ blur, Geom g,
+                         const uint32_t *__restrict__ n_kp, const uint32_t *__restrict__ kp_key,
+                         const uint8_t *__restrict__ kp_score, int report_score, float kp_size, fe_kpoint *__restrict__ kp,
+                         float *__restrict__ kx, float *__restrict__ ky, float2 *__restrict__ kcs, uint8_t *__restrict__ desc) {
+    extern __shared__ __align__(16) uint8_t s_blur[];                                // [DT_TROWS][DT_BLUR_B]
+    uint32_t *s_raw = reinterpret_cast<uint32_t *>(s_blur + DT_TROWS * DT_BLUR_B);   // [DT_TROWS][DT_RAW_W]
+    __shared__ uint32_t s_idx[DT_CHUNK], s_key[DT_CHUNK];
+    __shared__ int s_range[2], s_cnt;
+    const uint32_t FULL = 0xffffffffu;
+    const int image = blockIdx.z;
+    const int x0 = blockIdx.x * DT_COLS, y0 = blockIdx.y * DT_ROWS;
+    const int ty0 = y0 - BR_R, sx = x0 - DT_XL;                 // image coordinates of tile row 0 / tile byte 0
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    // both tiles, clipped to the image rows and the row pitch (what lies outside is never sampled: keypoints are >= 19 px
+    // inside the image).  The loads are issued first: their latency overlaps the keypoint search.
+    uint4 v[DT_STAGE];
+#pragma unroll
+    for (int k = 0; k < DT_STAGE; ++k) {
+        const int i = threadIdx.x + k * DT_THREADS;
+        const int t = i >= DT_TROWS * DT_VECS;                      // 0: blurred tile, 1: raw tile
+        const int j = i - t * DT_TROWS * DT_VECS, r = j / DT_VECS, c = sx + 16 * (j - r * DT_VECS), gy = ty0 + r;
+        v[k] = make_uint4(0u, 0u, 0u, 0u);
+        if (i < 2 * DT_TROWS * DT_VECS && gy >= 0 && gy < g.h && c >= 0 && c < g.pitch)
+            v[k] = __ldg(reinterpret_cast<const uint4 *>((t ? img : blur) + (size_t)image * g.img_stride + (size_t)gy * g.pitch + c));
+    }
+    const int n = min((int)n_kp[image], g.kp_cap);
+    const uint32_t *keys = kp_key + (size_t)image * g.kp_cap;
+    if (warp < 2) {                                             // the keypoints of rows y0 .. y0 + DT_ROWS - 1
+        const int r = warp_lower_bound(keys, n, (uint32_t)(y0 + warp * DT_ROWS) << 16, lane);
+        if (lane == 0) s_range[warp] = r;
+    }
+    if (threadIdx.x == 0) s_cnt = 0;
+    __syncthreads();
+    const int lo = s_range[0], hi = s_range[1];
+    if (lo >= hi) return;
+#pragma unroll
+    for (int k = 0; k < DT_STAGE; ++k) {
+        const int i = threadIdx.x + k * DT_THREADS;
+        if (i >= 2 * DT_TROWS * DT_VECS) break;
+        const int t = i >= DT_TROWS * DT_VECS;
+        const int j = i - t * DT_TROWS * DT_VECS, r = j / DT_VECS, q = j - r * DT_VECS;
+        if (t == 0) {
+            *reinterpret_cast<uint4 *>(s_blur + r * DT_BLUR_B + 16 * q) = v[k];
+        } else {
+            uint32_t *d = s_raw + r * DT_RAW_W + 4 * q;
+            d[0] = v[k].x; d[1] = v[k].y; d[2] = v[k].z; d[3] = v[k].w;
+        }
+    }
+    // per-lane slot geometry of the orientation (same for every keypoint), relative to the patch's first word
+    int soff[(ORI_SLOTS + 31) / 32], sv[(ORI_SLOTS + 31) / 32];
+#pragma unroll
+    for (int k = 0; k < (ORI_SLOTS + 31) / 32; ++k) {
+        const int slot = min(lane + 32 * k, ORI_SLOTS - 1);
+        const int r = slot / ORI_WORDS, w = slot - r * ORI_WORDS;
+        soff[k] = r * DT_RAW_W + w;
+        sv[k] = r - 15;
+    }
+    // rBRIEF: lane l evaluates tests l, l + 32, ..., l + 224 (rbrief_kernel); the sample address comes from the bits of the
+    // 1.5 * 2^23-rounded coordinates:  centre + iy * DT_BLUR_B + ix = (centre - (DT_BLUR_B + 1) * 0x4B400000) + by * DT_BLUR_B + bx
+    float4 pat[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const char4 pt = reinterpret_cast<const char4 *>(d_pattern)[j * 32 + lane];
+        pat[j] = make_float4((float)pt.x, (float)pt.y, (float)pt.z, (float)pt.w);
+    }
+    constexpr uint32_t BIAS = 0x4B400000u * (uint32_t)(DT_BLUR_B + 1);
+    const uint32_t blur_s = (uint32_t)__cvta_generic_to_shared(s_blur) - (uint32_t)(ty0 * DT_BLUR_B + sx) - BIAS;
+    for (int base = lo; base < hi; base += DT_CHUNK) {
+        // the band's keypoints whose x lies in the tile (any order: every result goes to its keypoint's own index)
+#pragma unroll
+        for (int q = 0; q < DT_CHUNK / DT_THREADS; ++q) {
+            const int i = base + q * DT_THREADS + (int)threadIdx.x;
+            uint32_t key = 0;
+            bool in = false;
+            if (i < hi) {
+                key = keys[i];
+                in = (int)(key & 0xFFFF) >= x0 && (int)(key & 0xFFFF) < x0 + DT_COLS;
+            }
+            const uint32_t m = __ballot_sync(FULL, in);
+            int pos = 0;
+            if (lane == 0 && m) pos = atomicAdd(&s_cnt, __popc(m));
+            pos = __shfl_sync(FULL, pos, 0) + __popc(m & ((1u << lane) - 1u));
+            if (in) { s_idx[pos] = (uint32_t)i; s_key[pos] = key; }
+        }
+        __syncthreads();                                        // (also: the tiles are staged)
+        const int m = s_cnt;
+        __syncthreads();
+        if (threadIdx.x == 0) s_cnt = 0;
+        // warp w takes list entries w, w + 8, ...: lane j holds entry w + 8 j of each group of 256
+        for (int grp = 0; grp < m; grp += DT_THREADS) {
+            const int e = grp + warp + DT_WARPS * lane;
+            const bool valid = e < m;
+            const int cnt = __popc(__ballot_sync(FULL, valid));
+            if (cnt == 0) break;
+            const uint32_t my_key = valid ? s_key[e] : 0u;
+            const int my_i = valid ? (int)s_idx[e] : 0;
+            float my_angle = 0.f;
+            // intensity-centroid orientation, two keypoints per round (orient_pack_kernel)
+#pragma unroll 1
+            for (int it = 0; it < cnt; it += 2) {
+                const bool two = it + 1 < cnt;
+                const uint32_t key0 = __shfl_sync(FULL, my_key, it), key1 = __shfl_sync(FULL, my_key, two ? it + 1 : it);
+                const int xl0 = (int)(key0 & 0xFFFF) - 15, xa0 = xl0 & ~3, off0 = xl0 - xa0;
+                const int xl1 = (int)(key1 & 0xFFFF) - 15, xa1 = xl1 & ~3, off1 = xl1 - xa1;
+                const uint32_t *p0 = s_raw + ((int)(key0 >> 16) - 15 - ty0) * DT_RAW_W + ((xa0 - sx) >> 2);
+                const uint32_t *p1 = s_raw + ((int)(key1 >> 16) - 15 - ty0) * DT_RAW_W + ((xa1 - sx) >> 2);
+                const uint32_t *tu0 = d_ori_tab.u[off0], *tm0 = d_ori_tab.m[off0], *tu1 = d_ori_tab.u[off1], *tm1 = d_ori_tab.m[off1];
+                int m10a = 0, m01a = 0, m10b = 0, m01b = 0;
+#pragma unroll
+                for (int k = 0; k < (ORI_SLOTS + 31) / 32; ++k) {
+                    const bool in = lane + 32 * k < ORI_SLOTS;
+                    const int slot = min(lane + 32 * k, ORI_SLOTS - 1);     // words past the last slot are 0
+                    const uint32_t wa = in ? p0[soff[k]] : 0u, wb = in ? p1[soff[k]] : 0u;
+                    m10a = dp4a_u8s8(wa, __ldg(tu0 + slot), m10a);
+                    m01a += sv[k] * dp4a_u8s8(wa, __ldg(tm0 + slot), 0);
+                    m10b = dp4a_u8s8(wb, __ldg(tu1 + slot), m10b);
+                    m01b += sv[k] * dp4a_u8s8(wb, __ldg(tm1 + slot), 0);
+                }
+#pragma unroll
+                for (int off2 = 16; off2; off2 >>= 1) {
+                    m10a += __shfl_xor_sync(FULL, m10a, off2);
+                    m01a += __shfl_xor_sync(FULL, m01a, off2);
+                    m10b += __shfl_xor_sync(FULL, m10b, off2);
+                    m01b += __shfl_xor_sync(FULL, m01b, off2);
+                }
+                const float angle0 = fast_atan2_deg((float)m01a, (float)m10a);
+                const float angle1 = fast_atan2_deg((float)m01b, (float)m10b);
+                if (lane == it) my_angle = angle0;
+                if (two && lane == it + 1) my_angle = angle1;
+            }
+            // the record and the steering (cos, sin) in double, every lane its own keypoint
+            float2 cs = make_float2(1.f, 0.f);
+            if (valid) {
+                const size_t o = (size_t)image * g.kp_cap + my_i;
+                const int x = my_key & 0xFFFF, y = my_key >> 16;
+                const float th = __fmul_rn(my_angle, (float)(3.14159265358979323846 / 180.0));
+                cs = make_float2((float)cos((double)th), (float)sin((double)th));
+                fe_kpoint k;
+                k.x = (float)x; k.y = (float)y; k.size = kp_size; k.angle = my_angle;
+                k.response = report_score ? (float)kp_score[o] : 0.f;
+                k.octave = 0; k.class_id = -1;
+                kp[o] = k;
+                kx[o] = (float)x; ky[o] = (float)y;
+                kcs[o] = cs;
+            }
+            // rBRIEF-256 from the blurred tile (rbrief_kernel)
+#pragma unroll 1
+            for (int it = 0; it < cnt; ++it) {
+                const uint32_t key = __shfl_sync(FULL, my_key, it);
+                const int i = __shfl_sync(FULL, my_i, it);
+                const float a = __shfl_sync(FULL, cs.x, it), b = __shfl_sync(FULL, cs.y, it);
+                const uint32_t pcs = blur_s + (key >> 16) * (uint32_t)DT_BLUR_B + (key & 0xFFFF);
+                auto sample = [&](float fx, float fy) {
+                    const uint32_t bx = __float_as_uint(__fadd_rn(fx, 12582912.f)), by = __float_as_uint(__fadd_rn(fy, 12582912.f));
+                    uint32_t v;
+                    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(pcs + by * (uint32_t)DT_BLUR_B + bx));
+                    return v;
+                };
+                uint32_t word = 0;
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const float4 pt = pat[j];
+                    const float px0 = pt.x, py0 = pt.y, px1 = pt.z, py1 = pt.w;
+                    const uint32_t t0 = sample(__fsub_rn(__fmul_rn(px0, a), __fmul_rn(py0, b)), __fadd_rn(__fmul_rn(px0, b), __fmul_rn(py0, a)));
+                    const uint32_t t1 = sample(__fsub_rn(__fmul_rn(px1, a), __fmul_rn(py1, b)), __fadd_rn(__fmul_rn(px1, b), __fmul_rn(py1, a)));
+                    const uint32_t w = __ballot_sync(FULL, t0 < t1);
+                    if (lane == j) word = w;
+                }
+                if (lane < 8) reinterpret_cast<uint32_t *>(desc + ((size_t)image * g.kp_cap + i) * 32)[lane] = word;
+            }
+        }
+        __syncthreads();                                        // the list is rewritten by the next pass
+    }
+}
+
+int launch_describe_tile(const Geom &g, const DetectParams &p, const Buffers &b, float kp_size, cudaStream_t s) {
+    static bool smem_set[64] = {false};         // per device: the attribute belongs to the device's context
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (!smem_set[dev & 63]) {
+        cudaFuncSetAttribute(orb_describe_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DT_SMEM);
+        smem_set[dev & 63] = true;
+    }
+    dim3 grid(div_up(g.w, DT_COLS), div_up(g.h, DT_ROWS), g.n_images);
+    orb_describe_tile_kernel<<<grid, DT_THREADS, DT_SMEM, s>>>(b.img, b.blur, g, b.n_kp, b.kp_key, b.kp_score, p.nonmax ? 1 : 0,
+                                                               kp_size, b.kp, b.kx, b.ky, b.kcs, b.desc);
+    return 1;
+}
+
 // rBRIEF-256 with a caller-selected pattern (ORB::setPatchSize != 31 -> makeRandomPattern, bin/detect_node:50-51).
 // No staging: the pattern may reach half_patch * sqrt(2) px.  cv2 samples a bordered copy of the image in which
 // only the image area was blurred: a sample outside the image is the RAW pixel at the BORDER_REFLECT_101 position

@@ -990,7 +990,9 @@ int launch_hamming_cross_pruned(const Geom &g, int n_pairs, float max_dy, bool h
     static const int cx_t = getenv("FE_CX_T") ? atoi(getenv("FE_CX_T")) : CX_T;      // B / C split (tuning knob; any value is exact)
     static const int cx_t2 = std::max(cx_t, getenv("FE_CX_T2") ? atoi(getenv("FE_CX_T2")) : CX_T2);   // C / D split (likewise)
     static const bool wide_kill = !(getenv("FE_CX_WIDE") && atoi(getenv("FE_CX_WIDE")) == 0);        // A/B testing
-    cross_classify_kernel<<<dim3(n_pairs, 2), 1024, 0, s>>>(g, mih ? CX_T1 : -2, cx_t, cx_t2, counts, b.cx_bestL, b.cx_bestR,
+    // the splits must not decrease: a B / C split below the A / B split would put an entry into class A and class D at once
+    const int t1 = mih ? CX_T1 : -2, t2 = std::max(cx_t, t1), t3 = std::max(cx_t2, t2);
+    cross_classify_kernel<<<dim3(n_pairs, 2), 1024, 0, s>>>(g, t1, t2, t3, counts, b.cx_bestL, b.cx_bestR,
                                                    have_band && wide_kill ? b.best : nullptr, b.allbest,
                                                    b.colbest, b.cx_thrq, b.cx_thrt, b.cx_qperm, b.cx_tperm, b.cx_n);
     int n_launch = have_band ? 5 : 6;

@@ -319,7 +319,7 @@ int launch_hamming_cross_pruned(const Geom &g, int n_pairs, float max_dy, bool h
                                 const uint32_t *counts, double fused_ratio, cudaStream_t s, cudaStream_t aux = nullptr,
                                 cudaEvent_t ev_fork = nullptr, cudaEvent_t ev_join = nullptr);      // aux: side stream for the join
 // masked kNN-2; train_sorted = train keypoints are in raster order (enables the banded kernel)
-// inner_thr >= 0 (banded path only): additionally produce the cross-check's band candidates b.cx_bestL / b.cx_bestR for
+// inner_thr >= 0 (epipolar band path only): additionally produce the cross-check's band candidates b.cx_bestL / b.cx_bestR for
 // |dy| <= inner_thr in the same pass
 int launch_hamming_knn2(const Geom &g, int n_pairs, const MatchParams &mp, bool train_sorted, const Buffers &b,
                         const uint32_t *counts, float inner_thr, cudaStream_t s);

@@ -12,7 +12,7 @@
 // Keys are (distance << 16 | index): an unsigned min yields the smallest distance and, among ties,
 // the lowest index -- OpenCV's stable ordering (SURVEY.md A.5).  Requires index < 65536.
 //
-// Three kernels:
+// Four kernels:
 //   hamming_cross_kernel  all Nq x Nt pairs, no mask (OpenCV asserts mask.empty() with crossCheck).
 //                         A CTA owns THREADS*QPT queries in registers and streams the train
 //                         descriptors through shared memory; every train word is a warp-wide
@@ -20,10 +20,12 @@
 //                         the 16-lane XU pipe and bounds the kernel, so three of the eight xor
 //                         words are first folded by carry-save adders (LOP3 0x96 / 0xE8 on the
 //                         64-lane ALU pipe): 5 POPCs per 256-bit distance instead of 8.
-//   hamming_band_kernel   masked kNN-2 when the train keypoints are in raster order (always true
-//                         for keypoints this library detected): the allowed trains of a query are
-//                         one contiguous index range, found with a warp-wide 32-ary search, so only
-//                         ~1 % of the pairs are evaluated.  One warp per query.
+//   hamming_band_tile_kernel  epipolar-masked kNN-2 when the train keypoints are in raster order
+//                         (always true for keypoints this library detected): the allowed trains of a
+//                         query are one contiguous index range read from a row table, so only ~1 %
+//                         of the pairs are evaluated.  One thread per query; a CTA stages the trains
+//                         its 256 queries need in shared memory.
+//   hamming_band_kernel   the same for the window mask (WindowMatcher), one warp per query.
 //   hamming_match_kernel  masked kNN-2 over all pairs, for caller-supplied keypoints in any order.
 #include <algorithm>
 #include <cstdlib>
@@ -201,18 +203,108 @@ int launch_rowstart(const Geom &g, const Buffers &b, const uint32_t *counts, cud
     return 1;
 }
 
-template <int MASK, bool H2 = false>
-// (the stereo band is latency-bound: full occupancy, 32 registers, pays -- 0.28 -> 0.23 ms; the window variant carries its
-// candidate list and more state and slows down when squeezed)
-__global__ void __launch_bounds__(BAND_WARPS * 32, MASK == FE_MASK_EPIPOLAR ? 8 : 1)
+// ---- epipolar band, one thread per query over shared-memory train chunks --------------------------------------------------
+// The band of a query holds ~36 trains at the bench's densities, about one per lane of a warp: a warp per query spent its time
+// on the dependent round trips (row table, two ballot trims, scattered train rows, a global atomic per inner-band pair), not on
+// the distances.  Here a CTA takes BT_Q consecutive query indices, one per thread, and stages the span of train rows its
+// queries need -- [min lo, max hi) of their row-table ranges, ~290 trains for a block of detected keypoints -- in shared memory
+// with coalesced loads.  Each thread walks its own range over the staged rows (lanes of one image row read the same train at
+// the same step: broadcasts) and applies band_trim's exact predicate itself; y is non-decreasing, so that keeps the same run.
+// Keys are unique (they carry the index), so best / second / inner best do not depend on the visiting order.
+// Optional inner band (col_out != nullptr): pairs with |yq - yt| <= inner_thr also feed the cross-check's band candidates --
+// row arg-min to inner_best, column arg-min to col_out (the band is symmetric, so this pass sees every pair of every train's
+// band).  The column keys meet in shared memory and leave with one global atomicMin per staged train: the trains at a block's
+// edge are shared with the neighbouring CTAs.
+constexpr int BT_Q = 256;      // queries per CTA, one per thread
+constexpr int BT_T = 512;      // trains per chunk: 16 KB of rows, 2 KB of y, 2 KB of column keys (a bench block's span fits one)
+
+template <bool H2>
+__global__ void __launch_bounds__(BT_Q, 4)
+hamming_band_tile_kernel(Geom g, MatchParams mp, const uint32_t *__restrict__ counts, const uint8_t *__restrict__ desc,
+                         const float *__restrict__ ky, uint32_t *__restrict__ best_out, uint32_t *__restrict__ second_out,
+                         float inner_thr, uint32_t *__restrict__ inner_best, uint32_t *__restrict__ col_out,
+                         const int *__restrict__ rowstart) {
+    __shared__ uint4 s_desc[BT_T * 2];
+    __shared__ float s_ty[BT_T];
+    __shared__ uint32_t s_col[BT_T];
+    __shared__ int s_lo, s_hi;
+    const int pair = blockIdx.y;
+    const int qi = 2 * pair, ti = 2 * pair + 1;
+    const int nq = min((int)counts[qi], g.kp_cap), nt = min((int)counts[ti], g.kp_cap);
+    if ((int)blockIdx.x * BT_Q >= nq) return;
+    const int qidx = blockIdx.x * BT_Q + threadIdx.x;
+    const bool valid = qidx < nq;
+    const float reach = mp.epi_threshold;
+    float qy = 0.f;
+    int lo = nt, hi = 0;                 // empty unless the thread has a query
+    uint32_t q[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    if (valid) {
+        qy = __fadd_rn(ky[(size_t)qi * g.kp_cap + qidx], mp.q_off);
+        band_range(rowstart + (size_t)ti * (g.rs_h + 2), g.rs_h, qy - mp.t_off, reach, lo, hi);
+        hi = min(hi, nt);
+        const uint4 *p = reinterpret_cast<const uint4 *>(desc + ((size_t)qi * g.kp_cap + qidx) * 32);
+        const uint4 a = __ldg(p), b = __ldg(p + 1);
+        q[0] = a.x; q[1] = a.y; q[2] = a.z; q[3] = a.w; q[4] = b.x; q[5] = b.y; q[6] = b.z; q[7] = b.w;
+    }
+    // the CTA's span: min lo / max hi over all its threads -- queries may come in any order
+    if (threadIdx.x == 0) { s_lo = nt; s_hi = 0; }
+    __syncthreads();
+    const int wlo = __reduce_min_sync(0xffffffffu, lo < hi ? lo : nt), whi = __reduce_max_sync(0xffffffffu, lo < hi ? hi : 0);
+    if ((threadIdx.x & 31) == 0) { atomicMin(&s_lo, wlo); atomicMax(&s_hi, whi); }
+    __syncthreads();
+    const int span_lo = s_lo, span_hi = s_hi;
+
+    const uint4 *tdesc = reinterpret_cast<const uint4 *>(desc + (size_t)ti * g.kp_cap * 32);
+    const float *tky = ky + (size_t)ti * g.kp_cap;
+    uint32_t *col = col_out ? col_out + (size_t)pair * g.kp_cap : nullptr;
+    uint32_t best = KEY_NONE, second = KEY_NONE, ibest = KEY_NONE;
+    for (int c0 = span_lo; c0 < span_hi; c0 += BT_T) {
+        const int cn = min(BT_T, span_hi - c0);
+        __syncthreads();                 // the previous chunk is measured and flushed
+        for (int i = threadIdx.x; i < 2 * cn; i += BT_Q) s_desc[i] = __ldg(tdesc + 2 * (size_t)c0 + i);
+        for (int i = threadIdx.x; i < cn; i += BT_Q) {
+            s_ty[i] = tky[c0 + i];
+            if (col) s_col[i] = KEY_NONE;
+        }
+        __syncthreads();
+        const int e = min(hi, c0 + cn);
+        for (int t = max(lo, c0); t < e; ++t) {
+            const int k = t - c0;
+            const float ty = s_ty[k];
+            const float d = __fsub_rn(qy, __fadd_rn(ty, mp.t_off));
+            if (d <= reach && !(d < -reach)) {
+                const uint32_t d16 = hamming256<H2>(q, s_desc[2 * k], s_desc[2 * k + 1]) << 16;
+                const uint32_t key = d16 | (uint32_t)t;
+                second = min(second, max(best, key));
+                best = min(best, key);
+                if (col && fabsf(__fsub_rn(qy, ty)) <= inner_thr) {
+                    ibest = min(ibest, key);
+                    atomicMin(&s_col[k], d16 | (uint32_t)qidx);
+                }
+            }
+        }
+        if (col) {
+            __syncthreads();
+            for (int i = threadIdx.x; i < cn; i += BT_Q)
+                if (s_col[i] != KEY_NONE) atomicMin(&col[c0 + i], s_col[i]);
+        }
+    }
+    if (valid) {
+        const size_t o = (size_t)pair * g.kp_cap + qidx;
+        best_out[o] = best;
+        second_out[o] = second;
+        if (col) inner_best[o] = ibest;
+    }
+}
+
+// ---- window-masked kNN-2 for raster-ordered train keypoints (WindowMatcher), one warp per query --------------------------
+// (one CTA per SM minimum: the kernel carries its candidate list and more state and slows down when squeezed)
+template <bool H2 = false>
+__global__ void __launch_bounds__(BAND_WARPS * 32, 1)
 hamming_band_kernel(Geom g, MatchParams mp, const uint32_t *__restrict__ counts,
                     const uint8_t *__restrict__ desc, const float *__restrict__ kx,
                     const float *__restrict__ ky, uint32_t *__restrict__ best_out,
-                    uint32_t *__restrict__ second_out, float inner_thr, uint32_t *__restrict__ inner_best,
-                    uint32_t *__restrict__ col_out, const int *__restrict__ rowstart) {
-    // Optional inner band (col_out != nullptr): among the visited pairs, those with |yq - yt| <= inner_thr also feed the
-    // cross-check's band candidates -- row arg-min to inner_best, column arg-min to col_out by atomicMin (the band is
-    // symmetric, so this pass sees every pair of every train's band).  One pass then serves mode A and mode B.
+                    uint32_t *__restrict__ second_out, const int *__restrict__ rowstart) {
     const int pair = blockIdx.y;
     const int qi = 2 * pair, ti = 2 * pair + 1;
     const int nq = min((int)counts[qi], g.kp_cap), nt = min((int)counts[ti], g.kp_cap);
@@ -223,17 +315,13 @@ hamming_band_kernel(Geom g, MatchParams mp, const uint32_t *__restrict__ counts,
     const float qx = kx[(size_t)qi * g.kp_cap + qidx];
     const float qy = __fadd_rn(ky[(size_t)qi * g.kp_cap + qidx], mp.q_off);
     // candidate rows from the train image's row table (no search), trimmed to the exact allowed run with the float
-    // arithmetic of allowed<MASK>
-    const float reach = MASK == FE_MASK_EPIPOLAR ? mp.epi_threshold : mp.half_h;
+    // arithmetic of allowed<FE_MASK_WINDOW>
+    const float reach = mp.half_h;
     int lo, hi;
     band_range(rowstart + (size_t)ti * (g.rs_h + 2), g.rs_h, qy - mp.t_off, reach, lo, hi);
     hi = min(hi, nt);
-    if (MASK == FE_MASK_EPIPOLAR)
-        band_trim(lo, hi, lane, [&](int t) { return __fsub_rn(qy, __fadd_rn(tky[t], mp.t_off)) <= reach; },
-                  [&](int t) { return __fsub_rn(qy, __fadd_rn(tky[t], mp.t_off)) < -reach; });
-    else
-        band_trim(lo, hi, lane, [&](int t) { return __fsub_rn(qy, __fadd_rn(tky[t], mp.t_off)) < reach; },
-                  [&](int t) { return __fsub_rn(qy, __fadd_rn(tky[t], mp.t_off)) <= -reach; });
+    band_trim(lo, hi, lane, [&](int t) { return __fsub_rn(qy, __fadd_rn(tky[t], mp.t_off)) < reach; },
+              [&](int t) { return __fsub_rn(qy, __fadd_rn(tky[t], mp.t_off)) <= -reach; });
     uint32_t q[8];
     {
         const uint4 *p = reinterpret_cast<const uint4 *>(desc + ((size_t)qi * g.kp_cap + qidx) * 32);
@@ -241,40 +329,32 @@ hamming_band_kernel(Geom g, MatchParams mp, const uint32_t *__restrict__ counts,
         q[0] = a.x; q[1] = a.y; q[2] = a.z; q[3] = a.w; q[4] = b.x; q[5] = b.y; q[6] = b.z; q[7] = b.w;
     }
     const uint4 *tdesc = reinterpret_cast<const uint4 *>(desc + (size_t)ti * g.kp_cap * 32);
-    uint32_t best = KEY_NONE, second = KEY_NONE, ibest = KEY_NONE;
+    uint32_t best = KEY_NONE, second = KEY_NONE;
     auto measure = [&](int t) {
         const uint4 ta = __ldg(tdesc + 2 * (size_t)t), tb = __ldg(tdesc + 2 * (size_t)t + 1);
-        const uint32_t d16 = hamming256<H2>(q, ta, tb) << 16;
-        const uint32_t key = d16 | (uint32_t)t;
+        const uint32_t key = (hamming256<H2>(q, ta, tb) << 16) | (uint32_t)t;
         second = min(second, max(best, key));
         best = min(best, key);
-        if (col_out && fabsf(__fsub_rn(qy, tky[t])) <= inner_thr) {
-            ibest = min(ibest, key);
-            atomicMin(&col_out[(size_t)pair * g.kp_cap + t], d16 | (uint32_t)qidx);
-        }
     };
-    if (MASK == FE_MASK_WINDOW) {
-        // The row range holds every keypoint of ~100 image rows; the |dx| test keeps ~8 % of them.  Testing and measuring in
-        // the same loop would run the distance code in almost every round for two or three lanes: compact the survivors
-        // into a per-warp list first (ballot + prefix), then measure them densely.
-        __shared__ uint16_t s_list[BAND_WARPS][BAND_LIST];
-        uint16_t *list = s_list[threadIdx.x >> 5];
-        int cnt = 0;
-        for (int t0 = lo; t0 < hi; t0 += 32) {
-            const int t = t0 + lane;
-            const bool pass = t < hi && fabsf(__fsub_rn(qx, tkx[t])) < mp.half_w;
-            const uint32_t m = __ballot_sync(0xffffffffu, pass);
-            if (pass) list[cnt + __popc(m & ((1u << lane) - 1u))] = (uint16_t)t;
-            cnt += __popc(m);
-            if (cnt > BAND_LIST - 32 || t0 + 32 >= hi) {
-                __syncwarp();
-                for (int i = lane; i < cnt; i += 32) measure((int)list[i]);
-                __syncwarp();
-                cnt = 0;
-            }
+    // The row range holds every keypoint of ~100 image rows; the |dx| test keeps ~8 % of them.  Testing and measuring in
+    // the same loop would run the distance code in almost every round for two or three lanes: compact the survivors
+    // into a per-warp list first (ballot + prefix), then measure them densely.
+    __shared__ uint16_t s_list[BAND_WARPS][BAND_LIST];
+    uint16_t *list = s_list[threadIdx.x >> 5];
+    int cnt = 0;
+    for (int t0 = lo; t0 < hi; t0 += 32) {
+        const int t = t0 + lane;
+        const bool pass = t < hi && fabsf(__fsub_rn(qx, tkx[t])) < mp.half_w;
+        const uint32_t m = __ballot_sync(0xffffffffu, pass);
+        if (pass) list[cnt + __popc(m & ((1u << lane) - 1u))] = (uint16_t)t;
+        cnt += __popc(m);
+        if (cnt > BAND_LIST - 32 || t0 + 32 >= hi) {
+            __syncwarp();
+#pragma unroll 1          // (unrolled, the kernel needs 72 registers instead of 40)
+            for (int i = lane; i < cnt; i += 32) measure((int)list[i]);
+            __syncwarp();
+            cnt = 0;
         }
-    } else {
-        for (int t = lo + lane; t < hi; t += 32) measure(t);
     }
 #pragma unroll
     for (int off = 16; off; off >>= 1) {
@@ -283,11 +363,9 @@ hamming_band_kernel(Geom g, MatchParams mp, const uint32_t *__restrict__ counts,
         second = min(min(second, os), max(best, ob));
         best = min(best, ob);
     }
-    if (col_out) ibest = __reduce_min_sync(0xffffffffu, ibest);
     if (lane == 0) {
         best_out[(size_t)pair * g.kp_cap + qidx] = best;
         second_out[(size_t)pair * g.kp_cap + qidx] = second;
-        if (col_out) inner_best[(size_t)pair * g.kp_cap + qidx] = ibest;
     }
 }
 
@@ -412,11 +490,18 @@ int launch_hamming_knn2(const Geom &g, int n_pairs, const MatchParams &mp, bool 
     if (train_sorted && mp.mask != FE_MASK_NONE) {
         if (inner_thr >= 0.f) cudaMemsetAsync(b.cx_bestR, 0xFF, sizeof(uint32_t) * (size_t)n_pairs * g.kp_cap, s);
         launch_rowstart(g, b, counts, s);
-        dim3 grid(div_up(g.kp_cap, BAND_WARPS), n_pairs);
-#define FE_BAND_GO(MASK, H2) hamming_band_kernel<MASK, H2><<<grid, BAND_WARPS * 32, 0, s>>>(g, mp, counts, b.desc, b.kx, b.ky, b.best, b.second, inner_thr, inner_thr >= 0.f ? b.cx_bestL : nullptr, inner_thr >= 0.f ? b.cx_bestR : nullptr, b.rowstart)
-        if (mp.mask == FE_MASK_EPIPOLAR) { if (mp.h2) FE_BAND_GO(FE_MASK_EPIPOLAR, true); else FE_BAND_GO(FE_MASK_EPIPOLAR, false); }
-        else { if (mp.h2) FE_BAND_GO(FE_MASK_WINDOW, true); else FE_BAND_GO(FE_MASK_WINDOW, false); }
+        if (mp.mask == FE_MASK_EPIPOLAR) {
+            dim3 grid(div_up(g.kp_cap, BT_Q), n_pairs);
+#define FE_BAND_GO(H2) hamming_band_tile_kernel<H2><<<grid, BT_Q, 0, s>>>(g, mp, counts, b.desc, b.ky, b.best, b.second, inner_thr, \
+            inner_thr >= 0.f ? b.cx_bestL : nullptr, inner_thr >= 0.f ? b.cx_bestR : nullptr, b.rowstart)
+            if (mp.h2) FE_BAND_GO(true); else FE_BAND_GO(false);
 #undef FE_BAND_GO
+        } else {
+            dim3 grid(div_up(g.kp_cap, BAND_WARPS), n_pairs);
+#define FE_BAND_GO(H2) hamming_band_kernel<H2><<<grid, BAND_WARPS * 32, 0, s>>>(g, mp, counts, b.desc, b.kx, b.ky, b.best, b.second, b.rowstart)
+            if (mp.h2) FE_BAND_GO(true); else FE_BAND_GO(false);
+#undef FE_BAND_GO
+        }
         return 2;
     }
     if (mp.h2) {
@@ -978,12 +1063,12 @@ int launch_hamming_cross_pruned(const Geom &g, int n_pairs, float max_dy, bool h
                                 cudaEvent_t ev_join) {
     MatchParams mp{};
     mp.mask = FE_MASK_EPIPOLAR; mp.epi_threshold = max_dy;
-    dim3 bgrid(div_up(g.kp_cap, BAND_WARPS), n_pairs);
     if (!have_band) {      // (otherwise mode A's band pass already produced cx_bestL / cx_bestR as its inner band)
         cudaMemsetAsync(b.cx_bestR, 0xFF, sizeof(uint32_t) * (size_t)n_pairs * g.kp_cap, s);
         launch_rowstart(g, b, counts, s);
-        hamming_band_kernel<FE_MASK_EPIPOLAR, false><<<bgrid, BAND_WARPS * 32, 0, s>>>(g, mp, counts, b.desc, b.kx, b.ky, reinterpret_cast<uint32_t *>(b.cx_thrq) /* scratch until classify */, b.cx_dummy,
-                                                                                       max_dy, b.cx_bestL, b.cx_bestR, b.rowstart);
+        hamming_band_tile_kernel<false><<<dim3(div_up(g.kp_cap, BT_Q), n_pairs), BT_Q, 0, s>>>(
+            g, mp, counts, b.desc, b.ky, reinterpret_cast<uint32_t *>(b.cx_thrq) /* scratch until classify */, b.cx_dummy, max_dy,
+            b.cx_bestL, b.cx_bestR, b.rowstart);
     }
     const bool mih = use_join && g.kp_cap <= MIH_MAX && b.cx_half;
     // without the join class A is empty (t1 = -2: even "no candidate" entries, d* = -1, fall into class B)

@@ -28,10 +28,9 @@ struct fe_ctx {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     Buffers b;
+    unsigned allocated = 0;   // BufGroup bits of the allocated buffer groups
     Geom g{};                 // geometry of the batch currently resident on the device
-    int max_pitch = 0, max_strips = 0;
-    size_t max_slab_img = 0;
-    size_t max_img_stride = 0;
+    Geom gmax{};              // capacity geometry (fe_config.max_*): what the buffers are sized for
     uint32_t *h_counts = nullptr;   // pinned: [3 * max_images]
     // chunked pipeline (fe_pipeline_batch): copy-in, two compute lanes, copy-out
     cudaStream_t s_in = nullptr, s_out = nullptr, s_cmp[2] = {nullptr, nullptr};
@@ -51,14 +50,9 @@ struct fe_ctx {
     int batch_desc = FE_DESC_ORB256;  // what the batched pipeline describes with (fe_set_batch_descriptor)
     int wu_frames = 0, wu_prev_n = 0;  // fe_window_update: frames in the window, landmarks of the previous frame
     bool wu_prev_sorted = true;
-    int brief_bytes[3] = {0, 0, 0};   // fe_set_brief_pattern: table present for BRIEF-16 / 32 / 64
+    int brief_bytes[3] = {0, 0, 0};   // fe_set_brief_pattern: table present for BRIEF-16 / 32 / 64 (Buffers::brief_tab)
     int brief_orient[3] = {0, 0, 0};
-    int8_t *brief_tab[3] = {nullptr, nullptr, nullptr};   // device tables [bytes * 8][4]
-    // fe_set_freak: cv::FREAK's pattern (device), pattern sizes and parameters (host)
-    float *freak_tab = nullptr;       // [64][256][43][3] (x, y, sigma)
-    int4 *freak_opairs = nullptr;     // [45] (i, j, weight_dx, weight_dy)
-    uchar2 *freak_dpairs = nullptr;   // [512] (i, j)
-    int32_t *freak_scale = nullptr;   // [max_keypoints] scale index per keypoint
+    // fe_set_freak: cv::FREAK's pattern sizes and parameters (the pattern itself is in Buffers::freak_*)
     int freak_sizes[64] = {0};
     int freak_orient = 1, freak_scale_norm = 1, freak_octaves = 4;
     bool cross_prune = true;        // FE_CROSS_PRUNE=0 forces the all-pairs cross-check kernel (A/B testing)
@@ -90,14 +84,48 @@ namespace {
         }                                                                                         \
     } while (0)
 
-template <typename T>
-cudaError_t dev_alloc(T **p, size_t n) {
-    return cudaMalloc(reinterpret_cast<void **>(p), n * sizeof(T));
-}
-
 int fail(fe_ctx *ctx, int code, const char *msg) {
     if (ctx) ctx->err = msg;
     return code;
+}
+
+// Calls f(pointer member, elements per unit at geometry g, scope, group, name) for every entry of FE_BUFFERS.
+template <typename F>
+void for_each_buffer(Buffers &b, const Geom &g, F &&f) {
+#define FE_VISIT(T, name, scope, group, n) f(b.name, (size_t)(n), scope, (unsigned)group, #name);
+    FE_BUFFERS(FE_VISIT)
+#undef FE_VISIT
+}
+
+// Images, or pairs, among the first n_images images: the units per-image and per-pair buffers are laid out in.
+size_t units(BufScope s, int n_images) { return s == PER_IMAGE ? (size_t)n_images : (size_t)(n_images + 1) / 2; }
+
+// Allocates every buffer of the groups in `groups` that is not allocated yet, sized at the capacity geometry, and
+// zero-fills it on the ctx stream (a non-blocking stream does not order against the legacy default stream, so a plain
+// cudaMemset could land after the kernels that follow).  Each allocation carries 64 bytes of slack past its end, which
+// the image kernels' vector loads may touch.
+int ensure(fe_ctx *c, unsigned groups) {
+    groups &= ~c->allocated;
+    if (!groups) return FE_OK;
+    cudaError_t e = cudaSuccess;
+    for_each_buffer(c->b, c->gmax, [&](auto *&p, size_t n, BufScope s, unsigned grp, const char *name) {
+        if (e != cudaSuccess || !(grp & groups) || p || n == 0) return;
+        const size_t bytes = (s == PER_CTX ? 1 : units(s, c->gmax.n_images)) * n * sizeof(*p) + 64;
+        if ((e = cudaMalloc(reinterpret_cast<void **>(&p), bytes)) == cudaSuccess) e = cudaMemsetAsync(p, 0, bytes, c->stream);
+        if (e != cudaSuccess) c->err = std::string("allocating ") + name + ": " + cudaGetErrorString(e);
+    });
+    if (e != cudaSuccess) return FE_ERR_CUDA;
+    c->allocated |= groups;
+    return FE_OK;
+}
+
+// The buffers of images [first, ...) (first even) of the resident geometry g, seen as a batch of their own.
+Buffers view_of(const Buffers &b, const Geom &g, int first) {
+    Buffers v = b;
+    for_each_buffer(v, g, [&](auto *&p, size_t n, BufScope s, unsigned, const char *) {
+        if (p && s != PER_CTX) p += units(s, first) * n;
+    });
+    return v;
 }
 
 cudaEvent_t get_event(fe_ctx *c) {
@@ -152,19 +180,24 @@ void resolve_pending(fe_ctx *c) {
     c->pending.clear();
 }
 
+Geom geom_of(const fe_config &cfg, int w, int h, int n_images) {
+    Geom g{};
+    g.w = w; g.h = h; g.pitch = round_up(w, 16);
+    g.n_images = n_images;
+    set_strip_geometry(g, cfg.nonmax != 0);
+    g.kp_cap = cfg.max_keypoints;
+    g.img_stride = (size_t)g.pitch * h;
+    g.rs_h = cfg.max_height;
+    return g;
+}
+
 int set_geom(fe_ctx *c, int w, int h, int n_images) {
     if (w < 1 || h < 1 || n_images < 1) return fail(c, FE_ERR_BAD_ARG, "non-positive image geometry");
     if (w > c->cfg.max_width || h > c->cfg.max_height)
         return fail(c, FE_ERR_BAD_ARG, "image larger than fe_config.max_width/max_height");
     if (n_images > c->cfg.max_images)
         return fail(c, FE_ERR_CAPACITY, "batch larger than fe_config.max_images");
-    Geom &g = c->g;
-    g.w = w; g.h = h; g.pitch = round_up(w, 16);
-    g.n_images = n_images;
-    set_strip_geometry(g, c->cfg.nonmax != 0);
-    g.kp_cap = c->cfg.max_keypoints;
-    g.img_stride = (size_t)g.pitch * h;
-    g.rs_h = c->cfg.max_height;
+    c->g = geom_of(c->cfg, w, h, n_images);
     return FE_OK;
 }
 
@@ -255,15 +288,7 @@ int run_detect_pyramid(fe_ctx *c, bool describe) {
     const Geom g0 = c->g;
     Buffers &b = c->b;
     const int NI = g0.n_images, L = c->nlevels;
-    if (!b.pyr_kp) {
-        const size_t MI = c->cfg.max_images, C = c->cfg.max_keypoints;
-        FE_CUDA(c, dev_alloc(&b.pyr_img[0], MI * c->max_img_stride + 64));
-        FE_CUDA(c, dev_alloc(&b.pyr_img[1], MI * c->max_img_stride + 64));
-        FE_CUDA(c, dev_alloc(&b.pyr_tab, 2 * (size_t)(c->cfg.max_width + c->cfg.max_height)));
-        FE_CUDA(c, dev_alloc(&b.pyr_kp, MI * C));
-        FE_CUDA(c, dev_alloc(&b.pyr_desc, MI * C * 32));
-        FE_CUDA(c, dev_alloc(&b.pyr_n, MI));
-    }
+    { const int r = ensure(c, GRP_PYRAMID); if (r != FE_OK) return r; }
     FE_CUDA(c, cudaMemsetAsync(b.pyr_n, 0, sizeof(uint32_t) * NI, c->stream));
     // quotas: orb.cpp computeKeyPoints
     const float factor = (float)(1.0 / c->scale_factor);
@@ -307,7 +332,7 @@ int run_detect_pyramid(fe_ctx *c, bool describe) {
             gl.w = dw; gl.h = dh; gl.pitch = round_up(dw, 16);
             set_strip_geometry(gl, c->cfg.nonmax != 0);
             gl.img_stride = (size_t)gl.pitch * dh;
-            uint8_t *cur = b.pyr_img[l & 1];
+            uint8_t *cur = (l & 1) ? b.pyr_img1 : b.pyr_img0;
             { StageTimer t(c, ST_BLUR);
               t.done(launch_resize_linear_exact(prev, pw, ph, ppitch, pstride, cur, dw, dh, gl.pitch, gl.img_stride, b.pyr_tab, NI, c->stream)); }
             v.img = cur;
@@ -355,29 +380,11 @@ MatchParams match_params(const fe_match_cfg *a) {
     return mp;
 }
 
-// Float-descriptor buffers are allocated on first use (a ctx that only ever sees ORB never pays for them).
-int ensure_float_buffers(fe_ctx *c, bool need_integral) {
-    const size_t MI = c->cfg.max_images, C = c->cfg.max_keypoints, P = (MI + 1) / 2;
-    Buffers &b = c->b;
-    if (!b.fdesc) {
-        FE_CUDA(c, dev_alloc(&b.fdesc, MI * C * 128));
-        FE_CUDA(c, cudaMemsetAsync(b.fdesc, 0, MI * C * 128 * sizeof(float), c->stream));
-        FE_CUDA(c, dev_alloc(&b.best64, P * C));
-        FE_CUDA(c, dev_alloc(&b.second64, P * C));
-        FE_CUDA(c, dev_alloc(&b.allbest64, P * C));
-        FE_CUDA(c, dev_alloc(&b.colbest64, P * C));
-        const size_t tiles = ((C + 127) / 128 + 1) / 2 * 2;
-        FE_CUDA(c, dev_alloc(&b.bf16desc, MI * tiles * 128 * 160));   // (128 / 8 + 4) chunks x 128 rows x 8 bf16 per tile
-        FE_CUDA(c, dev_alloc(&b.fnorm, MI * tiles * 128));
-        FE_CUDA(c, dev_alloc(&b.cand, P * 2 * C * 4));
-        FE_CUDA(c, dev_alloc(&b.tc_error, 1));
-        FE_CUDA(c, cudaMemsetAsync(b.tc_error, 0, sizeof(int), c->stream));
-        FE_CUDA(c, cudaHostAlloc(reinterpret_cast<void **>(&c->h_tc_error), sizeof(int), cudaHostAllocDefault));
-        *c->h_tc_error = 0;
-    }
-    if (need_integral && !b.integral)
-        FE_CUDA(c, dev_alloc(&b.integral, MI * (size_t)(c->cfg.max_height + 1) * (c->cfg.max_width + 1)));
-    return FE_OK;
+// What the matchers read beyond the core buffers: L2 keys for float descriptors (dim > 0), and mode B's scratch -- the
+// tensor-core verification for L2, the pruned cross-check for Hamming.  Allocated before any view of the buffers is taken.
+unsigned match_groups(int dim, bool cross) {
+    if (dim > 0) return GRP_FLOAT | (cross ? GRP_VERIFY : 0u);
+    return cross ? GRP_CROSS : 0u;
 }
 
 // Largest SURF window among the keypoints this ctx detects itself: size 7 for plain FAST keypoints, patchSize * scale^level
@@ -393,20 +400,8 @@ int desc_dim(int kind) { return kind == FE_DESC_SURF64 ? 64 : kind == FE_DESC_SU
 int brief_width(int kind) { return kind == FE_DESC_BRIEF16 ? 16 : kind == FE_DESC_BRIEF32 ? 32 : kind == FE_DESC_BRIEF64 ? 64 : 0; }
 int brief_slot(int kind) { return kind - FE_DESC_BRIEF16; }
 
-// L2 matching buffers that only the tensor-core verification needs (lazily allocated once per ctx)
-int ensure_verify_buffers(fe_ctx *c) {
-    Buffers &b = c->b;
-    if (!b.vf_candL) {
-        const size_t PP = (c->cfg.max_images + 1) / 2, C = c->cfg.max_keypoints, CP = (size_t)round_up((int)C, 128);
-        FE_CUDA(c, dev_alloc(&b.vf_candL, PP * C)); FE_CUDA(c, dev_alloc(&b.vf_candR, PP * C));
-        FE_CUDA(c, dev_alloc(&b.vf_limq, PP * CP)); FE_CUDA(c, dev_alloc(&b.vf_limt, PP * CP)); FE_CUDA(c, dev_alloc(&b.vf_limqd, PP * CP)); FE_CUDA(c, dev_alloc(&b.vf_limtd, PP * CP));
-        FE_CUDA(c, dev_alloc(&b.vf_list, PP * l2_verify_list_entries((int)C)));
-        FE_CUDA(c, dev_alloc(&b.vf_npush, PP)); FE_CUDA(c, dev_alloc(&b.vf_maxnorm, (size_t)c->cfg.max_images));
-    }
-    return FE_OK;
-}
-
-// (g, b, st): the batch -- or the chunk view of it -- to match; timed = false on the auxiliary streams of the chunked pipeline
+// (g, b, st): the batch -- or the chunk view of it -- to match; timed = false on the auxiliary streams of the chunked pipeline.
+// Needs the groups of match_groups(dim, cfg_b != nullptr).
 int run_match_l2_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bool timed, int n_pairs, int dim,
                     const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b, const uint32_t *counts, bool train_sorted) {
     const bool masked = cfg_a && cfg_a->mask != FE_MASK_NONE;
@@ -415,7 +410,6 @@ int run_match_l2_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st,
     // Mode B with the |dy| post-filter on raster-ordered trains: band candidates + ONE tcgen05 GEMM + verification.  Exact.
     const bool verify = c->l2_tensor >= 1 && cfg_b && cfg_b->max_dy >= 0.f && train_sorted;
     if (verify) {
-        { const int ra = ensure_verify_buffers(c); if (ra != FE_OK) return ra; }
         // mode A's band pass visits a superset of mode B's band: let it produce the cross-check candidates as well
         const bool fuse = cfg_a && cfg_a->mask == FE_MASK_EPIPOLAR && cfg_a->q_y_offset == 0.f && cfg_a->t_y_offset == 0.f &&
                           cfg_a->epi_threshold >= cfg_b->max_dy;
@@ -459,13 +453,9 @@ int run_match_l2_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st,
     return FE_OK;
 }
 
-int run_match_l2(fe_ctx *c, int n_pairs, int dim, const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b,
-                 const uint32_t *counts, bool train_sorted) {
-    return run_match_l2_on(c, c->g, c->b, c->stream, true, n_pairs, dim, cfg_a, cfg_b, counts, train_sorted);
-}
-
 // train_sorted: the train keypoints of every pair are in raster order (y non-decreasing), which
-// makes the mask-allowed trains of a query one contiguous index range (banded kernel).
+// makes the mask-allowed trains of a query one contiguous index range (banded kernel).  Needs the groups of
+// match_groups(0, cfg_b != nullptr).
 int run_match_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bool timed, int n_pairs,
                  const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b, const uint32_t *counts, bool train_sorted,
                  bool both_sorted) {
@@ -475,32 +465,12 @@ int run_match_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bo
     // Mode B with the |dy| post-filter on raster-ordered keypoints: band candidates + pruned verification (exact; about
     // half the instructions of the all-pairs kernel).  FE_CROSS_PRUNE=0 forces the all-pairs kernel (A/B testing).
     const bool pruned = cfg_b && c->cross_prune && both_sorted && cfg_b->norm == FE_NORM_HAMMING && cfg_b->max_dy >= 0.f;
-    if (pruned && !c->b.cx_bestL) {
-        const size_t PP = (c->cfg.max_images + 1) / 2, C = c->cfg.max_keypoints;
-        Buffers &bb = c->b;
-        FE_CUDA(c, dev_alloc(&bb.cx_bestL, PP * C)); FE_CUDA(c, dev_alloc(&bb.cx_bestR, PP * C)); FE_CUDA(c, dev_alloc(&bb.cx_dummy, PP * C));
-        FE_CUDA(c, dev_alloc(&bb.cx_thrq, PP * C)); FE_CUDA(c, dev_alloc(&bb.cx_thrt, PP * C));
-        FE_CUDA(c, dev_alloc(&bb.cx_qperm, PP * C)); FE_CUDA(c, dev_alloc(&bb.cx_tperm, PP * C));
-        FE_CUDA(c, dev_alloc(&bb.cx_n, PP * 8));
-        if (C <= 16384) {          // multi-index join scratch (match.cu MIH_MAX)
-            FE_CUDA(c, dev_alloc(&bb.cx_half, PP * 2 * 16 * C)); FE_CUDA(c, dev_alloc(&bb.cx_star, PP * 2 * C));
-        }
-    }
-    Buffers bp = b;                // `b` may be a chunk view: give it the (offset) scratch arrays of the ctx
-    if (pruned) {
-        const size_t pr = (size_t)(b.best - c->b.best) / (size_t)g.kp_cap;      // first pair of the view
-        const size_t off = pr * (size_t)g.kp_cap;
-        bp.cx_bestL = c->b.cx_bestL + off; bp.cx_bestR = c->b.cx_bestR + off; bp.cx_dummy = c->b.cx_dummy + off;
-        bp.cx_thrq = c->b.cx_thrq + off; bp.cx_thrt = c->b.cx_thrt + off;
-        bp.cx_qperm = c->b.cx_qperm + off; bp.cx_tperm = c->b.cx_tperm + off; bp.cx_n = c->b.cx_n + pr * 8;
-        if (c->b.cx_half) { bp.cx_half = c->b.cx_half + 2 * off * 16; bp.cx_star = c->b.cx_star + 2 * off; }
-    }
     // mode A's band pass visits a superset of mode B's band: let it produce the cross-check candidates as well
     const bool fuse_band = pruned && cfg_a && train_sorted && cfg_a->norm == FE_NORM_HAMMING && cfg_a->mask == FE_MASK_EPIPOLAR &&
                            cfg_a->q_y_offset == 0.f && cfg_a->t_y_offset == 0.f && cfg_a->epi_threshold >= cfg_b->max_dy;
     if (cfg_a) {
         StageTimer t(c, ST_KNN, st, timed);
-        t.done(launch_hamming_knn2(g, n_pairs, match_params(cfg_a), train_sorted, bp, counts, fuse_band ? cfg_b->max_dy : -1.f, st));
+        t.done(launch_hamming_knn2(g, n_pairs, match_params(cfg_a), train_sorted, b, counts, fuse_band ? cfg_b->max_dy : -1.f, st));
     }
     if (cfg_b) {
         StageTimer t(c, ST_MATCH, st, timed);
@@ -515,7 +485,7 @@ int run_match_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bo
                 FE_CUDA(c, cudaEventCreateWithFlags(&c->ev_join[lane], cudaEventDisableTiming));
             }
             const bool side = overlap && lane >= 0;
-            t.done(launch_hamming_cross_pruned(g, n_pairs, cfg_b->max_dy, fuse_band, c->cross_mih, bp, counts, cfg_a ? std::max(cfg_a->ratio, 0.0) : -1.0, st,
+            t.done(launch_hamming_cross_pruned(g, n_pairs, cfg_b->max_dy, fuse_band, c->cross_mih, b, counts, cfg_a ? std::max(cfg_a->ratio, 0.0) : -1.0, st,
                                                side ? c->s_aux[lane] : nullptr, side ? c->ev_fork[lane] : nullptr, side ? c->ev_join[lane] : nullptr));
         }
         else t.done(launch_hamming_cross(g, n_pairs, cfg_b->norm == FE_NORM_HAMMING2, b, counts, st));
@@ -531,46 +501,114 @@ int run_match_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bo
     return FE_OK;
 }
 
-int run_match(fe_ctx *c, int n_pairs, const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b,
-              const uint32_t *counts, bool train_sorted, bool both_sorted) {
-    return run_match_on(c, c->g, c->b, c->stream, true, n_pairs, cfg_a, cfg_b, counts, train_sorted, both_sorted);
+// Checks the match configs against the batch descriptor and allocates what run_batch_on reads beyond the core buffers.  Runs
+// before any view of the buffers is taken, and its zero-fills are on the ctx stream.
+int prepare_batch(fe_ctx *c, const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b) {
+    const int dim = desc_dim(c->batch_desc);
+    if (dim > 0 && ((cfg_a && cfg_a->norm != FE_NORM_L2) || (cfg_b && cfg_b->norm != FE_NORM_L2)))
+        return fail(c, FE_ERR_UNSUPPORTED, "SURF descriptors are matched with FE_NORM_L2");
+    return ensure(c, match_groups(dim, cfg_b != nullptr) | (dim > 0 && !c->cfg.surf_upright ? GRP_INTEGRAL : 0u));
 }
 
-// The buffers of images [first, first + n) (first even) seen as a batch of their own.
-Buffers view_of(const Buffers &b, const Geom &g, int first) {
-    Buffers v = b;
-    const size_t f = (size_t)first, pr = (size_t)first / 2, C = (size_t)g.kp_cap;
-    v.img += f * g.img_stride; v.blur += f * g.img_stride; v.respmap += f * g.img_stride;
-    v.slab += f * g.slab_img; v.strip_raw += f * g.n_strips; v.strip_sel += f * g.n_strips;
-    v.hist += f * 256; v.n_kp += f; v.n_override += f; v.rowstart += f * (size_t)(g.rs_h + 2);
-    if (v.harris) v.harris += f * C;
-    v.kp_key += f * C; v.kp_score += f * C; v.kp += f * C; v.kx += f * C; v.ky += f * C; v.kcs += f * C;
-    v.desc += f * C * 32;
-    v.best += pr * C; v.second += pr * C; v.allbest += pr * C; v.colbest += pr * C;
-    v.match_a += pr * C; v.match_b += pr * C; v.n_a += pr; v.n_b += pr;
-    if (v.fdesc) {       // float descriptors + L2 matching (lazily allocated; SURF batches)
-        const size_t tiles = ((C + 127) / 128 + 1) / 2 * 2, CP = (size_t)round_up((int)C, 128);
-        v.fdesc += f * C * 128;
-        v.best64 += pr * C; v.second64 += pr * C; v.allbest64 += pr * C; v.colbest64 += pr * C;
-        v.bf16desc += f * tiles * 128 * 160; v.fnorm += f * tiles * 128; v.cand += pr * 2 * C * 4;
-        if (v.integral) v.integral += f * (size_t)(g.h + 1) * (g.w + 1);
-        if (v.vf_candL) {
-            v.vf_candL += pr * C; v.vf_candR += pr * C;
-            v.vf_limq += pr * CP; v.vf_limt += pr * CP; v.vf_limqd += pr * CP; v.vf_limtd += pr * CP;
-            v.vf_list += pr * l2_verify_list_entries((int)C); v.vf_npush += pr; v.vf_maxnorm += f;
-        }
+// Detect, describe and match the batch (g, b) on st: the resident batch, or a chunk view of it.  ORB-256 with Hamming
+// matching, or FAST / ORB-mode keypoints with SURF descriptors (bin/detect_node:33-41) and L2 matching.  The caller applies
+// pending detection changes and calls prepare_batch; the pyramid (nlevels > 1) runs on the whole resident batch only.
+int run_batch_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bool timed, int n_pairs,
+                 const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b) {
+    const int dim = desc_dim(c->batch_desc);
+    const bool sorted = c->nlevels == 1;          // the pyramid's keypoints are level-major, not in raster order
+    int r = sorted ? run_detect_on(c, g, b, st, dim == 0, timed) : run_detect_pyramid(c, dim == 0);
+    if (r != FE_OK) return r;
+    if (dim > 0) {
+        StageTimer t(c, ST_SURF, st, timed);
+        t.done(launch_surf(g, b, b.n_kp, dim == 128, c->cfg.surf_upright != 0, detected_surf_win(c), st));
     }
-    return v;
+    if (!cfg_a && !cfg_b) return FE_OK;
+    if (dim > 0) return run_match_l2_on(c, g, b, st, timed, n_pairs, dim, cfg_a, cfg_b, b.n_kp, sorted);
+    return run_match_on(c, g, b, st, timed, n_pairs, cfg_a, cfg_b, b.n_kp, sorted, sorted);
+}
+
+// Counts of pairs [p0, p0 + np) into h_counts: keypoints of image i at [i], n_a of pair p at [NI + p], n_b at [NI + NP + p]
+// (NI images, NP pairs resident).
+int copy_counts(fe_ctx *c, int p0, int np, cudaStream_t st) {
+    const int NI = c->g.n_images, NP = NI / 2;
+    uint32_t *hc = c->h_counts;
+    FE_CUDA(c, cudaMemcpyAsync(hc + 2 * p0, c->b.n_kp + 2 * p0, sizeof(uint32_t) * 2 * np, cudaMemcpyDeviceToHost, st));
+    FE_CUDA(c, cudaMemcpyAsync(hc + NI + p0, c->b.n_a + p0, sizeof(uint32_t) * np, cudaMemcpyDeviceToHost, st));
+    FE_CUDA(c, cudaMemcpyAsync(hc + NI + NP + p0, c->b.n_b + p0, sizeof(uint32_t) * np, cudaMemcpyDeviceToHost, st));
+    return FE_OK;
+}
+
+// Host arrays of a whole batch: kp_cap keypoints / descriptors per image and matches per pair; null arrays are skipped.
+struct HostBatch {
+    int32_t kp_cap;
+    fe_kpoint *kps;
+    uint8_t *desc;
+    int32_t *n_kps;
+    fe_match *ma;
+    int32_t *n_a;
+    fe_match *mb;
+    int32_t *n_b;
+};
+
+// Downloads pairs [p0, p0 + np) of the resident batch on st into o, sized by the counts copy_counts left in h_counts:
+// reports the counts, sets `overflow` if a keypoint count exceeds either capacity, accounts the bytes and copies the used
+// prefix of every array, one strided copy per array (rows = images or pairs).
+int download_pairs(fe_ctx *c, int p0, int np, cudaStream_t st, const HostBatch &o, bool &overflow) {
+    const Geom &g = c->g;
+    const int NI = g.n_images, NP = NI / 2, i0 = 2 * p0, ni = 2 * np, cap = o.kp_cap;
+    const uint32_t *hc = c->h_counts;
+    int max_kp = 0, max_a = 0, max_b = 0;
+    for (int i = i0; i < i0 + ni; ++i) {
+        if ((int)hc[i] > cap || (int)hc[i] > g.kp_cap) overflow = true;
+        max_kp = std::max(max_kp, std::min(std::min((int)hc[i], cap), g.kp_cap));
+        if (o.n_kps) o.n_kps[i] = (int32_t)hc[i];
+    }
+    for (int p = p0; p < p0 + np; ++p) {
+        max_a = std::max(max_a, std::min((int)hc[NI + p], cap));
+        max_b = std::max(max_b, std::min((int)hc[NI + NP + p], cap));
+        if (o.n_a) o.n_a[p] = (int32_t)hc[NI + p];
+        if (o.n_b) o.n_b[p] = (int32_t)hc[NI + NP + p];
+    }
+    const int dim = desc_dim(c->batch_desc);
+    const size_t drow = dim > 0 ? sizeof(float) * dim : 32;       // descriptor bytes per keypoint on the host
+    c->d2h_bytes += (int64_t)sizeof(uint32_t) * 2 * ni + (o.kps ? (int64_t)sizeof(fe_kpoint) * max_kp * ni : 0) +
+                    (o.desc ? (int64_t)drow * max_kp * ni : 0) + (o.ma ? (int64_t)sizeof(fe_match) * max_a * np : 0) +
+                    (o.mb ? (int64_t)sizeof(fe_match) * max_b * np : 0);
+    const Buffers v = view_of(c->b, g, i0);
+    const size_t C = g.kp_cap, K = cap;
+    if (o.kps && max_kp > 0)
+        FE_CUDA(c, cudaMemcpy2DAsync(o.kps + i0 * K, sizeof(fe_kpoint) * K, v.kp, sizeof(fe_kpoint) * C, sizeof(fe_kpoint) * max_kp,
+                                     ni, cudaMemcpyDeviceToHost, st));
+    if (o.desc && max_kp > 0 && dim != 64)       // host rows as on the device (32 bytes or 128 floats): one strided copy
+        FE_CUDA(c, cudaMemcpy2DAsync(o.desc + i0 * K * drow, drow * K, dim ? (const void *)v.fdesc : v.desc, drow * C,
+                                     drow * max_kp, ni, cudaMemcpyDeviceToHost, st));
+    if (o.desc && max_kp > 0 && dim == 64)       // 64-d: pack the first 64 floats of every 128-float device row
+        for (int i = 0; i < ni; ++i)
+            FE_CUDA(c, cudaMemcpy2DAsync(o.desc + (i0 + i) * K * 256, 256, v.fdesc + i * C * 128, 512, 256,
+                                         std::min((int)hc[i0 + i], max_kp), cudaMemcpyDeviceToHost, st));
+    if (o.ma && max_a > 0)
+        FE_CUDA(c, cudaMemcpy2DAsync(o.ma + p0 * K, sizeof(fe_match) * K, v.match_a, sizeof(fe_match) * C, sizeof(fe_match) * max_a,
+                                     np, cudaMemcpyDeviceToHost, st));
+    if (o.mb && max_b > 0)
+        FE_CUDA(c, cudaMemcpy2DAsync(o.mb + p0 * K, sizeof(fe_match) * K, v.match_b, sizeof(fe_match) * C, sizeof(fe_match) * max_b,
+                                     np, cudaMemcpyDeviceToHost, st));
+    return FE_OK;
+}
+
+// Reads and clears the tcgen05 completion-barrier flag that the L2 tensor-core matchers copy to the host (the streams they
+// ran on must be synchronised).
+bool take_tc_error(fe_ctx *c) {
+    if (!*c->h_tc_error) return false;
+    *c->h_tc_error = 0;
+    cudaMemsetAsync(c->b.tc_error, 0, sizeof(int), c->stream);
+    return true;
 }
 
 int sync_and_resolve(fe_ctx *c) {
     FE_CUDA(c, cudaStreamSynchronize(c->stream));
     resolve_pending(c);
-    if (c->h_tc_error && *c->h_tc_error) {
-        *c->h_tc_error = 0;
-        cudaMemsetAsync(c->b.tc_error, 0, sizeof(int), c->stream);
-        return fail(c, FE_ERR_CUDA, "l2_tensor: tcgen05 completion barrier timed out");
-    }
+    if (take_tc_error(c)) return fail(c, FE_ERR_CUDA, "l2_tensor: tcgen05 completion barrier timed out");
     return FE_OK;
 }
 
@@ -638,51 +676,12 @@ int32_t fe_create(const fe_config *cfg_in, fe_ctx **out) {
         if ((e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)) != cudaSuccess) return bail(e, "cudaStreamCreate");
         c->own_stream = true;
     }
-    c->max_pitch = round_up(cfg.max_width, 16);
-    Geom gmax{};
-    gmax.w = cfg.max_width; gmax.h = cfg.max_height; gmax.pitch = c->max_pitch;
-    set_strip_geometry(gmax, cfg.nonmax != 0);
-    c->max_strips = gmax.n_strips;
-    c->max_slab_img = gmax.slab_img;
-    c->max_img_stride = (size_t)c->max_pitch * cfg.max_height;
-    const size_t MI = cfg.max_images, C = cfg.max_keypoints, P = (MI + 1) / 2;
-    Buffers &b = c->b;
-#define FE_ALLOC(ptr, n)                                                                          \
-    if ((e = dev_alloc(&(ptr), (n))) != cudaSuccess) return bail(e, "cudaMalloc " #ptr);          \
-    if ((e = cudaMemsetAsync((ptr), 0, (n) * sizeof(*(ptr)), c->stream)) != cudaSuccess) return bail(e, "cudaMemset " #ptr)
-    FE_ALLOC(b.img, MI * c->max_img_stride + 64);
-    FE_ALLOC(b.blur, MI * c->max_img_stride + 64);
-    FE_ALLOC(b.respmap, MI * c->max_img_stride + 64);
-    FE_ALLOC(b.slab, MI * c->max_slab_img);
-    FE_ALLOC(b.strip_raw, MI * c->max_strips);
-    FE_ALLOC(b.strip_sel, MI * c->max_strips);
-    FE_ALLOC(b.hist, MI * 256);
-    FE_ALLOC(b.n_kp, MI);
-    FE_ALLOC(b.n_override, MI);
-    FE_ALLOC(b.rowstart, MI * (size_t)(cfg.max_height + 2));
-    FE_ALLOC(b.thr_img, MI);
-    FE_ALLOC(b.pattern, 1024);
-    FE_ALLOC(b.umax, 128);
-    FE_ALLOC(b.kp_key, MI * C);
-    FE_ALLOC(b.kp_score, MI * C);
-    FE_ALLOC(b.kp, MI * C);
-    FE_ALLOC(b.kx, MI * C);
-    FE_ALLOC(b.ky, MI * C);
-    FE_ALLOC(b.kcs, MI * C);
-    FE_ALLOC(b.desc, MI * C * 32);
-    FE_ALLOC(b.best, P * C);
-    FE_ALLOC(b.second, P * C);
-    FE_ALLOC(b.allbest, P * C);
-    FE_ALLOC(b.colbest, P * C);
-    FE_ALLOC(b.match_a, P * C);
-    FE_ALLOC(b.match_b, P * C);
-    FE_ALLOC(b.n_a, P);
-    FE_ALLOC(b.n_b, P);
-#undef FE_ALLOC
-    if ((e = cudaHostAlloc(reinterpret_cast<void **>(&c->h_counts), sizeof(uint32_t) * 3 * MI, cudaHostAllocDefault)) != cudaSuccess)
+    c->gmax = geom_of(cfg, cfg.max_width, cfg.max_height, cfg.max_images);
+    if (ensure(c, GRP_CORE) != FE_OK) { g_create_error = c->err; fe_destroy(c); return FE_ERR_CUDA; }
+    if ((e = cudaHostAlloc(reinterpret_cast<void **>(&c->h_counts), sizeof(uint32_t) * 3 * cfg.max_images, cudaHostAllocDefault)) != cudaSuccess ||
+        (e = cudaHostAlloc(reinterpret_cast<void **>(&c->h_tc_error), sizeof(int), cudaHostAllocDefault)) != cudaSuccess)
         return bail(e, "cudaHostAlloc");
-    // the zero-fills above run on the ctx stream (a non-blocking stream does not order against the
-    // legacy default stream, so a plain cudaMemset could land after the first frame's kernels)
+    *c->h_tc_error = 0;
     if ((e = cudaStreamSynchronize(c->stream)) != cudaSuccess) return bail(e, "cudaStreamSynchronize");
     if (upload_orb_pattern(c, 31, 2) != FE_OK) { g_create_error = c->err; fe_destroy(c); return FE_ERR_CUDA; }
     *out = c;
@@ -693,17 +692,7 @@ void fe_destroy(fe_ctx *c) {
     if (!c) return;
     cudaSetDevice(c->cfg.device);
     if (c->stream) cudaStreamSynchronize(c->stream);
-    Buffers &b = c->b;
-    void *ptrs[] = {b.img, b.blur, b.respmap, b.slab, b.strip_raw, b.strip_sel, b.hist, b.n_kp, b.n_override, b.rowstart, b.thr_img, b.pattern, b.umax, b.pyr_img[0], b.pyr_img[1], b.pyr_tab, b.pyr_kp, b.pyr_desc, b.pyr_n, b.wdesc, b.wkx, b.wky, b.wcount, b.wbest, b.wsecond, b.wmatch, b.wn, b.wq, b.wxyz, b.cx_bestL, b.cx_bestR, b.cx_dummy, b.cx_thrq, b.cx_thrt, b.cx_qperm, b.cx_tperm, b.cx_n, b.cx_half, b.cx_star, b.hes_det, b.hes_trace, b.hes_count, b.hes_kp, b.lm_lkp, b.lm_rkp, b.lm_ldesc, b.lm_rdesc, b.lm_match, b.harris, b.kp_key,
-                    b.kp_score, b.kp, b.kx, b.ky, b.kcs, b.desc, b.fdesc, b.integral, b.best, b.second, b.allbest,
-                    b.colbest, b.best64, b.second64, b.allbest64, b.colbest64, b.bf16desc, b.fnorm, b.cand, b.tc_error, b.match_a, b.match_b, b.n_a, b.n_b};
-    for (void *p : ptrs) if (p) cudaFree(p);
-    for (void *p : {(void *)b.wdesc_r, (void *)b.wbest_r, (void *)b.wcol_r, (void *)b.wu_kp, (void *)b.wu_desc, (void *)b.wu_rdesc, (void *)b.wu_kx,
-                    (void *)b.wu_ky, (void *)b.wu_kcs, (void *)b.wu_n}) if (p) cudaFree(p);
-    for (void *p : {(void *)b.vf_candL, (void *)b.vf_candR, (void *)b.vf_limq, (void *)b.vf_limt, (void *)b.vf_limqd, (void *)b.vf_limtd, (void *)b.vf_list, (void *)b.vf_npush,
-                    (void *)b.vf_maxnorm}) if (p) cudaFree(p);
-    for (void *p : {(void *)b.brief_desc, (void *)c->brief_tab[0], (void *)c->brief_tab[1], (void *)c->brief_tab[2]}) if (p) cudaFree(p);
-    for (void *p : {(void *)c->freak_tab, (void *)c->freak_opairs, (void *)c->freak_dpairs, (void *)c->freak_scale}) if (p) cudaFree(p);
+    for_each_buffer(c->b, c->gmax, [](auto *&p, size_t, BufScope, unsigned, const char *) { if (p) cudaFree(p); });
     if (c->h_counts) cudaFreeHost(c->h_counts);
     if (c->h_tc_error) cudaFreeHost(c->h_tc_error);
     for (auto &p : c->pending) { cudaEventDestroy(p.a); cudaEventDestroy(p.b); }
@@ -969,7 +958,7 @@ static int surf_detect_impl(fe_ctx *c, int n_images, const uint8_t *imgs, int w,
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     int r = set_geom(c, w, h, n_images);
     if (r != FE_OK) return r;
-    if ((r = ensure_float_buffers(c, true)) != FE_OK) return r;
+    if ((r = ensure(c, GRP_FLOAT | GRP_INTEGRAL | GRP_SURFDET)) != FE_OK) return r;
     const Geom &g = c->g;
     Buffers &b = c->b;
     const int R = h, C = w, stride_i = w + 1;              // the integral image is (h + 1) x (w + 1)
@@ -985,13 +974,7 @@ static int surf_detect_impl(fe_ctx *c, int n_images, const uint8_t *imgs, int w,
             offs[idx + 1] = offs[idx] + (size_t)(R / step) * (size_t)(C / step);
         }
     const size_t per_image = (size_t)c->cfg.max_width * c->cfg.max_height * 10 * 2;     // floats of scale space per image (capacity)
-    const int IC = (int)std::min<size_t>(MI, 8);                                          // images per scale-space chunk
-    if (!b.hes_det) {
-        FE_CUDA(c, dev_alloc(&b.hes_det, per_image * IC));
-        FE_CUDA(c, dev_alloc(&b.hes_trace, per_image * IC));
-        FE_CUDA(c, dev_alloc(&b.hes_count, 2 * MI));
-        FE_CUDA(c, dev_alloc(&b.hes_kp, MI * (size_t)c->cfg.max_keypoints));
-    }
+    const int IC = std::min(c->cfg.max_images, HESSIAN_CHUNK_IMAGES);                       // images per scale-space chunk
     if (offs[nTotal] > per_image)
         return fail(c, FE_ERR_CAPACITY, "fe_surf_detect: too many octave layers for the scale-space buffer");
     { StageTimer t(c, ST_H2D); if ((r = upload_images(c, imgs, n_images, stride, 0, 1)) != FE_OK) return r; t.done(0); }
@@ -1152,7 +1135,7 @@ int32_t fe_describe(fe_ctx *c, const uint8_t *img, int32_t w, int32_t h, int32_t
             max_win = std::max(max_win, wsz);
         }
         const bool upright = c->cfg.surf_upright != 0;
-        if ((r = ensure_float_buffers(c, !upright)) != FE_OK) return r;
+        if ((r = ensure(c, GRP_FLOAT | (upright ? 0u : GRP_INTEGRAL))) != FE_OK) return r;
         { StageTimer t(c, ST_H2D);
           if ((r = upload_images(c, img, 1, stride, 0, 1)) != FE_OK) return r;
           if ((r = upload_kps(c, 0, kps, nullptr, n)) != FE_OK) return r;
@@ -1180,7 +1163,7 @@ int32_t fe_describe(fe_ctx *c, const uint8_t *img, int32_t w, int32_t h, int32_t
     if (brief_width(desc_kind) > 0) {
         // cv::BriefDescriptorExtractor::compute: runByImageBorder(PATCH_SIZE / 2 + KERNEL_SIZE / 2 = 28), integral, tests
         const int bw = brief_width(desc_kind), slot = brief_slot(desc_kind);
-        if (!c->brief_tab[slot]) return fail(c, FE_ERR_UNSUPPORTED, "fe_describe: no BRIEF test table for this width (fe_set_brief_pattern)");
+        if (!c->brief_bytes[slot]) return fail(c, FE_ERR_UNSUPPORTED, "fe_describe: no BRIEF test table for this width (fe_set_brief_pattern)");
         const int edge = 28;
         int m = 0;
         for (int i = 0; i < *n_inout; ++i) {
@@ -1190,9 +1173,8 @@ int32_t fe_describe(fe_ctx *c, const uint8_t *img, int32_t w, int32_t h, int32_t
         *n_inout = m;
         if (m == 0) return FE_OK;
         if (m > c->g.kp_cap) return fail(c, FE_ERR_CAPACITY, "more keypoints than fe_config.max_keypoints");
+        if ((r = ensure(c, GRP_INTEGRAL | GRP_BRIEF)) != FE_OK) return r;
         Buffers &bb = c->b;
-        if (!bb.integral) FE_CUDA(c, dev_alloc(&bb.integral, (size_t)c->cfg.max_images * (size_t)(c->cfg.max_height + 1) * (c->cfg.max_width + 1)));
-        if (!bb.brief_desc) FE_CUDA(c, dev_alloc(&bb.brief_desc, (size_t)c->cfg.max_images * c->cfg.max_keypoints * 64));
         { StageTimer t(c, ST_H2D);
           if ((r = upload_images(c, img, 1, stride, 0, 1)) != FE_OK) return r;
           if ((r = upload_kps(c, 0, kps, nullptr, m)) != FE_OK) return r;
@@ -1201,14 +1183,14 @@ int32_t fe_describe(fe_ctx *c, const uint8_t *img, int32_t w, int32_t h, int32_t
           t.done(0); }
         { StageTimer t(c, ST_BLUR); t.done(launch_integral(c->g, bb, c->stream)); }
         { StageTimer t(c, ST_BRIEF);
-          t.done(launch_brief_ext(c->g, bb, bb.n_override, c->brief_tab[slot], bw, c->brief_orient[slot], bb.brief_desc, c->stream)); }
+          t.done(launch_brief_ext(c->g, bb, bb.n_override, bb.brief_tab + (size_t)slot * 512 * 4, bw, c->brief_orient[slot], bb.brief_desc, c->stream)); }
         FE_CUDA(c, cudaGetLastError());
         FE_CUDA(c, cudaMemcpy2DAsync(desc, (size_t)bw, bb.brief_desc, 64, (size_t)bw, m, cudaMemcpyDeviceToHost, c->stream));
         return sync_and_resolve(c);
     }
     if (desc_kind == FE_DESC_FREAK) {
         // cv::FREAK::computeImpl: scale index per keypoint, erase what does not fit, orientation, 512 pair tests
-        if (!c->freak_tab) return fail(c, FE_ERR_UNSUPPORTED, "fe_describe: FREAK is not configured (fe_set_freak)");
+        if (!c->b.freak_tab) return fail(c, FE_ERR_UNSUPPORTED, "fe_describe: FREAK is not configured (fe_set_freak)");
         const float size_cst = static_cast<float>(64 / (0.693147180559945 * c->freak_octaves));
         std::vector<int32_t> sidx;
         int m = 0;
@@ -1225,19 +1207,18 @@ int32_t fe_describe(fe_ctx *c, const uint8_t *img, int32_t w, int32_t h, int32_t
         *n_inout = m;
         if (m == 0) return FE_OK;
         if (m > c->g.kp_cap) return fail(c, FE_ERR_CAPACITY, "more keypoints than fe_config.max_keypoints");
+        if ((r = ensure(c, GRP_INTEGRAL | GRP_BRIEF)) != FE_OK) return r;
         Buffers &bb = c->b;
-        if (!bb.integral) FE_CUDA(c, dev_alloc(&bb.integral, (size_t)c->cfg.max_images * (size_t)(c->cfg.max_height + 1) * (c->cfg.max_width + 1)));
-        if (!bb.brief_desc) FE_CUDA(c, dev_alloc(&bb.brief_desc, (size_t)c->cfg.max_images * c->cfg.max_keypoints * 64));
         { StageTimer t(c, ST_H2D);
           if ((r = upload_images(c, img, 1, stride, 0, 1)) != FE_OK) return r;
           if ((r = upload_kps(c, 0, kps, nullptr, m)) != FE_OK) return r;
           c->h_counts[0] = (uint32_t)m;
           FE_CUDA(c, cudaMemcpyAsync(bb.n_override, c->h_counts, sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
-          FE_CUDA(c, cudaMemcpyAsync(c->freak_scale, sidx.data(), sizeof(int32_t) * m, cudaMemcpyHostToDevice, c->stream));
+          FE_CUDA(c, cudaMemcpyAsync(bb.freak_scale, sidx.data(), sizeof(int32_t) * m, cudaMemcpyHostToDevice, c->stream));
           t.done(0); }
         { StageTimer t(c, ST_BLUR); t.done(launch_integral(c->g, bb, c->stream)); }
         { StageTimer t(c, ST_BRIEF);
-          t.done(launch_freak(c->g, bb, bb.n_override, c->freak_scale, c->freak_tab, c->freak_opairs, c->freak_dpairs, c->freak_orient,
+          t.done(launch_freak(c->g, bb, bb.n_override, bb.freak_scale, bb.freak_tab, bb.freak_opairs, bb.freak_dpairs, c->freak_orient,
                               bb.brief_desc, c->stream)); }
         FE_CUDA(c, cudaGetLastError());
         FE_CUDA(c, cudaMemcpyAsync(kps, bb.kp, sizeof(fe_kpoint) * m, cudaMemcpyDeviceToHost, c->stream));
@@ -1279,8 +1260,9 @@ static int match_host_inputs(fe_ctx *c, const fe_kpoint *qk, const void *qd, int
     const bool wide = desc_kind == FE_DESC_BRIEF64 || desc_kind == FE_DESC_FREAK;      // 512-bit rows (match512.cu)
     if (wide && cfg->norm != FE_NORM_HAMMING) return fail(c, FE_ERR_UNSUPPORTED, "match: BRIEF-64 / FREAK rows go with FE_NORM_HAMMING");
     const int bin_bytes = desc_kind == FE_DESC_BRIEF16 ? 16 : 32;
+    const bool cross = cfg->mode == FE_MATCH_CROSSCHECK;
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
-    if (dim > 0) { int r0 = ensure_float_buffers(c, false); if (r0 != FE_OK) return r0; }
+    { int r0 = ensure(c, wide ? GRP_BRIEF : match_groups(dim, cross)); if (r0 != FE_OK) return r0; }
     if (c->cfg.max_images < 2) return fail(c, FE_ERR_CAPACITY, "matching needs fe_config.max_images >= 2");
     // geometry only matters for kp_cap here; keep whatever image geometry is resident
     if (c->g.kp_cap == 0) { int r = set_geom(c, 16, 16, 2); if (r != FE_OK) return r; }
@@ -1291,7 +1273,6 @@ static int match_host_inputs(fe_ctx *c, const fe_kpoint *qk, const void *qd, int
     if ((r = upload_kps(c, 1, tk, wide ? nullptr : td, nt, dim, bin_bytes)) != FE_OK) return r;
     if (wide) {
         const size_t C = c->g.kp_cap;
-        if (!c->b.brief_desc) FE_CUDA(c, dev_alloc(&c->b.brief_desc, (size_t)c->cfg.max_images * c->cfg.max_keypoints * 64));
         if (nq > 0) FE_CUDA(c, cudaMemcpyAsync(c->b.brief_desc, qd, (size_t)64 * nq, cudaMemcpyHostToDevice, c->stream));
         if (nt > 0) FE_CUDA(c, cudaMemcpyAsync(c->b.brief_desc + C * 64, td, (size_t)64 * nt, cudaMemcpyHostToDevice, c->stream));
     }
@@ -1299,7 +1280,6 @@ static int match_host_inputs(fe_ctx *c, const fe_kpoint *qk, const void *qd, int
     FE_CUDA(c, cudaMemcpyAsync(c->b.n_override, c->h_counts, 2 * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
     t.done(0);
     { StageTimer t2(c, ST_ORIENT); t2.done(launch_unpack_kps(c->g, c->b, c->b.n_override, c->stream)); }
-    const bool cross = cfg->mode == FE_MATCH_CROSSCHECK;
     if (wide) {
         if (cross) {
             { StageTimer t2(c, ST_MATCH); t2.done(launch_hamming512_cross(c->g, 1, c->b.brief_desc, c->b, c->b.n_override, c->stream)); }
@@ -1313,10 +1293,10 @@ static int match_host_inputs(fe_ctx *c, const fe_kpoint *qk, const void *qd, int
     }
     bool sorted = true;
     for (int i = 1; i < nt && sorted; ++i) sorted = !(tk[i].y < tk[i - 1].y);
-    if (dim > 0) return run_match_l2(c, 1, dim, cross ? nullptr : cfg, cross ? cfg : nullptr, c->b.n_override, sorted);
+    if (dim > 0) return run_match_l2_on(c, c->g, c->b, c->stream, true, 1, dim, cross ? nullptr : cfg, cross ? cfg : nullptr, c->b.n_override, sorted);
     bool qsorted = sorted;
     for (int i = 1; i < nq && qsorted; ++i) qsorted = !(qk[i].y < qk[i - 1].y);
-    return run_match(c, 1, cross ? nullptr : cfg, cross ? cfg : nullptr, c->b.n_override, sorted, qsorted);
+    return run_match_on(c, c->g, c->b, c->stream, true, 1, cross ? nullptr : cfg, cross ? cfg : nullptr, c->b.n_override, sorted, qsorted);
 }
 
 int32_t fe_knn2(fe_ctx *c, const fe_kpoint *qk, const void *qd, int32_t nq, const fe_kpoint *tk, const void *td,
@@ -1416,15 +1396,10 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     const size_t C = c->cfg.max_keypoints;
     if (n > (int)C) return fail(c, FE_ERR_CAPACITY, "more landmarks than fe_config.max_keypoints");
+    int r;
+    if ((r = ensure(c, GRP_WUPDATE | (live ? GRP_WLIVE : 0u))) != FE_OK) return r;
     Buffers &b = c->b;
-    if (!b.wu_kp) {
-        FE_CUDA(c, dev_alloc(&b.wu_kp, 2 * C)); FE_CUDA(c, dev_alloc(&b.wu_desc, 2 * C * 32)); FE_CUDA(c, dev_alloc(&b.wu_rdesc, 2 * C * 32));
-        FE_CUDA(c, dev_alloc(&b.wu_kx, 2 * C)); FE_CUDA(c, dev_alloc(&b.wu_ky, 2 * C)); FE_CUDA(c, dev_alloc(&b.wu_kcs, 2 * C));
-        FE_CUDA(c, dev_alloc(&b.wu_n, 2));
-        FE_CUDA(c, dev_alloc(&b.wbest_r, ((size_t)c->cfg.max_images + 1) / 2 * C)); FE_CUDA(c, dev_alloc(&b.wcol_r, ((size_t)c->cfg.max_images + 1) / 2 * C));
-    }
-    if (!b.wbest_r) { FE_CUDA(c, dev_alloc(&b.wbest_r, ((size_t)c->cfg.max_images + 1) / 2 * C)); FE_CUDA(c, dev_alloc(&b.wcol_r, ((size_t)c->cfg.max_images + 1) / 2 * C)); }
-    if (c->g.kp_cap == 0) { int r0 = set_geom(c, 16, 16, 2); if (r0 != FE_OK) return r0; }
+    if (c->g.kp_cap == 0 && (r = set_geom(c, 16, 16, 2)) != FE_OK) return r;
     const int bin_bytes = desc_kind == FE_DESC_BRIEF16 ? 16 : 32;
     auto put_desc = [&](uint8_t *dst, const void *src) -> int {
         if (bin_bytes == 32) { FE_CUDA(c, cudaMemcpyAsync(dst, src, (size_t)32 * n, cudaMemcpyHostToDevice, c->stream)); }
@@ -1434,7 +1409,6 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
         }
         return FE_OK;
     };
-    int r;
     {   // slot 0 <- the new frame
         StageTimer t(c, ST_H2D);
         if (n > 0) {
@@ -1527,20 +1501,9 @@ int32_t fe_window_batch(fe_ctx *c, const fe_match_cfg *cfg, const double *Q, int
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     const Geom &g = c->g;
     const int F = g.n_images / 2, V = F - 1;
+    int r = ensure(c, GRP_WINDOW | (live ? GRP_WLIVE : 0u));
+    if (r != FE_OK) return r;
     Buffers &b = c->b;
-    if (!b.wdesc) {
-        const size_t MI = c->cfg.max_images, C = c->cfg.max_keypoints, P = (MI + 1) / 2;
-        FE_CUDA(c, dev_alloc(&b.wdesc, MI * C * 32));
-        FE_CUDA(c, dev_alloc(&b.wkx, MI * C));
-        FE_CUDA(c, dev_alloc(&b.wky, MI * C));
-        FE_CUDA(c, dev_alloc(&b.wcount, MI));
-        FE_CUDA(c, dev_alloc(&b.wbest, P * C));
-        FE_CUDA(c, dev_alloc(&b.wsecond, P * C));
-        FE_CUDA(c, dev_alloc(&b.wmatch, P * C));
-        FE_CUDA(c, dev_alloc(&b.wn, P));
-        FE_CUDA(c, dev_alloc(&b.wq, 16));
-        FE_CUDA(c, dev_alloc(&b.wxyz, P * C * 3));
-    }
     { StageTimer t(c, ST_ORIENT); t.done(launch_gather_landmarks(g, F, b, 0, b.wdesc, b.wkx, b.wky, b.wcount, c->stream)); }
     // the stereo matcher's kernels on the virtual pairs: a Buffers view whose inputs / outputs are the w* arrays
     Buffers v = b;
@@ -1548,15 +1511,8 @@ int32_t fe_window_batch(fe_ctx *c, const fe_match_cfg *cfg, const double *Q, int
     v.best = b.wbest; v.second = b.wsecond; v.match_a = b.wmatch; v.n_a = b.wn;
     Geom gv = g;
     gv.n_images = 2 * V;
-    int r = FE_OK;
     if (live) {
         // cur <-> prev cross-check on the LEFT descriptors and on the RIGHT descriptors, then the same-landmark intersection
-        if (!b.wdesc_r) {
-            const size_t MI = c->cfg.max_images, C = c->cfg.max_keypoints, P = (MI + 1) / 2;
-            FE_CUDA(c, dev_alloc(&b.wdesc_r, MI * C * 32));
-            FE_CUDA(c, dev_alloc(&b.wbest_r, P * C));
-            FE_CUDA(c, dev_alloc(&b.wcol_r, P * C));
-        }
         { StageTimer t(c, ST_ORIENT); t.done(launch_gather_landmarks(g, F, b, 1, b.wdesc_r, nullptr, nullptr, b.wcount, c->stream)); }
         const bool h2 = cfg->norm == FE_NORM_HAMMING2;
         Buffers vl = b, vr = b;
@@ -1687,8 +1643,7 @@ int32_t fe_set_orb_score_type(fe_ctx *c, int32_t score_type) {
     if (score_type == 0 && (!c->cfg.orientation || c->cfg.fast_type != FE_FAST_9_16 || !c->cfg.nonmax))
         return fail(c, FE_ERR_UNSUPPORTED, "fe_set_orb_score_type: HARRIS_SCORE is cv::ORB's (FAST-9_16, NMS, orientation)");
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
-    if (score_type == 0 && !c->b.harris)
-        FE_CUDA(c, dev_alloc(&c->b.harris, (size_t)c->cfg.max_images * c->cfg.max_keypoints));
+    if (score_type == 0) { const int r = ensure(c, GRP_HARRIS); if (r != FE_OK) return r; }
     c->score_type = score_type;
     return FE_OK;
 }
@@ -1713,15 +1668,9 @@ int32_t fe_batch_landmarks(fe_ctx *c, int32_t which, int32_t cap, fe_kpoint *l_k
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     const Geom &g = c->g;
     const int P = g.n_images / 2;
+    int r = ensure(c, GRP_LANDMARKS);
+    if (r != FE_OK) return r;
     Buffers &b = c->b;
-    if (!b.lm_lkp) {
-        const size_t PP = (c->cfg.max_images + 1) / 2, C = c->cfg.max_keypoints;
-        FE_CUDA(c, dev_alloc(&b.lm_lkp, PP * C));
-        FE_CUDA(c, dev_alloc(&b.lm_rkp, PP * C));
-        FE_CUDA(c, dev_alloc(&b.lm_ldesc, PP * C * 32));
-        FE_CUDA(c, dev_alloc(&b.lm_rdesc, PP * C * 32));
-        FE_CUDA(c, dev_alloc(&b.lm_match, PP * C));
-    }
     const uint32_t *cnt = which == 0 ? b.n_a : b.n_b;
     { StageTimer t(c, ST_FINALIZE);
       t.done(launch_pack_landmarks(g, P, b, cnt, which == 0 ? b.match_a : b.match_b, b.lm_lkp, b.lm_rkp, b.lm_ldesc, b.lm_rdesc,
@@ -1744,8 +1693,7 @@ int32_t fe_batch_landmarks(fe_ctx *c, int32_t which, int32_t cap, fe_kpoint *l_k
         if (r_desc) FE_CUDA(c, cudaMemcpy2DAsync(r_desc, (size_t)32 * cap, b.lm_rdesc, 32 * C, (size_t)32 * mx, P, cudaMemcpyDeviceToHost, c->stream));
         if (matches) FE_CUDA(c, cudaMemcpy2DAsync(matches, sizeof(fe_match) * (size_t)cap, b.lm_match, sizeof(fe_match) * C, sizeof(fe_match) * (size_t)mx, P, cudaMemcpyDeviceToHost, c->stream));
     }
-    int r = sync_and_resolve(c);
-    if (r != FE_OK) return r;
+    if ((r = sync_and_resolve(c)) != FE_OK) return r;
     if (overflow) return fail(c, FE_ERR_CAPACITY, "fe_batch_landmarks: more landmarks than capacity");
     return FE_OK;
 }
@@ -1756,8 +1704,9 @@ int32_t fe_set_brief_pattern(fe_ctx *c, int32_t bytes, const int8_t *tests, int3
         if (tests[i] < -24 || tests[i] > 24) return fail(c, FE_ERR_BAD_ARG, "fe_set_brief_pattern: test offsets must lie in [-24, 24] (PATCH_SIZE 48)");
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     const int slot = bytes == 16 ? 0 : bytes == 32 ? 1 : 2;
-    if (!c->brief_tab[slot]) FE_CUDA(c, dev_alloc(&c->brief_tab[slot], (size_t)512 * 4));
-    FE_CUDA(c, cudaMemcpyAsync(c->brief_tab[slot], tests, (size_t)bytes * 8 * 4, cudaMemcpyHostToDevice, c->stream));
+    const int r = ensure(c, GRP_BRIEF_TAB);
+    if (r != FE_OK) return r;
+    FE_CUDA(c, cudaMemcpyAsync(c->b.brief_tab + (size_t)slot * 512 * 4, tests, (size_t)bytes * 8 * 4, cudaMemcpyHostToDevice, c->stream));
     FE_CUDA(c, cudaStreamSynchronize(c->stream));
     c->brief_bytes[slot] = bytes;
     c->brief_orient[slot] = use_orientation ? 1 : 0;
@@ -1828,13 +1777,11 @@ int32_t fe_set_freak(fe_ctx *c, int32_t orientation_normalized, int32_t scale_no
         dp[k] = make_uchar2((unsigned char)i, (unsigned char)(selected[k] - i * (i - 1) / 2));
     }
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
-    if (!c->freak_tab) FE_CUDA(c, dev_alloc(&c->freak_tab, tab.size()));
-    if (!c->freak_opairs) FE_CUDA(c, dev_alloc(&c->freak_opairs, (size_t)NOP));
-    if (!c->freak_dpairs) FE_CUDA(c, dev_alloc(&c->freak_dpairs, (size_t)NPAIRS));
-    if (!c->freak_scale) FE_CUDA(c, dev_alloc(&c->freak_scale, (size_t)c->cfg.max_images * c->cfg.max_keypoints));
-    FE_CUDA(c, cudaMemcpyAsync(c->freak_tab, tab.data(), tab.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    FE_CUDA(c, cudaMemcpyAsync(c->freak_opairs, op, sizeof(op), cudaMemcpyHostToDevice, c->stream));
-    FE_CUDA(c, cudaMemcpyAsync(c->freak_dpairs, dp, sizeof(dp), cudaMemcpyHostToDevice, c->stream));
+    const int r = ensure(c, GRP_FREAK);
+    if (r != FE_OK) return r;
+    FE_CUDA(c, cudaMemcpyAsync(c->b.freak_tab, tab.data(), tab.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    FE_CUDA(c, cudaMemcpyAsync(c->b.freak_opairs, op, sizeof(op), cudaMemcpyHostToDevice, c->stream));
+    FE_CUDA(c, cudaMemcpyAsync(c->b.freak_dpairs, dp, sizeof(dp), cudaMemcpyHostToDevice, c->stream));
     FE_CUDA(c, cudaStreamSynchronize(c->stream));
     c->freak_orient = orientation_normalized ? 1 : 0;
     c->freak_scale_norm = scale_normalized ? 1 : 0;
@@ -1860,85 +1807,26 @@ int32_t fe_set_batch_descriptor(fe_ctx *c, int32_t desc_kind) {
 int32_t fe_batch_run(fe_ctx *c, const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b, int32_t sync) {
     if (!c || c->g.n_images < 2) return fail(c, FE_ERR_BAD_ARG, "fe_batch_run: nothing uploaded");
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
-    const int dim = desc_dim(c->batch_desc);
-    int r;
-    if (dim > 0) {
-        // FAST / ORB-mode keypoints, SURF descriptors (bin/detect_node:33-41), L2 matching
-        const bool upright = c->cfg.surf_upright != 0;
-        if ((r = ensure_float_buffers(c, !upright)) != FE_OK) return r;
-        if ((r = run_detect(c, false)) != FE_OK) return r;
-        { StageTimer t(c, ST_SURF); t.done(launch_surf(c->g, c->b, c->b.n_kp, dim == 128, upright, detected_surf_win(c), c->stream)); }
-        if (cfg_a || cfg_b) {
-            if ((cfg_a && cfg_a->norm != FE_NORM_L2) || (cfg_b && cfg_b->norm != FE_NORM_L2))
-                return fail(c, FE_ERR_UNSUPPORTED, "SURF descriptors are matched with FE_NORM_L2");
-            if ((r = run_match_l2(c, c->g.n_images / 2, dim, cfg_a, cfg_b, c->b.n_kp, c->nlevels == 1)) != FE_OK) return r;
-        }
-        if (sync) return sync_and_resolve(c);
-        return FE_OK;
-    }
-    r = run_detect(c, true);
-    if (r != FE_OK) return r;
-    if (cfg_a || cfg_b) {
-        if ((r = run_match(c, c->g.n_images / 2, cfg_a, cfg_b, c->b.n_kp, c->nlevels == 1, c->nlevels == 1)) != FE_OK) return r;
-    }
-    if (sync) return sync_and_resolve(c);
-    return FE_OK;
+    apply_pending_detection(c);
+    int r = prepare_batch(c, cfg_a, cfg_b);
+    if (r == FE_OK) r = run_batch_on(c, c->g, c->b, c->stream, true, c->g.n_images / 2, cfg_a, cfg_b);
+    if (r != FE_OK || !sync) return r;
+    return sync_and_resolve(c);
 }
 
 int32_t fe_batch_download(fe_ctx *c, int32_t kp_cap, fe_kpoint *kps, uint8_t *desc, int32_t *n_kps,
                           fe_match *ma, int32_t *n_a, fe_match *mb, int32_t *n_b) {
     if (!c || c->g.n_images < 2 || kp_cap < 1) return fail(c, FE_ERR_BAD_ARG, "fe_batch_download: bad argument");
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
-    const Geom &g = c->g;
-    const int NI = g.n_images, NP = NI / 2;
-    StageTimer t(c, ST_D2H);
-    uint32_t *hc = c->h_counts;
-    FE_CUDA(c, cudaMemcpyAsync(hc, c->b.n_kp, sizeof(uint32_t) * NI, cudaMemcpyDeviceToHost, c->stream));
-    FE_CUDA(c, cudaMemcpyAsync(hc + NI, c->b.n_a, sizeof(uint32_t) * NP, cudaMemcpyDeviceToHost, c->stream));
-    FE_CUDA(c, cudaMemcpyAsync(hc + NI + NP, c->b.n_b, sizeof(uint32_t) * NP, cudaMemcpyDeviceToHost, c->stream));
-    FE_CUDA(c, cudaStreamSynchronize(c->stream));
+    const int NP = c->g.n_images / 2;
     bool overflow = false;
-    int max_kp = 0, max_a = 0, max_b = 0;
-    for (int i = 0; i < NI; ++i) {
-        if ((int)hc[i] > kp_cap || (int)hc[i] > g.kp_cap) overflow = true;
-        max_kp = std::max(max_kp, std::min(std::min((int)hc[i], kp_cap), g.kp_cap));
-        if (n_kps) n_kps[i] = (int32_t)hc[i];
-    }
-    for (int p = 0; p < NP; ++p) {
-        max_a = std::max(max_a, std::min((int)hc[NI + p], kp_cap));
-        max_b = std::max(max_b, std::min((int)hc[NI + NP + p], kp_cap));
-        if (n_a) n_a[p] = (int32_t)hc[NI + p];
-        if (n_b) n_b[p] = (int32_t)hc[NI + NP + p];
-    }
-    c->d2h_bytes += (int64_t)sizeof(uint32_t) * (NI + 2 * NP) + (kps ? (int64_t)sizeof(fe_kpoint) * max_kp * NI : 0) +
-                    (desc ? (int64_t)32 * max_kp * NI : 0) + (ma ? (int64_t)sizeof(fe_match) * max_a * NP : 0) +
-                    (mb ? (int64_t)sizeof(fe_match) * max_b * NP : 0);
-    // one strided copy per array: rows = images (or pairs), width = the longest used prefix
-    if (kps && max_kp > 0)
-        FE_CUDA(c, cudaMemcpy2DAsync(kps, sizeof(fe_kpoint) * (size_t)kp_cap, c->b.kp, sizeof(fe_kpoint) * (size_t)g.kp_cap,
-                                     sizeof(fe_kpoint) * (size_t)max_kp, NI, cudaMemcpyDeviceToHost, c->stream));
-    const int ddim = desc_dim(c->batch_desc);
-    if (desc && max_kp > 0 && ddim == 0)
-        FE_CUDA(c, cudaMemcpy2DAsync(desc, (size_t)32 * kp_cap, c->b.desc, (size_t)32 * g.kp_cap, (size_t)32 * max_kp, NI,
-                                     cudaMemcpyDeviceToHost, c->stream));
-    if (desc && max_kp > 0 && ddim > 0) {
-        if (ddim == 128)       // device rows are 128 floats: one strided copy per batch
-            FE_CUDA(c, cudaMemcpy2DAsync(desc, (size_t)512 * kp_cap, c->b.fdesc, (size_t)512 * g.kp_cap, (size_t)512 * max_kp, NI,
-                                         cudaMemcpyDeviceToHost, c->stream));
-        else                   // 64-d: pack the first 64 floats of every 128-float device row
-            for (int i = 0; i < NI; ++i)
-                FE_CUDA(c, cudaMemcpy2DAsync(desc + (size_t)i * kp_cap * 256, 256, c->b.fdesc + (size_t)i * g.kp_cap * 128, 512, 256,
-                                             std::min((int)hc[i], max_kp), cudaMemcpyDeviceToHost, c->stream));
-    }
-    if (ma && max_a > 0)
-        FE_CUDA(c, cudaMemcpy2DAsync(ma, sizeof(fe_match) * (size_t)kp_cap, c->b.match_a, sizeof(fe_match) * (size_t)g.kp_cap,
-                                     sizeof(fe_match) * (size_t)max_a, NP, cudaMemcpyDeviceToHost, c->stream));
-    if (mb && max_b > 0)
-        FE_CUDA(c, cudaMemcpy2DAsync(mb, sizeof(fe_match) * (size_t)kp_cap, c->b.match_b, sizeof(fe_match) * (size_t)g.kp_cap,
-                                     sizeof(fe_match) * (size_t)max_b, NP, cudaMemcpyDeviceToHost, c->stream));
-    t.done(0);
-    int r = sync_and_resolve(c);
+    StageTimer t(c, ST_D2H);
+    int r = copy_counts(c, 0, NP, c->stream);
     if (r != FE_OK) return r;
+    FE_CUDA(c, cudaStreamSynchronize(c->stream));
+    if ((r = download_pairs(c, 0, NP, c->stream, {kp_cap, kps, desc, n_kps, ma, n_a, mb, n_b}, overflow)) != FE_OK) return r;
+    t.done(0);
+    if ((r = sync_and_resolve(c)) != FE_OK) return r;
     if (overflow) return fail(c, FE_ERR_CAPACITY, "fe_batch_download: keypoint capacity exceeded (counts report the required size)");
     return FE_OK;
 }
@@ -1955,20 +1843,13 @@ static const int kChunkPairs = chunk_pairs_init();
 static int chunk_pairs_of(const fe_ctx *c) { return c->chunk_pairs > 0 ? c->chunk_pairs : kChunkPairs; }
 
 static int pipeline_chunked(fe_ctx *c, int32_t n_pairs, const uint8_t *left, const uint8_t *right, int32_t w, int32_t h,
-                            const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b, int32_t kp_cap, fe_kpoint *kps,
-                            uint8_t *desc, int32_t *n_kps, fe_match *ma, int32_t *n_a, fe_match *mb, int32_t *n_b) {
+                            const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b, const HostBatch &out) {
     int r = set_geom(c, w, h, 2 * n_pairs);
     if (r != FE_OK) return r;
     apply_pending_detection(c);
+    // the chunk views below copy the buffer pointers: everything the batch body reads must exist now
+    if ((r = prepare_batch(c, cfg_a, cfg_b)) != FE_OK) return r;
     const Geom &g = c->g;
-    const int dim = desc_dim(c->batch_desc);             // 0: ORB-256 / Hamming; 64 / 128: SURF / L2
-    const bool upright = c->cfg.surf_upright != 0;
-    if (dim > 0) {       // the chunk views below copy the buffer pointers: everything the float path needs must exist now
-        if ((r = ensure_float_buffers(c, !upright)) != FE_OK) return r;
-        if ((r = ensure_verify_buffers(c)) != FE_OK) return r;
-        if ((cfg_a && cfg_a->norm != FE_NORM_L2) || (cfg_b && cfg_b->norm != FE_NORM_L2))
-            return fail(c, FE_ERR_UNSUPPORTED, "SURF descriptors are matched with FE_NORM_L2");
-    }
     const int kChunk = chunk_pairs_of(c);
     const int n_chunks = div_up(n_pairs, kChunk);
     if (!c->s_in) {
@@ -1985,12 +1866,10 @@ static int pipeline_chunked(fe_ctx *c, int32_t n_pairs, const uint8_t *left, con
         c->ev_in.push_back(a);
         c->ev_done.push_back(b);
     }
-    // order the auxiliary streams after whatever is still running on the ctx stream
+    // order the auxiliary streams after whatever is still running on the ctx stream (the zero-fills of prepare_batch included)
     FE_CUDA(c, cudaEventRecord(c->ev_sync, c->stream));
     for (cudaStream_t st : {c->s_in, c->s_out, c->s_cmp[0], c->s_cmp[1]}) FE_CUDA(c, cudaStreamWaitEvent(st, c->ev_sync, 0));
 
-    const int NI = g.n_images, NP = n_pairs;
-    uint32_t *hc = c->h_counts;
     for (int k = 0; k < n_chunks; ++k) {
         const int p0 = k * kChunk, np = std::min(kChunk, n_pairs - p0);
         // H2D of this chunk's images: left -> even slots, right -> odd slots
@@ -2011,74 +1890,21 @@ static int pipeline_chunked(fe_ctx *c, int32_t n_pairs, const uint8_t *left, con
         FE_CUDA(c, cudaStreamWaitEvent(cs, c->ev_in[k], 0));
         Geom gk = g;
         gk.n_images = 2 * np;
-        const Buffers bk = view_of(c->b, g, 2 * p0);
-        if (dim == 0) {
-            if ((r = run_detect_on(c, gk, bk, cs, true, false)) != FE_OK) return r;
-            if (cfg_a || cfg_b)
-                if ((r = run_match_on(c, gk, bk, cs, false, np, cfg_a, cfg_b, bk.n_kp, true, true)) != FE_OK) return r;
-        } else {
-            // FAST / ORB-mode keypoints, SURF descriptors (bin/detect_node:33-41), L2 matching -- as fe_batch_run, per chunk
-            if ((r = run_detect_on(c, gk, bk, cs, false, false)) != FE_OK) return r;
-            c->launches += launch_surf(gk, bk, bk.n_kp, dim == 128, upright, detected_surf_win(c), cs);
-            if (cfg_a || cfg_b)
-                if ((r = run_match_l2_on(c, gk, bk, cs, false, np, dim, cfg_a, cfg_b, bk.n_kp, true)) != FE_OK) return r;
-        }
+        if ((r = run_batch_on(c, gk, view_of(c->b, g, 2 * p0), cs, false, np, cfg_a, cfg_b)) != FE_OK) return r;
         // counts ride on the compute lane so that the host can size this chunk's downloads
-        FE_CUDA(c, cudaMemcpyAsync(hc + 2 * p0, bk.n_kp, sizeof(uint32_t) * 2 * np, cudaMemcpyDeviceToHost, cs));
-        FE_CUDA(c, cudaMemcpyAsync(hc + NI + p0, bk.n_a, sizeof(uint32_t) * np, cudaMemcpyDeviceToHost, cs));
-        FE_CUDA(c, cudaMemcpyAsync(hc + NI + NP + p0, bk.n_b, sizeof(uint32_t) * np, cudaMemcpyDeviceToHost, cs));
+        if ((r = copy_counts(c, p0, np, cs)) != FE_OK) return r;
         FE_CUDA(c, cudaEventRecord(c->ev_done[k], cs));
     }
     bool overflow = false;
-    const size_t C = (size_t)g.kp_cap;
     for (int k = 0; k < n_chunks; ++k) {
         const int p0 = k * kChunk, np = std::min(kChunk, n_pairs - p0);
         FE_CUDA(c, cudaEventSynchronize(c->ev_done[k]));
         FE_CUDA(c, cudaStreamWaitEvent(c->s_out, c->ev_done[k], 0));
-        int max_kp = 0, max_a = 0, max_b = 0;
-        for (int i = 2 * p0; i < 2 * (p0 + np); ++i) {
-            if ((int)hc[i] > kp_cap || (int)hc[i] > g.kp_cap) overflow = true;
-            max_kp = std::max(max_kp, std::min(std::min((int)hc[i], kp_cap), g.kp_cap));
-            if (n_kps) n_kps[i] = (int32_t)hc[i];
-        }
-        for (int p = p0; p < p0 + np; ++p) {
-            max_a = std::max(max_a, std::min((int)hc[NI + p], kp_cap));
-            max_b = std::max(max_b, std::min((int)hc[NI + NP + p], kp_cap));
-            if (n_a) n_a[p] = (int32_t)hc[NI + p];
-            if (n_b) n_b[p] = (int32_t)hc[NI + NP + p];
-        }
-        const size_t i0 = (size_t)2 * p0;
-        const int64_t drow = dim > 0 ? (int64_t)dim * 4 : 32;       // descriptor bytes per keypoint
-        c->d2h_bytes += (int64_t)sizeof(uint32_t) * 4 * np + (kps ? (int64_t)sizeof(fe_kpoint) * max_kp * 2 * np : 0) +
-                        (desc ? drow * max_kp * 2 * np : 0) + (ma ? (int64_t)sizeof(fe_match) * max_a * np : 0) +
-                        (mb ? (int64_t)sizeof(fe_match) * max_b * np : 0);
-        if (kps && max_kp > 0)
-            FE_CUDA(c, cudaMemcpy2DAsync(kps + i0 * kp_cap, sizeof(fe_kpoint) * (size_t)kp_cap, c->b.kp + i0 * C, sizeof(fe_kpoint) * C,
-                                         sizeof(fe_kpoint) * (size_t)max_kp, 2 * np, cudaMemcpyDeviceToHost, c->s_out));
-        if (desc && max_kp > 0 && dim == 0)
-            FE_CUDA(c, cudaMemcpy2DAsync(desc + i0 * kp_cap * 32, (size_t)32 * kp_cap, c->b.desc + i0 * C * 32, 32 * C, (size_t)32 * max_kp,
-                                         2 * np, cudaMemcpyDeviceToHost, c->s_out));
-        if (desc && max_kp > 0 && dim == 128)      // device rows are 128 floats: one strided copy per chunk
-            FE_CUDA(c, cudaMemcpy2DAsync(desc + i0 * kp_cap * 512, (size_t)512 * kp_cap, c->b.fdesc + i0 * C * 128, (size_t)512 * C,
-                                         (size_t)512 * max_kp, 2 * np, cudaMemcpyDeviceToHost, c->s_out));
-        if (desc && max_kp > 0 && dim == 64)       // 64-d: pack the first 64 floats of every 128-float device row
-            for (int i = 2 * p0; i < 2 * (p0 + np); ++i)
-                FE_CUDA(c, cudaMemcpy2DAsync(desc + (size_t)i * kp_cap * 256, 256, c->b.fdesc + (size_t)i * C * 128, 512, 256,
-                                             std::min(std::min((int)hc[i], kp_cap), g.kp_cap), cudaMemcpyDeviceToHost, c->s_out));
-        if (ma && max_a > 0)
-            FE_CUDA(c, cudaMemcpy2DAsync(ma + (size_t)p0 * kp_cap, sizeof(fe_match) * (size_t)kp_cap, c->b.match_a + (size_t)p0 * C,
-                                         sizeof(fe_match) * C, sizeof(fe_match) * (size_t)max_a, np, cudaMemcpyDeviceToHost, c->s_out));
-        if (mb && max_b > 0)
-            FE_CUDA(c, cudaMemcpy2DAsync(mb + (size_t)p0 * kp_cap, sizeof(fe_match) * (size_t)kp_cap, c->b.match_b + (size_t)p0 * C,
-                                         sizeof(fe_match) * C, sizeof(fe_match) * (size_t)max_b, np, cudaMemcpyDeviceToHost, c->s_out));
+        if ((r = download_pairs(c, p0, np, c->s_out, out, overflow)) != FE_OK) return r;
     }
     FE_CUDA(c, cudaStreamSynchronize(c->s_out));
     FE_CUDA(c, cudaStreamSynchronize(c->s_in));
-    if (c->h_tc_error && *c->h_tc_error) {
-        *c->h_tc_error = 0;
-        cudaMemsetAsync(c->b.tc_error, 0, sizeof(int), c->stream);
-        return fail(c, FE_ERR_CUDA, "l2 verification: tcgen05 completion barrier timed out");
-    }
+    if (take_tc_error(c)) return fail(c, FE_ERR_CUDA, "l2 verification: tcgen05 completion barrier timed out");
     if (overflow) return fail(c, FE_ERR_CAPACITY, "fe_pipeline_batch: keypoint capacity exceeded (counts report the required size)");
     return FE_OK;
 }
@@ -2090,7 +1916,7 @@ int32_t fe_pipeline_batch(fe_ctx *c, int32_t n_pairs, const uint8_t *left, const
         (c->batch_desc == FE_DESC_ORB256 || desc_dim(c->batch_desc) > 0)) {
         // overlapped path: H2D of chunk k+1, kernels of chunk k and D2H of chunk k-1 run concurrently
         FE_CUDA(c, cudaSetDevice(c->cfg.device));
-        return pipeline_chunked(c, n_pairs, left, right, w, h, cfg_a, cfg_b, kp_cap, kps, desc, n_kps, ma, n_a, mb, n_b);
+        return pipeline_chunked(c, n_pairs, left, right, w, h, cfg_a, cfg_b, {kp_cap, kps, desc, n_kps, ma, n_a, mb, n_b});
     }
     int r = fe_batch_upload(c, n_pairs, left, right, w, h);
     if (r != FE_OK) return r;
@@ -2112,7 +1938,7 @@ int32_t fe_stereo_features(fe_ctx *c, const uint8_t *left, const uint8_t *right,
     if (dim > 0) {
         if (detected_surf_win(c) > SURF_DIRECT_MAX_WIN)
             return fail(c, FE_ERR_UNSUPPORTED, "fe_stereo_features: SURF keypoint size not supported");
-        if ((r = ensure_float_buffers(c, !upright)) != FE_OK) return r;
+        if ((r = ensure(c, GRP_FLOAT | (upright ? 0u : GRP_INTEGRAL))) != FE_OK) return r;
     }
     const bool was = c->profiling;
     c->profiling = true;     // the service reports per-stage ProcTime (bin/feature_node:27-34,72-75)

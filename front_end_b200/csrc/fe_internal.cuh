@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <atomic>
 #include <string>
 
@@ -105,81 +106,146 @@ struct WarpRow {
 };
 
 // ---- device buffers (one set per ctx, sized for cfg.max_*) ------------------------------------
+// Largest per-image keypoint capacity the multi-index join of the pruned cross-check serves (match.cu: its shared-memory
+// hash table holds 2 x cap x 4 B = 128 KB); above it the join's scratch (cx_half, cx_star) is not allocated.
+constexpr int MIH_MAX = 16384;
+constexpr int HESSIAN_CHUNK_IMAGES = 8;   // images per scale-space pass of the SURF detector (Buffers::hes_det / hes_trace)
+
+// Layout unit of a buffer: one slice per image, one per pair (image 2p = query/left, 2p+1 = train/right), or one per ctx.
+enum BufScope { PER_IMAGE, PER_PAIR, PER_CTX };
+// Allocation groups: fe_create allocates GRP_CORE, the paths that need another group allocate it on first use, so that a
+// ctx never pays for memory its descriptors and matchers do not read.
+enum BufGroup : unsigned {
+    GRP_CORE = 1u << 0,        // detection, ORB-256 descriptors, Hamming matching
+    GRP_FLOAT = 1u << 1,       // float descriptors (SURF) and L2 matching
+    GRP_INTEGRAL = 1u << 2,    // integral images (SURF orientation, BRIEF, FREAK)
+    GRP_VERIFY = 1u << 3,      // exact tensor-core L2 cross-check (l2verify.cu)
+    GRP_CROSS = 1u << 4,       // pruned Hamming cross-check
+    GRP_HARRIS = 1u << 5,      // cv::ORB HARRIS_SCORE
+    GRP_BRIEF = 1u << 6,       // 64-byte binary rows (BRIEF-16 / 32 / 64, FREAK)
+    GRP_BRIEF_TAB = 1u << 7,   // cv::BriefDescriptorExtractor test tables
+    GRP_FREAK = 1u << 8,       // cv::FREAK pattern
+    GRP_WINDOW = 1u << 9,      // WindowMatcher over a resident sequence (fe_window_batch)
+    GRP_WLIVE = 1u << 10,      // its liveGraph variant: right-descriptor cross-check
+    GRP_WUPDATE = 1u << 11,    // fe_window_update's current / previous landmark lists
+    GRP_SURFDET = 1u << 12,    // Fast-Hessian scale space
+    GRP_LANDMARKS = 1u << 13,  // stereoLandmarks packing
+    GRP_PYRAMID = 1u << 14,    // multi-level ORB
+};
+
+// Every device buffer of a ctx, declared once: X(element type, name, scope, group, elements per unit).  The element count is
+// an expression of the Geom `g`: at the capacity geometry (fe_config.max_*) it sizes the allocation, at the resident geometry
+// it is the stride by which a view of images [first, ...) offsets the buffer.  Buffers, allocation, views and teardown are
+// all generated from this list.
+#define FE_BUFFERS(X) \
+    X(uint8_t, img, PER_IMAGE, GRP_CORE, g.img_stride)             /* [h][pitch] */ \
+    X(uint8_t, blur, PER_IMAGE, GRP_CORE, g.img_stride)            /* same layout */ \
+    X(uint8_t, respmap, PER_IMAGE, GRP_CORE, g.img_stride)         /* same layout: NMS-surviving FAST responses (s - t), 0 elsewhere */ \
+    X(uint32_t, slab, PER_IMAGE, GRP_CORE, g.slab_img)             /* per strip (StripView) records score<<24 | ylocal<<16 | x */ \
+    X(uint32_t, strip_raw, PER_IMAGE, GRP_CORE, g.n_strips)        /* candidates emitted per strip */ \
+    X(uint32_t, strip_sel, PER_IMAGE, GRP_CORE, g.n_strips)        /* survivors of the top-N cut per strip */ \
+    X(uint32_t, hist, PER_IMAGE, GRP_CORE, 256)                    /* response histogram (inside the border) */ \
+    X(uint32_t, n_kp, PER_IMAGE, GRP_CORE, 1)                      /* keypoints found (may exceed kp_cap) */ \
+    X(uint32_t, n_override, PER_IMAGE, GRP_CORE, 1)                /* counts for externally supplied kps */ \
+    X(int, thr_img, PER_IMAGE, GRP_CORE, 1)                        /* per-image FAST thresholds (grid detector) */ \
+    X(int, rowstart, PER_IMAGE, GRP_CORE, g.rs_h + 2)              /* first keypoint whose floor(y) >= row (raster-ordered lists) */ \
+    X(int8_t, pattern, PER_CTX, GRP_CORE, 1024)                    /* [512][2] rBRIEF points when patch size != 31 or WTA_K != 2 (else the built-in table) */ \
+    X(int, umax, PER_CTX, GRP_CORE, 128)                           /* OpenCV's umax table of the general orientation kernel */ \
+    X(uint32_t, kp_key, PER_IMAGE, GRP_CORE, g.kp_cap)             /* (y<<16 | x), ascending = raster order */ \
+    X(uint8_t, kp_score, PER_IMAGE, GRP_CORE, g.kp_cap) \
+    X(fe_kpoint, kp, PER_IMAGE, GRP_CORE, g.kp_cap)                /* wire layout */ \
+    X(float, kx, PER_IMAGE, GRP_CORE, g.kp_cap) \
+    X(float, ky, PER_IMAGE, GRP_CORE, g.kp_cap) \
+    X(float2, kcs, PER_IMAGE, GRP_CORE, g.kp_cap)                  /* (cos, sin) of the steering angle */ \
+    X(uint8_t, desc, PER_IMAGE, GRP_CORE, 32 * g.kp_cap) \
+    X(uint32_t, best, PER_PAIR, GRP_CORE, g.kp_cap)                /* matching keys (distance << 16 | index) */ \
+    X(uint32_t, second, PER_PAIR, GRP_CORE, g.kp_cap) \
+    X(uint32_t, allbest, PER_PAIR, GRP_CORE, g.kp_cap) \
+    X(uint32_t, colbest, PER_PAIR, GRP_CORE, g.kp_cap) \
+    X(fe_match, match_a, PER_PAIR, GRP_CORE, g.kp_cap) \
+    X(fe_match, match_b, PER_PAIR, GRP_CORE, g.kp_cap) \
+    X(uint32_t, n_a, PER_PAIR, GRP_CORE, 1) \
+    X(uint32_t, n_b, PER_PAIR, GRP_CORE, 1) \
+    X(float, fdesc, PER_IMAGE, GRP_FLOAT, 128 * g.kp_cap)          /* rows of 128 floats (SURF-64 uses the first 64) */ \
+    X(unsigned long long, best64, PER_PAIR, GRP_FLOAT, g.kp_cap)   /* L2 keys: float bits of d^2 << 32 | index */ \
+    X(unsigned long long, second64, PER_PAIR, GRP_FLOAT, g.kp_cap) \
+    X(unsigned long long, allbest64, PER_PAIR, GRP_FLOAT, g.kp_cap) \
+    X(unsigned long long, colbest64, PER_PAIR, GRP_FLOAT, g.kp_cap) \
+    X(uint16_t, bf16desc, PER_IMAGE, GRP_FLOAT, round_up(div_up(g.kp_cap, 128), 2) * 128 * 160)  /* bf16 UMMA operands: [tiles][dim/8 + 4][128][8] */ \
+    X(float, fnorm, PER_IMAGE, GRP_FLOAT, round_up(div_up(g.kp_cap, 128), 2) * 128)             /* |x|^2 per row: [tiles * 128] */ \
+    X(uint32_t, cand, PER_PAIR, GRP_FLOAT, 8 * g.kp_cap)           /* [2][kp_cap][4] per-row candidates */ \
+    X(int, tc_error, PER_CTX, GRP_FLOAT, 1)                        /* tcgen05 completion-barrier timeout flag */ \
+    X(int32_t, integral, PER_IMAGE, GRP_INTEGRAL, (size_t)(g.h + 1) * (g.w + 1))   /* CV_32S integral image */ \
+    X(unsigned long long, vf_candL, PER_PAIR, GRP_VERIFY, g.kp_cap)   /* band candidates */ \
+    X(unsigned long long, vf_candR, PER_PAIR, GRP_VERIFY, g.kp_cap) \
+    X(float, vf_limq, PER_PAIR, GRP_VERIFY, round_up(g.kp_cap, 128))  /* thresholds */ \
+    X(float, vf_limt, PER_PAIR, GRP_VERIFY, round_up(g.kp_cap, 128)) \
+    X(float, vf_limqd, PER_PAIR, GRP_VERIFY, round_up(g.kp_cap, 128)) \
+    X(float, vf_limtd, PER_PAIR, GRP_VERIFY, round_up(g.kp_cap, 128)) \
+    X(uint32_t, vf_list, PER_PAIR, GRP_VERIFY, l2_verify_list_entries(g.kp_cap))   /* flagged-element lists */ \
+    X(uint32_t, vf_npush, PER_PAIR, GRP_VERIFY, 1) \
+    X(uint32_t, vf_maxnorm, PER_IMAGE, GRP_VERIFY, 1) \
+    X(uint32_t, cx_bestL, PER_PAIR, GRP_CROSS, g.kp_cap)           /* band candidates */ \
+    X(uint32_t, cx_bestR, PER_PAIR, GRP_CROSS, g.kp_cap) \
+    X(uint32_t, cx_dummy, PER_PAIR, GRP_CROSS, g.kp_cap) \
+    X(int, cx_thrq, PER_PAIR, GRP_CROSS, g.kp_cap)                 /* thresholds */ \
+    X(int, cx_thrt, PER_PAIR, GRP_CROSS, g.kp_cap) \
+    X(uint16_t, cx_qperm, PER_PAIR, GRP_CROSS, g.kp_cap)           /* easy / hard partitions */ \
+    X(uint16_t, cx_tperm, PER_PAIR, GRP_CROSS, g.kp_cap) \
+    X(uint32_t, cx_n, PER_PAIR, GRP_CROSS, 8)                      /* class sizes A, B, C of the queries, then of the trains */ \
+    X(uint16_t, cx_half, PER_PAIR, GRP_CROSS, g.kp_cap <= MIH_MAX ? 32 * g.kp_cap : 0)   /* [2][16][kp_cap] halves in permutation order */ \
+    X(uint16_t, cx_star, PER_PAIR, GRP_CROSS, g.kp_cap <= MIH_MAX ? 2 * g.kp_cap : 0)    /* [2][kp_cap] own candidate */ \
+    X(float, harris, PER_IMAGE, GRP_HARRIS, g.kp_cap)              /* Harris responses */ \
+    X(uint8_t, brief_desc, PER_IMAGE, GRP_BRIEF, 64 * g.kp_cap)    /* rows 64 bytes apart */ \
+    X(int8_t, brief_tab, PER_CTX, GRP_BRIEF_TAB, 3 * 512 * 4)      /* [BRIEF-16 / 32 / 64][bytes * 8][4] (y1, x1, y2, x2) tests */ \
+    X(float, freak_tab, PER_CTX, GRP_FREAK, 64 * 256 * 43 * 3)     /* [scale][orientation][point] (x, y, sigma) */ \
+    X(int4, freak_opairs, PER_CTX, GRP_FREAK, 45)                  /* (i, j, weight_dx, weight_dy) */ \
+    X(uchar2, freak_dpairs, PER_CTX, GRP_FREAK, 512)               /* (i, j) */ \
+    X(int32_t, freak_scale, PER_IMAGE, GRP_FREAK, g.kp_cap)        /* scale index per keypoint */ \
+    /* WindowMatcher sequence: landmark lists as virtual pairs (cur = slot 2v, prev = slot 2v + 1) */ \
+    X(uint8_t, wdesc, PER_IMAGE, GRP_WINDOW, 32 * g.kp_cap) \
+    X(float, wkx, PER_IMAGE, GRP_WINDOW, g.kp_cap) \
+    X(float, wky, PER_IMAGE, GRP_WINDOW, g.kp_cap) \
+    X(uint32_t, wcount, PER_IMAGE, GRP_WINDOW, 1) \
+    X(uint32_t, wbest, PER_PAIR, GRP_WINDOW, g.kp_cap) \
+    X(uint32_t, wsecond, PER_PAIR, GRP_WINDOW, g.kp_cap) \
+    X(fe_match, wmatch, PER_PAIR, GRP_WINDOW, g.kp_cap) \
+    X(uint32_t, wn, PER_PAIR, GRP_WINDOW, 1) \
+    X(double, wq, PER_CTX, GRP_WINDOW, 16) \
+    X(double, wxyz, PER_PAIR, GRP_WINDOW, 3 * g.kp_cap) \
+    X(uint8_t, wdesc_r, PER_IMAGE, GRP_WLIVE, 32 * g.kp_cap)       /* right descriptors of the landmarks */ \
+    X(uint32_t, wbest_r, PER_PAIR, GRP_WLIVE, g.kp_cap)            /* row / column arg-mins of the right-descriptor cross-check */ \
+    X(uint32_t, wcol_r, PER_PAIR, GRP_WLIVE, g.kp_cap) \
+    /* fe_window_update: the current (slot 0) and previous (slot 1) frame's landmark lists */ \
+    X(fe_kpoint, wu_kp, PER_CTX, GRP_WUPDATE, 2 * g.kp_cap) \
+    X(uint8_t, wu_desc, PER_CTX, GRP_WUPDATE, 64 * g.kp_cap) \
+    X(uint8_t, wu_rdesc, PER_CTX, GRP_WUPDATE, 64 * g.kp_cap) \
+    X(float, wu_kx, PER_CTX, GRP_WUPDATE, 2 * g.kp_cap) \
+    X(float, wu_ky, PER_CTX, GRP_WUPDATE, 2 * g.kp_cap) \
+    X(float2, wu_kcs, PER_CTX, GRP_WUPDATE, 2 * g.kp_cap)          /* scratch of the keypoint unpack */ \
+    X(uint32_t, wu_n, PER_CTX, GRP_WUPDATE, 2) \
+    /* Fast-Hessian scale space: [image of the pass][all layers back to back] */ \
+    X(float, hes_det, PER_CTX, GRP_SURFDET, (size_t)std::min(g.n_images, HESSIAN_CHUNK_IMAGES) * g.w * g.h * 20) \
+    X(float, hes_trace, PER_CTX, GRP_SURFDET, (size_t)std::min(g.n_images, HESSIAN_CHUNK_IMAGES) * g.w * g.h * 20) \
+    X(uint32_t, hes_count, PER_CTX, GRP_SURFDET, 2 * g.n_images)   /* [n_images] accepted maxima, then [n_images] largest size (float bits) */ \
+    X(fe_kpoint, hes_kp, PER_IMAGE, GRP_SURFDET, g.kp_cap)         /* unsorted maxima */ \
+    X(fe_kpoint, lm_lkp, PER_PAIR, GRP_LANDMARKS, g.kp_cap) \
+    X(fe_kpoint, lm_rkp, PER_PAIR, GRP_LANDMARKS, g.kp_cap) \
+    X(uint8_t, lm_ldesc, PER_PAIR, GRP_LANDMARKS, 32 * g.kp_cap) \
+    X(uint8_t, lm_rdesc, PER_PAIR, GRP_LANDMARKS, 32 * g.kp_cap) \
+    X(fe_match, lm_match, PER_PAIR, GRP_LANDMARKS, g.kp_cap) \
+    /* multi-level ORB: two ping-pong level images (level-1 geometry is the largest), coefficient table, accumulated results */ \
+    X(uint8_t, pyr_img0, PER_IMAGE, GRP_PYRAMID, g.img_stride) \
+    X(uint8_t, pyr_img1, PER_IMAGE, GRP_PYRAMID, g.img_stride) \
+    X(int, pyr_tab, PER_CTX, GRP_PYRAMID, 2 * (g.w + g.h)) \
+    X(fe_kpoint, pyr_kp, PER_IMAGE, GRP_PYRAMID, g.kp_cap) \
+    X(uint8_t, pyr_desc, PER_IMAGE, GRP_PYRAMID, 32 * g.kp_cap) \
+    X(uint32_t, pyr_n, PER_IMAGE, GRP_PYRAMID, 1)
+
 struct Buffers {
-    uint8_t *img = nullptr;        // [n_images][h][pitch]
-    uint8_t *blur = nullptr;       // same layout
-    uint8_t *respmap = nullptr;    // same layout: NMS-surviving FAST responses (s - t), 0 elsewhere
-    uint32_t *slab = nullptr;      // [n_images][slab_img]: per strip (StripView) records score<<24 | ylocal<<16 | x
-    uint32_t *strip_raw = nullptr; // [n_images][n_strips] candidates emitted per strip
-    uint32_t *strip_sel = nullptr; // [n_images][n_strips] survivors of the top-N cut per strip
-    uint32_t *hist = nullptr;      // [n_images][256] response histogram (inside the border)
-    uint32_t *n_kp = nullptr;      // [n_images] keypoints found (may exceed kp_cap)
-    uint32_t *kp_key = nullptr;    // [n_images][kp_cap]  (y<<16 | x), ascending = raster order
-    uint8_t *kp_score = nullptr;   // [n_images][kp_cap]
-    float *harris = nullptr;       // [n_images][kp_cap] Harris responses (cv::ORB HARRIS_SCORE), lazily allocated
-    fe_kpoint *kp = nullptr;       // [n_images][kp_cap]  wire layout
-    float *kx = nullptr, *ky = nullptr;   // [n_images][kp_cap]
-    float2 *kcs = nullptr;         // [n_images][kp_cap]  (cos, sin) of the steering angle
-    uint8_t *desc = nullptr;       // [n_images][kp_cap][32]
-    float *fdesc = nullptr;        // [n_images][kp_cap][128] float descriptors (SURF), lazily allocated
-    int32_t *integral = nullptr;   // [n_images][(h+1)][(w+1)] CV_32S integral image (SURF orientation), lazy
-    // matching, per pair (image 2p = query/left, 2p+1 = train/right)
-    uint32_t *best = nullptr, *second = nullptr, *allbest = nullptr, *colbest = nullptr; // [n_pairs][kp_cap]
-    unsigned long long *best64 = nullptr, *second64 = nullptr, *allbest64 = nullptr, *colbest64 = nullptr;  // L2 keys, lazy
-    // tensor-core L2 path, lazy: bf16 operands in UMMA core-matrix layout, |x|^2, per-row candidates, error flag
-    uint16_t *bf16desc = nullptr;  // [n_images][tiles][dim/8][128][8]
-    float *fnorm = nullptr;        // [n_images][tiles * 128]
-    uint32_t *cand = nullptr;      // [n_pairs][2][kp_cap][4]
-    int *tc_error = nullptr;
-    // exact tensor-core cross-check (l2verify.cu), lazy: band candidates, thresholds, flagged-element lists
-    unsigned long long *vf_candL = nullptr, *vf_candR = nullptr;    // [n_pairs][kp_cap]
-    float *vf_limq = nullptr, *vf_limt = nullptr, *vf_limqd = nullptr, *vf_limtd = nullptr;   // [n_pairs][round_up(kp_cap, 128)]
-    uint32_t *vf_list = nullptr, *vf_npush = nullptr, *vf_maxnorm = nullptr;   // [n_pairs][32 kp_cap], [n_pairs], [n_images]
-    fe_match *match_a = nullptr, *match_b = nullptr;   // [n_pairs][kp_cap]
-    uint32_t *n_a = nullptr, *n_b = nullptr;           // [n_pairs]
-    int *rowstart = nullptr;                           // [n_images][rs_h + 2] first keypoint whose floor(y) >= row (raster-ordered lists)
-    uint32_t *n_override = nullptr;                    // [n_images] counts for externally supplied kps
-    int *thr_img = nullptr;                            // [n_images] per-image FAST thresholds (grid detector)
-    int *umax = nullptr;                               // [128] OpenCV's umax table of the general orientation kernel
-    int8_t *brief_pat = nullptr;                       // [512][4] (y1, x1, y2, x2) tests of cv::BriefDescriptorExtractor, lazy
-    uint8_t *brief_desc = nullptr;                     // [n_images][kp_cap][64] BRIEF-16 / 32 / 64 rows, lazy
-    int8_t *pattern = nullptr;                         // [512][2] rBRIEF points when patch size != 31 or WTA_K != 2 (else the built-in table)
-    // WindowMatcher sequence buffers, lazy: landmark lists as virtual pairs (cur = slot 2v, prev = slot 2v + 1)
-    uint8_t *wdesc = nullptr;      // [n_images][kp_cap][32]
-    float *wkx = nullptr, *wky = nullptr;              // [n_images][kp_cap]
-    uint32_t *wcount = nullptr;                        // [n_images]
-    uint32_t *wbest = nullptr, *wsecond = nullptr;     // [n_pairs][kp_cap]
-    fe_match *wmatch = nullptr;                        // [n_pairs][kp_cap]
-    uint32_t *wn = nullptr;                            // [n_pairs]
-    double *wq = nullptr, *wxyz = nullptr;             // [16], [n_pairs][kp_cap][3]
-    uint8_t *wdesc_r = nullptr;                        // [n_images][kp_cap][32] right descriptors of the landmarks (liveGraph mode), lazy
-    uint32_t *wbest_r = nullptr, *wcol_r = nullptr;    // [n_pairs][kp_cap] row / column arg-mins of the right-descriptor cross-check
-    // fe_window_update: the current (slot 0) and previous (slot 1) frame's landmark lists, lazy
-    fe_kpoint *wu_kp = nullptr;                        // [2][kp_cap]
-    uint8_t *wu_desc = nullptr, *wu_rdesc = nullptr;   // [2][kp_cap][32]
-    float *wu_kx = nullptr, *wu_ky = nullptr;          // [2][kp_cap]
-    float2 *wu_kcs = nullptr;                          // [2][kp_cap] (scratch of the keypoint unpack)
-    uint32_t *wu_n = nullptr;                          // [2]
-    // pruned cross-check, lazy: band candidates, thresholds, easy / hard partitions
-    uint32_t *cx_bestL = nullptr, *cx_bestR = nullptr, *cx_dummy = nullptr;   // [n_pairs][kp_cap]
-    int *cx_thrq = nullptr, *cx_thrt = nullptr;                                // [n_pairs][kp_cap]
-    uint16_t *cx_qperm = nullptr, *cx_tperm = nullptr;                         // [n_pairs][kp_cap]
-    uint32_t *cx_n = nullptr;                                                  // [n_pairs][8]: class sizes A, B, C of the queries, then of the trains
-    uint16_t *cx_half = nullptr, *cx_star = nullptr;   // [n_images][16][kp_cap] halves in permutation order, [n_images][kp_cap] own candidate
-    // Fast-Hessian scale space (single image), lazy
-    float *hes_det = nullptr, *hes_trace = nullptr;    // [image chunk][all layers back to back]
-    uint32_t *hes_count = nullptr;                     // [n_images] accepted maxima, then [n_images] largest size (float bits)
-    fe_kpoint *hes_kp = nullptr;                       // [n_images][kp_cap] unsorted maxima
-    // stereoLandmarks packing, lazy
-    fe_kpoint *lm_lkp = nullptr, *lm_rkp = nullptr;    // [n_pairs][kp_cap]
-    uint8_t *lm_ldesc = nullptr, *lm_rdesc = nullptr;  // [n_pairs][kp_cap][32]
-    fe_match *lm_match = nullptr;                      // [n_pairs][kp_cap]
-    // multi-level ORB, lazy: two ping-pong level images, coefficient table, accumulated results
-    uint8_t *pyr_img[2] = {nullptr, nullptr};          // [n_images][h1][pitch1] (level-1 geometry is the largest)
-    int *pyr_tab = nullptr;                            // [2 * (max_width + max_height)]
-    fe_kpoint *pyr_kp = nullptr;                       // [n_images][kp_cap]
-    uint8_t *pyr_desc = nullptr;                       // [n_images][kp_cap][32]
-    uint32_t *pyr_n = nullptr;                         // [n_images]
+#define FE_BUFFER_FIELD(T, name, scope, group, n) T *name = nullptr;
+    FE_BUFFERS(FE_BUFFER_FIELD)
+#undef FE_BUFFER_FIELD
 };
 
 // The strip layout the FAST kernel of this (geometry, parameters) writes and the top-N selection reads: strip s of an image

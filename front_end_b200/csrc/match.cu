@@ -713,7 +713,6 @@ int launch_finalize_cross_both(const Geom &g, int n_pairs, const uint32_t *count
 constexpr int CX_T = 24;             // B / C split of the LB scan (the LB4 filter stops paying above it)
 constexpr int CX_T2 = 48;            // C / D split: the two-POPC LB8 filter serves thresholds up to here, class D is evaluated in full
 constexpr int CX_T1 = 15;            // A / B split: 16 halves, at most 15 differing bits -> one half is identical
-constexpr int MIH_MAX = 16384;       // largest per-image keypoint capacity the shared-memory hash table serves (2 x cap x 4 B = 128 KB)
 
 __global__ void __launch_bounds__(1024)
 cross_classify_kernel(Geom g, int t1, int t2, int t3, const uint32_t *__restrict__ counts, const uint32_t *__restrict__ bestL,

@@ -215,18 +215,9 @@ DetectParams detect_params(const fe_ctx *c) {
     p.nonmax = c->cfg.nonmax;
     p.n_features = c->cfg.n_features;
     p.edge = c->cfg.edge_threshold;
+    p.patch_size = c->patch_size;
+    p.wta_k = c->wta_k;
     return p;
-}
-
-// The default ORB geometry (31-px patch, keypoints >= 19 px from the border) runs the staged / dp4a fast kernels; any other
-// patch size or a smaller edgeThreshold runs the general kernels, which follow cv::ORB's bordered-pyramid reads
-// (raw reflect-101 pixels outside the image).
-int general_half(const fe_ctx *c) { return (c->patch_size != 31 || c->cfg.edge_threshold < 16) ? c->patch_size / 2 : 0; }
-
-// rBRIEF variant of this ctx: learned 31-px pattern (staged fast path), generated pattern, or WTA_K 3 / 4 tuples
-int brief_dispatch(const fe_ctx *c, const Geom &g, const Buffers &b, const uint32_t *counts, cudaStream_t st) {
-    if (c->wta_k != 2) return launch_brief_wta(g, b, counts, c->wta_k, st);
-    return (c->patch_size == 31 && c->cfg.edge_threshold >= 19) ? launch_brief(g, b, counts, st) : launch_brief_general(g, b, counts, st);
 }
 
 // Upload n contiguous host images (row stride `stride`) into device image slots first, first+step, ...
@@ -263,18 +254,17 @@ int run_detect_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, b
     { StageTimer t(c, ST_SELECT, st, timed); t.done(launch_select(g, p, b, st)); }
     if (harris) { StageTimer t(c, ST_SELECT, st, timed); t.done(launch_harris_select(g, n_final, b, st)); }
     // default ORB geometry: orientation and rBRIEF in one pass over image tiles, after the blur (which needs no keypoints)
-    if (describe && c->cfg.orientation && c->patch_size == 31 && c->cfg.edge_threshold >= 19 && c->wta_k == 2 && !harris) {
+    if (describe && c->cfg.orientation && !harris && describe_tile_fits(p)) {
         { StageTimer t(c, ST_BLUR, st, timed); t.done(launch_blur(g, b, st)); }
-        { StageTimer t(c, ST_BRIEF, st, timed); t.done(launch_describe_tile(g, p, b, (float)c->patch_size, st)); }
+        { StageTimer t(c, ST_BRIEF, st, timed); t.done(launch_describe_tile(g, p, b, st)); }
         FE_CUDA(c, cudaGetLastError());
         return FE_OK;
     }
-    { StageTimer t(c, ST_ORIENT, st, timed);
-      t.done(launch_orient_pack(g, p, b, c->cfg.orientation != 0, c->cfg.orientation ? (float)c->patch_size : 7.f, general_half(c), st)); }
+    { StageTimer t(c, ST_ORIENT, st, timed); t.done(launch_orient(g, p, b, c->cfg.orientation != 0, st)); }
     if (harris) { StageTimer t(c, ST_ORIENT, st, timed); t.done(launch_harris_store(g, b, st)); }
     if (describe) {
         { StageTimer t(c, ST_BLUR, st, timed); t.done(launch_blur(g, b, st)); }
-        { StageTimer t(c, ST_BRIEF, st, timed); t.done(brief_dispatch(c, g, b, b.n_kp, st)); }
+        { StageTimer t(c, ST_BRIEF, st, timed); t.done(launch_rbrief(g, p, b, b.n_kp, st)); }
     }
     FE_CUDA(c, cudaGetLastError());
     return FE_OK;
@@ -344,11 +334,11 @@ int run_detect_pyramid(fe_ctx *c, bool describe) {
         { StageTimer t(c, ST_FAST); t.done(launch_fast(gl, p, v, c->stream)); }
         { StageTimer t(c, ST_SELECT); t.done(launch_select(gl, p, v, c->stream)); }
         if (harris) { StageTimer t(c, ST_SELECT); t.done(launch_harris_select(gl, quota[l], v, c->stream)); }
-        { StageTimer t(c, ST_ORIENT); t.done(launch_orient_pack(gl, p, v, true, (float)c->patch_size, general_half(c), c->stream)); }
+        { StageTimer t(c, ST_ORIENT); t.done(launch_orient(gl, p, v, true, c->stream)); }
         if (harris) { StageTimer t(c, ST_ORIENT); t.done(launch_harris_store(gl, v, c->stream)); }
         if (describe) {
             { StageTimer t(c, ST_BLUR); t.done(launch_blur(gl, v, c->stream)); }
-            { StageTimer t(c, ST_BRIEF); t.done(brief_dispatch(c, gl, v, v.n_kp, c->stream)); }
+            { StageTimer t(c, ST_BRIEF); t.done(launch_rbrief(gl, p, v, v.n_kp, c->stream)); }
         }
         { StageTimer t(c, ST_SELECT);
           t.done(launch_pyr_append(gl, l, scale, (float)c->patch_size * scale, v, b.pyr_kp, b.pyr_desc, b.pyr_n, describe, c->stream)); }
@@ -867,10 +857,11 @@ int32_t fe_grid_detect(fe_ctx *c, const uint8_t *img, int32_t w, int32_t h, int3
         t.done(0);
     }
     DetectParams p;
-    p.threshold = 0; p.ps = ps; p.nonmax = 1; p.n_features = -1; p.edge = 0; p.thr_img = c->b.thr_img;
+    p.threshold = 0; p.ps = ps; p.nonmax = 1; p.n_features = -1; p.edge = 0; p.patch_size = c->patch_size; p.wta_k = c->wta_k;
+    p.thr_img = c->b.thr_img;
     { StageTimer t(c, ST_FAST); t.done(launch_fast(g, p, c->b, c->stream)); }
     { StageTimer t(c, ST_SELECT); t.done(launch_select(g, p, c->b, c->stream)); }
-    { StageTimer t(c, ST_ORIENT); t.done(launch_orient_pack(g, p, c->b, false, 7.f, 0, c->stream)); }
+    { StageTimer t(c, ST_ORIENT); t.done(launch_orient(g, p, c->b, false, c->stream)); }
     SubpixParams sp{};
     for (int k = 0; k < nc; ++k) {
         const int cx = (k % cols) * cw, cy = (k / cols) * ch;       // gridROI.x / .y (relative to the ROI)
@@ -1243,7 +1234,7 @@ int32_t fe_describe(fe_ctx *c, const uint8_t *img, int32_t w, int32_t h, int32_t
       t.done(0); }
     { StageTimer t(c, ST_ORIENT); t.done(launch_unpack_kps(c->g, c->b, c->b.n_override, c->stream)); }
     { StageTimer t(c, ST_BLUR); t.done(launch_blur(c->g, c->b, c->stream)); }
-    { StageTimer t(c, ST_BRIEF); t.done(brief_dispatch(c, c->g, c->b, c->b.n_override, c->stream)); }
+    { StageTimer t(c, ST_BRIEF); t.done(launch_rbrief(c->g, detect_params(c), c->b, c->b.n_override, c->stream)); }
     FE_CUDA(c, cudaGetLastError());
     FE_CUDA(c, cudaMemcpyAsync(desc, c->b.desc, (size_t)32 * m, cudaMemcpyDeviceToHost, c->stream));
     return sync_and_resolve(c);

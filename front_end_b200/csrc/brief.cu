@@ -40,9 +40,9 @@ brief_kernel(const int32_t *__restrict__ integ, Geom g, const uint32_t *__restri
         const int cy = (int)((double)key.y + 0.5), cx = (int)((double)key.x + 0.5);
         float r0 = 0.f, r1 = 1.f;
         if (use_orientation) {
-            const float a = __fmul_rn(key.angle, (float)(3.14159265358979323846 / 180.0));
-            r0 = (float)sin((double)a);
-            r1 = (float)cos((double)a);
+            const float2 cs = steer(key.angle);
+            r0 = cs.y;
+            r1 = cs.x;
         }
         uint32_t *dst = reinterpret_cast<uint32_t *>(out + ((size_t)image * g.kp_cap + k) * 64);
         for (int base = 0; base < n_tests; base += 32) {

@@ -45,8 +45,17 @@ struct DetectParams {
     int nonmax;
     int n_features;        // < 0: keep all
     int edge;              // border filter
+    int patch_size;        // ORB patchSize: intensity-centroid disc diameter and rBRIEF pattern
+    int wta_k;             // ORB WTA_K
     const int *thr_img = nullptr;   // device, optional: per-image FAST thresholds (grid cells: live_stereo.cpp:293,306)
 };
+
+// cv::ORB's steering of a keypoint (orb.cpp): angle = kpt.angle * (float)(CV_PI/180.f), then (float)cos / (float)sin of it
+// in double.  Returns (cos, sin).
+__device__ __forceinline__ float2 steer(float angle_deg) {
+    const float th = __fmul_rn(angle_deg, (float)(3.14159265358979323846 / 180.0));
+    return make_float2((float)cos((double)th), (float)sin((double)th));
+}
 
 // cv::fastAtan2 (degrees).  Host+device so the exact polynomial can be unit-tested on the CPU.
 __host__ __device__ inline float fast_atan2_deg(float y, float x) {
@@ -256,12 +265,16 @@ StripView strip_view(const Geom &g, const DetectParams &p);
 // ---- kernel launchers (each returns the number of kernels it launched) -------------------------
 int launch_fast(const Geom &g, const DetectParams &p, const Buffers &b, cudaStream_t s);
 int launch_select(const Geom &g, const DetectParams &p, const Buffers &b, cudaStream_t s);
-int launch_orient_pack(const Geom &g, const DetectParams &p, const Buffers &b, bool orientation,
-                       float kp_size, int half_patch, cudaStream_t s);
+// Wire keypoints, kx / ky and the steering of the selected keypoints; with orientation, the intensity-centroid angle of
+// p.patch_size (the kernel follows from p.patch_size and p.edge, orb.cu)
+int launch_orient(const Geom &g, const DetectParams &p, const Buffers &b, bool orientation, cudaStream_t s);
 int launch_blur(const Geom &g, const Buffers &b, cudaStream_t s);
-// orientation + wire keypoints + rBRIEF-256 of the default ORB geometry (31-px patch, edgeThreshold >= 19, WTA_K 2, FAST score)
-// per image tile, from b.img and b.blur: writes what launch_orient_pack and launch_brief write
-int launch_describe_tile(const Geom &g, const DetectParams &p, const Buffers &b, float kp_size, cudaStream_t s);
+// Whether launch_describe_tile serves the geometry of p (patch size, edgeThreshold, WTA_K).  The caller still requires
+// orientation, descriptors and the FAST score.
+bool describe_tile_fits(const DetectParams &p);
+// orientation + wire keypoints + rBRIEF-256 per image tile, from b.img and b.blur: writes what launch_orient and launch_rbrief
+// write
+int launch_describe_tile(const Geom &g, const DetectParams &p, const Buffers &b, cudaStream_t s);
 // cv::ORB HARRIS_SCORE (harris.cu): score the selected FAST corners, keep the n_features best (ties kept, raster order);
 // then, after the keypoints are packed, store the score as their response
 int launch_harris_select(const Geom &g, int n_features, const Buffers &b, cudaStream_t s);
@@ -281,11 +294,9 @@ struct SubpixParams {
     float epsilon;           // 0.001
 };
 int launch_subpix(const Geom &g, const Buffers &b, const uint32_t *counts, const SubpixParams &sp, cudaStream_t s);
-int launch_brief(const Geom &g, const Buffers &b, const uint32_t *counts, cudaStream_t s);
-// rBRIEF with the ctx's own pattern (b.pattern; ORB::setPatchSize != 31), reflect-101 raw pixels outside the image
-int launch_brief_general(const Geom &g, const Buffers &b, const uint32_t *counts, cudaStream_t s);
-// ORB WTA_K = 3 / 4: 128 tuples of wta_k points from b.pattern, two bits per tuple
-int launch_brief_wta(const Geom &g, const Buffers &b, const uint32_t *counts, int wta_k, cudaStream_t s);
+// ORB descriptors of the keypoints in b.kx / b.ky / b.kcs from b.blur (and b.img outside the image): rBRIEF-256 for WTA_K 2,
+// 128 tuples of WTA_K points from b.pattern otherwise (the kernel follows from p.patch_size, p.edge and p.wta_k, orb.cu)
+int launch_rbrief(const Geom &g, const DetectParams &p, const Buffers &b, const uint32_t *counts, cudaStream_t s);
 int launch_unpack_kps(const Geom &g, const Buffers &b, const uint32_t *counts, cudaStream_t s);
 // cv::BriefDescriptorExtractor(bytes) at the keypoints in b.kp with the caller's test table (brief.cu); needs b.integral.
 // out rows are 64 bytes apart (bytes used)

@@ -27,12 +27,13 @@ __device__ __forceinline__ int reflect101(int i, int n) {
     return i;
 }
 
-__constant__ int c_ori_umax[16] = {15, 15, 15, 15, 14, 14, 14, 13, 13, 12, 11, 10, 9, 8, 6, 3};   // OpenCV's umax, radius 15
-
+constexpr int ORB_PATCH = 31;               // ORB's default patchSize: bit_pattern_31_ and the radius-15 intensity-centroid disc
+constexpr int ORI_R = ORB_PATCH / 2;
 constexpr int ORI_WARPS = 8;
 constexpr int ORI_KPW = 8;                  // keypoints per warp (amortises the weight-table copy)
 constexpr int ORI_WORDS = 9;                // 31 columns + up to 3 alignment bytes -> 9 words per patch row
-constexpr int ORI_SLOTS = 31 * ORI_WORDS;   // 279 (row, word) slots per keypoint, 9 rounds of 32 lanes
+constexpr int ORI_SLOTS = ORB_PATCH * ORI_WORDS;   // 279 (row, word) slots per keypoint, 9 rounds of 32 lanes
+constexpr int ORI_K = (ORI_SLOTS + 31) / 32;       // slots per lane
 
 __device__ __forceinline__ int dp4a_u8s8(uint32_t a, uint32_t b, int c) {
     int d;
@@ -40,48 +41,99 @@ __device__ __forceinline__ int dp4a_u8s8(uint32_t a, uint32_t b, int c) {
     return d;
 }
 
-// One warp per keypoint.  The radius-15 disc is read as aligned 32-bit words (31 rows x 9 words, coalesced per
-// row) instead of 709 byte gathers, and the moments are integer dot products: for word slot (row v, word w) and
-// alignment off = (x - 15) & 3, byte b is column u = 4w + b - off - 15; the tables hold u (as s8, 0 outside the
-// disc |u| <= umax[|v|]) and the 0/1 membership mask, so  m10 += dp4a(word, U)  and  m01 += v * dp4a(word, M).
-// Integer arithmetic: the moments are bit-identical to the byte loop.  Writes the wire-format keypoint, float
-// coordinates and the steering (cos, sin).
+// The radius-15 disc is read as aligned 32-bit words (31 rows x 9 words) instead of 709 byte gathers, and the moments are
+// integer dot products: for word slot (row v, word w) and alignment off = (x - 15) & 3, byte b is column u = 4w + b - off - 15;
+// the tables hold u (as s8, 0 outside the disc |u| <= umax[|v|]) and the 0/1 membership mask, so  m10 += dp4a(word, U)  and
+// m01 += v * dp4a(word, M).  Integer arithmetic: the moments are bit-identical to the byte loop.  Built at compile time.
+struct __align__(16) OriTables { uint32_t u[4][288], m[4][288]; };
+constexpr OriTables make_ori_tables() {
+    constexpr int umax[ORI_R + 1] = {15, 15, 15, 15, 14, 14, 14, 13, 13, 12, 11, 10, 9, 8, 6, 3};   // OpenCV's umax, radius 15
+    OriTables t{};
+    for (int off = 0; off < 4; ++off)
+        for (int slot = 0; slot < ORI_SLOTS; ++slot) {
+            const int r = slot / ORI_WORDS, w = slot - r * ORI_WORDS;
+            const int v = r - ORI_R, d = umax[v < 0 ? -v : v];
+            for (int b = 0; b < 4; ++b) {
+                const int u = 4 * w + b - off - ORI_R;
+                if (u >= -d && u <= d) { t.u[off][slot] |= (uint32_t)(u & 0xFF) << (8 * b); t.m[off][slot] |= 1u << (8 * b); }
+            }
+        }
+    return t;
+}
+__device__ const OriTables d_ori_tab = make_ori_tables();
+
+// Per-lane slot geometry, the same for every keypoint: slot lane + 32 k is (row r, word w) of the patch, at offset
+// r * row_stride + w * word_stride from its first word, and row v = r - 15 of the disc
+__device__ __forceinline__ void ori_slots(int lane, int row_stride, int word_stride, int (&soff)[ORI_K], int (&sv)[ORI_K]) {
+#pragma unroll
+    for (int k = 0; k < ORI_K; ++k) {
+        const int slot = min(lane + 32 * k, ORI_SLOTS - 1);
+        const int r = slot / ORI_WORDS, w = slot - r * ORI_WORDS;
+        soff[k] = r * row_stride + w * word_stride;
+        sv[k] = r - ORI_R;
+    }
+}
+
+// Intensity-centroid angles (degrees, cv::fastAtan2) of two keypoints, one warp: words(k) gives this lane's words of slot
+// lane + 32 k of both patches (0 past the last slot), whose alignments are off0 and off1; tu / tm are the weight tables
+template <class Words>
+__device__ __forceinline__ float2 ori_angles(Words words, int off0, int off1, const uint32_t (*tu)[288], const uint32_t (*tm)[288],
+                                             const int (&sv)[ORI_K], int lane) {
+    int m10a = 0, m01a = 0, m10b = 0, m01b = 0;
+#pragma unroll
+    for (int k = 0; k < ORI_K; ++k) {
+        const int slot = min(lane + 32 * k, ORI_SLOTS - 1);
+        const uint2 w = words(k);
+        m10a = dp4a_u8s8(w.x, tu[off0][slot], m10a);
+        m01a += sv[k] * dp4a_u8s8(w.x, tm[off0][slot], 0);
+        m10b = dp4a_u8s8(w.y, tu[off1][slot], m10b);
+        m01b += sv[k] * dp4a_u8s8(w.y, tm[off1][slot], 0);
+    }
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+        m10a += __shfl_xor_sync(0xffffffffu, m10a, o);
+        m01a += __shfl_xor_sync(0xffffffffu, m01a, o);
+        m10b += __shfl_xor_sync(0xffffffffu, m10b, o);
+        m01b += __shfl_xor_sync(0xffffffffu, m01b, o);
+    }
+    return make_float2(fast_atan2_deg((float)m01a, (float)m10a), fast_atan2_deg((float)m01b, (float)m10b));
+}
+
+// The detector's keypoint record at index o (cv::KeyPoint of cv::ORB::detect: octave 0, class_id -1, the FAST score as
+// response when reported), its float coordinates and its steering (cos, sin)
+__device__ __forceinline__ void store_keypoint(size_t o, uint32_t key, float angle, float2 cs, float kp_size,
+                                               const uint8_t *__restrict__ kp_score, int report_score, fe_kpoint *__restrict__ kp,
+                                               float *__restrict__ kx, float *__restrict__ ky, float2 *__restrict__ kcs) {
+    const int x = key & 0xFFFF, y = key >> 16;
+    fe_kpoint k;
+    k.x = (float)x; k.y = (float)y; k.size = kp_size; k.angle = angle;
+    k.response = report_score ? (float)kp_score[o] : 0.f;
+    k.octave = 0; k.class_id = -1;
+    kp[o] = k;
+    kx[o] = (float)x; ky[o] = (float)y;
+    kcs[o] = cs;
+}
+
+// One warp per keypoint, the disc's words loaded straight from the image (rows coalesced).  Writes the wire-format keypoint,
+// float coordinates and the steering (cos, sin).
 __global__ void __launch_bounds__(ORI_WARPS * 32)
 orient_pack_kernel(const uint8_t *__restrict__ img, Geom g, const uint32_t *__restrict__ n_kp,
                    const uint32_t *__restrict__ kp_key, const uint8_t *__restrict__ kp_score,
                    int orientation, int report_score, float kp_size, fe_kpoint *__restrict__ kp,
                    float *__restrict__ kx, float *__restrict__ ky, float2 *__restrict__ kcs) {
-    __shared__ uint32_t s_u[4][288], s_m[4][288];
+    __shared__ OriTables s_tab;
     const int image = blockIdx.y;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int n = min((int)n_kp[image], g.kp_cap);
     if (blockIdx.x * (ORI_WARPS * ORI_KPW) >= n) return;
-    if (orientation) {
-        for (int i = threadIdx.x; i < 4 * 288; i += ORI_WARPS * 32) {
-            const int off = i / 288, slot = i - off * 288;
-            uint32_t uw = 0, mw = 0;
-            if (slot < ORI_SLOTS) {
-                const int r = slot / ORI_WORDS, w = slot - r * ORI_WORDS;
-                const int v = r - 15, d = c_ori_umax[v < 0 ? -v : v];
-#pragma unroll
-                for (int b = 0; b < 4; ++b) {
-                    const int u = 4 * w + b - off - 15;
-                    if (u >= -d && u <= d) { uw |= (uint32_t)(u & 0xFF) << (8 * b); mw |= 1u << (8 * b); }
-                }
-            }
-            s_u[off][slot] = uw; s_m[off][slot] = mw;
-        }
+    if (orientation) {          // the moments read the weight tables once per slot: from shared memory
+        for (int i = threadIdx.x; i < (int)(sizeof(OriTables) / 16); i += ORI_WARPS * 32)
+            reinterpret_cast<uint4 *>(&s_tab)[i] = reinterpret_cast<const uint4 *>(&d_ori_tab)[i];
         __syncthreads();
     }
     // per-lane slot geometry is the same for every keypoint: hoist it out of the keypoint loop
-    int soff[(ORI_SLOTS + 31) / 32], sv[(ORI_SLOTS + 31) / 32];
-#pragma unroll
-    for (int k = 0; k < (ORI_SLOTS + 31) / 32; ++k) {
-        const int slot = min(lane + 32 * k, ORI_SLOTS - 1);
-        const int r = slot / ORI_WORDS, w = slot - r * ORI_WORDS;
-        soff[k] = r * g.pitch + 4 * w;
-        sv[k] = r - 15;
-    }
+    int soff[ORI_K], sv[ORI_K];
+    ori_slots(lane, g.pitch, 4, soff, sv);
     // lane `it` keeps keypoint `it` of this warp: the record, the double-precision cos / sin (the long pole of
     // the old kernel when evaluated by one lane per keypoint) and the stores are then done by 8 lanes at once
     uint32_t my_key = 0;
@@ -101,60 +153,29 @@ orient_pack_kernel(const uint8_t *__restrict__ img, Geom g, const uint32_t *__re
         const bool two = i0 + ORI_WARPS < n;
         const uint32_t key0 = __shfl_sync(0xffffffffu, my_key, it);
         const uint32_t key1 = two ? __shfl_sync(0xffffffffu, my_key, it + 1) : key0;
-        float angle0 = -1.f, angle1 = -1.f;
+        float2 angles = make_float2(-1.f, -1.f);
         if (orientation) {
-            const int xl0 = (int)(key0 & 0xFFFF) - 15, xa0 = xl0 & ~3, off0 = xl0 - xa0;
-            const int xl1 = (int)(key1 & 0xFFFF) - 15, xa1 = xl1 & ~3, off1 = xl1 - xa1;
-            const uint8_t *base0 = img + (size_t)image * g.img_stride + (size_t)((int)(key0 >> 16) - 15) * g.pitch + xa0;
-            const uint8_t *base1 = img + (size_t)image * g.img_stride + (size_t)((int)(key1 >> 16) - 15) * g.pitch + xa1;
-            uint32_t wa[(ORI_SLOTS + 31) / 32], wb[(ORI_SLOTS + 31) / 32];
+            const int xl0 = (int)(key0 & 0xFFFF) - ORI_R, xa0 = xl0 & ~3;
+            const int xl1 = (int)(key1 & 0xFFFF) - ORI_R, xa1 = xl1 & ~3;
+            const uint8_t *base0 = img + (size_t)image * g.img_stride + (size_t)((int)(key0 >> 16) - ORI_R) * g.pitch + xa0;
+            const uint8_t *base1 = img + (size_t)image * g.img_stride + (size_t)((int)(key1 >> 16) - ORI_R) * g.pitch + xa1;
+            uint32_t wa[ORI_K], wb[ORI_K];
 #pragma unroll
-            for (int k = 0; k < (ORI_SLOTS + 31) / 32; ++k) {
+            for (int k = 0; k < ORI_K; ++k) {
                 const bool in = lane + 32 * k < ORI_SLOTS;
                 wa[k] = in ? __ldg(reinterpret_cast<const uint32_t *>(base0 + soff[k])) : 0u;
                 wb[k] = in ? __ldg(reinterpret_cast<const uint32_t *>(base1 + soff[k])) : 0u;
             }
-            const uint32_t *tu0 = s_u[off0], *tm0 = s_m[off0], *tu1 = s_u[off1], *tm1 = s_m[off1];
-            int m10a = 0, m01a = 0, m10b = 0, m01b = 0;
-#pragma unroll
-            for (int k = 0; k < (ORI_SLOTS + 31) / 32; ++k) {
-                const int slot = min(lane + 32 * k, ORI_SLOTS - 1);     // words past the last slot are 0
-                m10a = dp4a_u8s8(wa[k], tu0[slot], m10a);
-                m01a += sv[k] * dp4a_u8s8(wa[k], tm0[slot], 0);
-                m10b = dp4a_u8s8(wb[k], tu1[slot], m10b);
-                m01b += sv[k] * dp4a_u8s8(wb[k], tm1[slot], 0);
-            }
-#pragma unroll
-            for (int off2 = 16; off2; off2 >>= 1) {
-                m10a += __shfl_xor_sync(0xffffffffu, m10a, off2);
-                m01a += __shfl_xor_sync(0xffffffffu, m01a, off2);
-                m10b += __shfl_xor_sync(0xffffffffu, m10b, off2);
-                m01b += __shfl_xor_sync(0xffffffffu, m01b, off2);
-            }
-            angle0 = fast_atan2_deg((float)m01a, (float)m10a);
-            angle1 = fast_atan2_deg((float)m01b, (float)m10b);
+            angles = ori_angles([&](int k) { return make_uint2(wa[k], wb[k]); }, xl0 - xa0, xl1 - xa1, s_tab.u, s_tab.m, sv, lane);
         }
-        if (lane == it) my_angle = angle0;
-        if (two && lane == it + 1) my_angle = angle1;
+        if (lane == it) my_angle = angles.x;
+        if (two && lane == it + 1) my_angle = angles.y;
         my_n = two ? it + 2 : it + 1;
     }
     if (lane < my_n) {
         const int i = (blockIdx.x * ORI_KPW + lane) * ORI_WARPS + warp;
-        const size_t o = (size_t)image * g.kp_cap + i;
-        const int x = my_key & 0xFFFF, y = my_key >> 16;
-        float2 cs = make_float2(1.f, 0.f);
-        if (orientation) {
-            // orb.cpp: float angle = kpt.angle * (float)(CV_PI/180.f); a = (float)cos(angle), b = (float)sin(angle)
-            const float th = __fmul_rn(my_angle, (float)(3.14159265358979323846 / 180.0));
-            cs = make_float2((float)cos((double)th), (float)sin((double)th));
-        }
-        fe_kpoint k;
-        k.x = (float)x; k.y = (float)y; k.size = kp_size; k.angle = my_angle;
-        k.response = report_score ? (float)kp_score[o] : 0.f;
-        k.octave = 0; k.class_id = -1;
-        kp[o] = k;
-        kx[o] = (float)x; ky[o] = (float)y;
-        kcs[o] = cs;
+        store_keypoint((size_t)image * g.kp_cap + i, my_key, my_angle, orientation ? steer(my_angle) : make_float2(1.f, 0.f),
+                       kp_size, kp_score, report_score, kp, kx, ky, kcs);
     }
 }
 
@@ -196,24 +217,21 @@ orient_general_kernel(const uint8_t *__restrict__ img, Geom g, const uint32_t *_
     }
     if (lane == 0) {
         const float angle = fast_atan2_deg((float)m01, (float)m10);
-        const float th = __fmul_rn(angle, (float)(3.14159265358979323846 / 180.0));
-        fe_kpoint k;
-        k.x = (float)x; k.y = (float)y; k.size = kp_size; k.angle = angle;
-        k.response = report_score ? (float)kp_score[o] : 0.f;
-        k.octave = 0; k.class_id = -1;
-        kp[o] = k;
-        kx[o] = (float)x; ky[o] = (float)y;
-        kcs[o] = make_float2((float)cos((double)th), (float)sin((double)th));
+        store_keypoint(o, key, angle, steer(angle), kp_size, kp_score, report_score, kp, kx, ky, kcs);
     }
 }
 
-// half_patch > 0 selects the general kernel (b.umax holds OpenCV's umax table for that radius)
-int launch_orient_pack(const Geom &g, const DetectParams &p, const Buffers &b, bool orientation,
-                       float kp_size, int half_patch, cudaStream_t s) {
-    if (orientation && half_patch > 0) {
+// orient_pack_kernel reads the 31-px disc as aligned words straight from the image, up to 5 bytes past the disc's right end
+// (they weigh 0).  Keypoints more than ORI_R px from the border keep the disc inside the image and a row of the image below
+// it, so those bytes stay inside the image buffer.  Other patch sizes and nearer keypoints take orient_general_kernel.
+static bool orient_fast(const DetectParams &p) { return p.patch_size == ORB_PATCH && p.edge > ORI_R; }
+
+int launch_orient(const Geom &g, const DetectParams &p, const Buffers &b, bool orientation, cudaStream_t s) {
+    const float kp_size = orientation ? (float)p.patch_size : 7.f;      // cv::ORB's keypoints are patchSize wide, cv::FAST's 7
+    if (orientation && !orient_fast(p)) {       // b.umax holds OpenCV's umax table for radius patch_size / 2
         dim3 grid(div_up(g.kp_cap, ORI_WARPS), g.n_images);
         orient_general_kernel<<<grid, ORI_WARPS * 32, 0, s>>>(b.img, g, b.n_kp, b.kp_key, b.kp_score, p.nonmax ? 1 : 0, kp_size,
-                                                              half_patch, b.umax, b.kp, b.kx, b.ky, b.kcs);
+                                                              p.patch_size / 2, b.umax, b.kp, b.kx, b.ky, b.kcs);
         return 1;
     }
     dim3 grid(div_up(g.kp_cap, ORI_WARPS * ORI_KPW), g.n_images);
@@ -234,8 +252,7 @@ __global__ void unpack_kps_kernel(Geom g, const uint32_t *__restrict__ counts,
     const size_t o = (size_t)image * g.kp_cap + i;
     const fe_kpoint k = kp[o];
     kx[o] = k.x; ky[o] = k.y;
-    const float th = __fmul_rn(k.angle, (float)(3.14159265358979323846 / 180.0));
-    kcs[o] = make_float2((float)cos((double)th), (float)sin((double)th));
+    kcs[o] = steer(k.angle);
 }
 
 int launch_unpack_kps(const Geom &g, const Buffers &b, const uint32_t *counts, cudaStream_t s) {
@@ -479,10 +496,50 @@ __device__ __forceinline__ int rint_small(float v) {
     return __float_as_int(__fadd_rn(v, 12582912.f)) - 0x4B400000;
 }
 
+// pattern point (x, y) steered by (a, b) = (cos, sin): orb.cpp's GET_VALUE in f32, without FMA
+__device__ __forceinline__ float2 steer_point(float x, float y, float a, float b) {
+    return make_float2(__fsub_rn(__fmul_rn(x, a), __fmul_rn(y, b)), __fadd_rn(__fmul_rn(x, b), __fmul_rn(y, a)));
+}
+
+// Lane l always evaluates tests l, l + 32, ..., l + 224: its eight point pairs of bit_pattern_31_ live in registers as f32 for
+// all the keypoints it describes (no I2F and no shared-memory pattern reads in the test loop -- the LSU pipe bounds it)
+__device__ __forceinline__ void load_pattern(float4 (&pat)[8], int lane) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const char4 pt = reinterpret_cast<const char4 *>(d_pattern)[j * 32 + lane];
+        pat[j] = make_float4((float)pt.x, (float)pt.y, (float)pt.z, (float)pt.w);
+    }
+}
+
+// The 256 tests of one keypoint steered by (a, b) on a blurred patch in shared memory with rows ROW_BYTES apart; `centre` is
+// the shared-memory address of the keypoint's pixel.  The ballot of test j * 32 + l is exactly little-endian word j of the
+// 32-byte descriptor (bit i of byte b <-> test 8b + i): returned in lane j (lanes 0-7).
+template <int ROW_BYTES>
+__device__ __forceinline__ uint32_t rbrief_tests(const float4 (&pat)[8], float a, float b, uint32_t centre, int lane) {
+    // rint_small() leaves 0x4B400000 + i in the float's bits: the address of sample (ix, iy) is then
+    //   centre + iy * ROW_BYTES + ix = (centre - (ROW_BYTES + 1) * 0x4B400000) + bits_y * ROW_BYTES + bits_x   (32-bit wrap-around)
+    const uint32_t base = centre - 0x4B400000u * (uint32_t)(ROW_BYTES + 1);
+    auto sample = [&](float px, float py) {      // blurred pixel at (rint, rint) of the steered point
+        const float2 r = steer_point(px, py, a, b);
+        const uint32_t bx = __float_as_uint(__fadd_rn(r.x, 12582912.f)), by = __float_as_uint(__fadd_rn(r.y, 12582912.f));
+        uint32_t v;
+        asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(base + by * (uint32_t)ROW_BYTES + bx));
+        return v;
+    };
+    uint32_t word = 0;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const uint32_t t0 = sample(pat[j].x, pat[j].y);
+        const uint32_t t1 = sample(pat[j].z, pat[j].w);
+        const uint32_t w = __ballot_sync(0xffffffffu, t0 < t1);
+        if (lane == j) word = w;
+    }
+    return word;
+}
+
 // One warp per keypoint.  The 39 x 39 neighbourhood of the blurred image is first staged in shared
 // memory with aligned 32-bit loads (rows coalesced: ~80 sectors per keypoint instead of 512 scattered
-// byte gathers from L1), then lane l evaluates tests l, l+32, ..., l+224; the ballot of test j*32+l
-// is exactly little-endian word j of the 32-byte descriptor (bit i of byte b <-> test 8b+i).
+// byte gathers from L1), then the 256 tests sample the staged patch.
 __global__ void __launch_bounds__(BR_WARPS * 32)
 rbrief_kernel(const uint8_t *__restrict__ blur, Geom g, const uint32_t *__restrict__ counts,
               const float *__restrict__ kx, const float *__restrict__ ky,
@@ -492,14 +549,8 @@ rbrief_kernel(const uint8_t *__restrict__ blur, Geom g, const uint32_t *__restri
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int n = min((int)counts[image], g.kp_cap);
     if (blockIdx.x * (BR_WARPS * BR_KPW) >= n) return;
-    // lane l always evaluates tests l, l + 32, ..., l + 224: its eight point pairs live in registers as f32 for all the
-    // warp's keypoints (no I2F and no shared-memory pattern reads in the test loop -- the LSU pipe bounds this kernel)
     float4 pat[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-        const char4 pt = reinterpret_cast<const char4 *>(d_pattern)[j * 32 + lane];
-        pat[j] = make_float4((float)pt.x, (float)pt.y, (float)pt.z, (float)pt.w);
-    }
+    load_pattern(pat, lane);
     uint32_t *patch = s_patch[warp];
     // lane `it` fetches the record of the warp's keypoint `it` up front: one load latency per warp, not per keypoint
     float pre_x = 0.f, pre_y = 0.f;
@@ -516,9 +567,6 @@ rbrief_kernel(const uint8_t *__restrict__ blur, Geom g, const uint32_t *__restri
     const int st_w = lane % BR_WORDS, st_r = lane / BR_WORDS;
     const int st_goff = st_r * g.pitch + 4 * st_w, st_soff = st_r * BR_STRIDE + st_w;
     const int st_xoff = (3 * lane + 2) * g.pitch + 4 * (BR_WORDS - 1), st_xs = (3 * lane + 2) * BR_STRIDE + BR_WORDS - 1;
-    // rint_small() leaves 0x4B400000 + i in the float's bits: the shared-memory address of sample (ix, iy) is then
-    //   centre + iy * 48 + ix = (centre - 49 * 0x4B400000) + bits_y * 48 + bits_x      (32-bit wrap-around arithmetic)
-    constexpr uint32_t BIAS49 = 0x4B400000u * 49u;
 #pragma unroll 1
     for (int it = 0; it < BR_KPW; ++it) {
     const int i = (blockIdx.x * BR_KPW + it) * BR_WARPS + warp;
@@ -541,35 +589,19 @@ rbrief_kernel(const uint8_t *__restrict__ blur, Geom g, const uint32_t *__restri
     }
     __syncwarp();
     const uint8_t *pc = reinterpret_cast<const uint8_t *>(patch) + BR_R * (BR_STRIDE * 4) + BR_R + off;  // centre
-    const uint32_t pcs = (uint32_t)__cvta_generic_to_shared(pc) - BIAS49;
-    auto sample = [&](float fx, float fy) {       // blurred pixel at (rint(fx), rint(fy)) relative to the centre
-        const uint32_t bx = __float_as_uint(__fadd_rn(fx, 12582912.f)), by = __float_as_uint(__fadd_rn(fy, 12582912.f));
-        uint32_t v;
-        asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(pcs + by * (uint32_t)(BR_STRIDE * 4) + bx));
-        return v;
-    };
-    uint32_t word = 0;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-        const float4 pt = pat[j];
-        const float x0 = pt.x, y0 = pt.y, x1 = pt.z, y1 = pt.w;
-        const uint32_t t0 = sample(__fsub_rn(__fmul_rn(x0, a), __fmul_rn(y0, b)), __fadd_rn(__fmul_rn(x0, b), __fmul_rn(y0, a)));
-        const uint32_t t1 = sample(__fsub_rn(__fmul_rn(x1, a), __fmul_rn(y1, b)), __fadd_rn(__fmul_rn(x1, b), __fmul_rn(y1, a)));
-        const uint32_t w = __ballot_sync(0xffffffffu, t0 < t1);
-        if (lane == j) word = w;
-    }
+    const uint32_t word = rbrief_tests<BR_STRIDE * 4>(pat, a, b, (uint32_t)__cvta_generic_to_shared(pc), lane);
     if (lane < 8) reinterpret_cast<uint32_t *>(desc + o * 32)[lane] = word;
     }
 }
 
 // ---- orientation + rBRIEF per image tile ---------------------------------------------------------------------------------
-// Detect-and-describe of the default geometry (31-px patch, edgeThreshold >= 19, WTA_K 2, FAST score, one level): one CTA
-// per (image, DT_ROWS x DT_COLS tile of keypoint centres).  The CTA stages the raw and the blurred tile with a 19-px halo in
-// shared memory once and describes every keypoint of the tile from there.  orient_pack_kernel + rbrief_kernel instead re-read
-// each keypoint's neighbourhood from global memory: at ~5 200 keypoints per 1280 x 720 image that is ~15x the image, the
-// tiles stage ~2x it (halo included).  Keypoints are in raster order (kp_key ascending y << 16 | x per image), so those of the
-// tile's rows are one index range, found by binary search.  Moments, angle, (cos, sin) and the 256 tests are computed by the
-// same arithmetic as orient_pack_kernel and rbrief_kernel: the outputs are bit-identical.
+// Detect-and-describe of the default geometry (describe_tile_fits, FAST score, one level): one CTA per (image, DT_ROWS x
+// DT_COLS tile of keypoint centres).  The CTA stages the raw and the blurred tile with a 19-px halo in shared memory once and
+// describes every keypoint of the tile from there.  orient_pack_kernel + rbrief_kernel instead re-read each keypoint's
+// neighbourhood from global memory: at ~5 200 keypoints per 1280 x 720 image that is ~15x the image, the tiles stage ~2x it
+// (halo included).  Keypoints are in raster order (kp_key ascending y << 16 | x per image), so those of the tile's rows are one
+// index range, found by binary search.  Moments, angle, steering and the 256 tests are the helpers orient_pack_kernel and
+// rbrief_kernel call: the outputs are bit-identical.
 constexpr int DT_ROWS = 64, DT_COLS = 256;          // 64 x 128 and 32 x 256 tiles measured slower (more CTAs and halo)
 constexpr int DT_TROWS = DT_ROWS + 2 * BR_R;                // staged rows y0 - 19 .. y0 + DT_ROWS + 18
 // staged columns x0 - 32 .. x0 + DT_COLS + 31: 16-byte aligned (x0 is), they cover the reach -19 .. +20 of a keypoint (the
@@ -589,25 +621,6 @@ static_assert(DT_COLS % 16 == 0 && DT_XL % 16 == 0 && DT_XL >= BR_R, "staged col
 static_assert(DT_VECS * 16 <= DT_BLUR_B && DT_VECS * 4 <= DT_RAW_W && DT_BLUR_B % 16 == 0, "staged row fits the tile row");
 static_assert(DT_COLS + 2 * DT_XL - DT_XL >= DT_COLS + 21, "right halo reaches x + 20");
 static_assert(DT_RAW_W % 32 == 9 && (DT_BLUR_B / 4) % 32 == 20, "bank spread of the tile rows");
-
-// orient_pack_kernel's dp4a weight tables (u, membership mask) for the 4 alignments, built at compile time: read through L1 by
-// every CTA instead of rebuilt in shared memory
-struct OriTables { uint32_t u[4][288], m[4][288]; };
-constexpr OriTables make_ori_tables() {
-    constexpr int umax[16] = {15, 15, 15, 15, 14, 14, 14, 13, 13, 12, 11, 10, 9, 8, 6, 3};
-    OriTables t{};
-    for (int off = 0; off < 4; ++off)
-        for (int slot = 0; slot < ORI_SLOTS; ++slot) {
-            const int r = slot / ORI_WORDS, w = slot - r * ORI_WORDS;
-            const int v = r - 15, d = umax[v < 0 ? -v : v];
-            for (int b = 0; b < 4; ++b) {
-                const int u = 4 * w + b - off - 15;
-                if (u >= -d && u <= d) { t.u[off][slot] |= (uint32_t)(u & 0xFF) << (8 * b); t.m[off][slot] |= 1u << (8 * b); }
-            }
-        }
-    return t;
-}
-__device__ const OriTables d_ori_tab = make_ori_tables();
 
 // first index in [0, n) whose key is >= target (n if none): 32-way search, one key per lane per round
 __device__ __forceinline__ int warp_lower_bound(const uint32_t *__restrict__ keys, int n, uint32_t target, int lane) {
@@ -672,25 +685,12 @@ orb_describe_tile_kernel(const uint8_t *__restrict__ img, const uint8_t *__restr
             d[0] = v[k].x; d[1] = v[k].y; d[2] = v[k].z; d[3] = v[k].w;
         }
     }
-    // per-lane slot geometry of the orientation (same for every keypoint), relative to the patch's first word
-    int soff[(ORI_SLOTS + 31) / 32], sv[(ORI_SLOTS + 31) / 32];
-#pragma unroll
-    for (int k = 0; k < (ORI_SLOTS + 31) / 32; ++k) {
-        const int slot = min(lane + 32 * k, ORI_SLOTS - 1);
-        const int r = slot / ORI_WORDS, w = slot - r * ORI_WORDS;
-        soff[k] = r * DT_RAW_W + w;
-        sv[k] = r - 15;
-    }
-    // rBRIEF: lane l evaluates tests l, l + 32, ..., l + 224 (rbrief_kernel); the sample address comes from the bits of the
-    // 1.5 * 2^23-rounded coordinates:  centre + iy * DT_BLUR_B + ix = (centre - (DT_BLUR_B + 1) * 0x4B400000) + by * DT_BLUR_B + bx
+    int soff[ORI_K], sv[ORI_K];                 // the orientation's slot geometry in raw-tile words
+    ori_slots(lane, DT_RAW_W, 1, soff, sv);
     float4 pat[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-        const char4 pt = reinterpret_cast<const char4 *>(d_pattern)[j * 32 + lane];
-        pat[j] = make_float4((float)pt.x, (float)pt.y, (float)pt.z, (float)pt.w);
-    }
-    constexpr uint32_t BIAS = 0x4B400000u * (uint32_t)(DT_BLUR_B + 1);
-    const uint32_t blur_s = (uint32_t)__cvta_generic_to_shared(s_blur) - (uint32_t)(ty0 * DT_BLUR_B + sx) - BIAS;
+    load_pattern(pat, lane);
+    // shared-memory address of image pixel (0, 0) in the blurred tile's coordinates
+    const uint32_t blur_o = (uint32_t)__cvta_generic_to_shared(s_blur) - (uint32_t)(ty0 * DT_BLUR_B + sx);
     for (int base = lo; base < hi; base += DT_CHUNK) {
         // the band's keypoints whose x lies in the tile (any order: every result goes to its keypoint's own index)
 #pragma unroll
@@ -726,48 +726,24 @@ orb_describe_tile_kernel(const uint8_t *__restrict__ img, const uint8_t *__restr
             for (int it = 0; it < cnt; it += 2) {
                 const bool two = it + 1 < cnt;
                 const uint32_t key0 = __shfl_sync(FULL, my_key, it), key1 = __shfl_sync(FULL, my_key, two ? it + 1 : it);
-                const int xl0 = (int)(key0 & 0xFFFF) - 15, xa0 = xl0 & ~3, off0 = xl0 - xa0;
-                const int xl1 = (int)(key1 & 0xFFFF) - 15, xa1 = xl1 & ~3, off1 = xl1 - xa1;
-                const uint32_t *p0 = s_raw + ((int)(key0 >> 16) - 15 - ty0) * DT_RAW_W + ((xa0 - sx) >> 2);
-                const uint32_t *p1 = s_raw + ((int)(key1 >> 16) - 15 - ty0) * DT_RAW_W + ((xa1 - sx) >> 2);
-                const uint32_t *tu0 = d_ori_tab.u[off0], *tm0 = d_ori_tab.m[off0], *tu1 = d_ori_tab.u[off1], *tm1 = d_ori_tab.m[off1];
-                int m10a = 0, m01a = 0, m10b = 0, m01b = 0;
-#pragma unroll
-                for (int k = 0; k < (ORI_SLOTS + 31) / 32; ++k) {
+                const int xl0 = (int)(key0 & 0xFFFF) - ORI_R, xa0 = xl0 & ~3;
+                const int xl1 = (int)(key1 & 0xFFFF) - ORI_R, xa1 = xl1 & ~3;
+                const uint32_t *p0 = s_raw + ((int)(key0 >> 16) - ORI_R - ty0) * DT_RAW_W + ((xa0 - sx) >> 2);
+                const uint32_t *p1 = s_raw + ((int)(key1 >> 16) - ORI_R - ty0) * DT_RAW_W + ((xa1 - sx) >> 2);
+                auto words = [&](int k) {
                     const bool in = lane + 32 * k < ORI_SLOTS;
-                    const int slot = min(lane + 32 * k, ORI_SLOTS - 1);     // words past the last slot are 0
-                    const uint32_t wa = in ? p0[soff[k]] : 0u, wb = in ? p1[soff[k]] : 0u;
-                    m10a = dp4a_u8s8(wa, __ldg(tu0 + slot), m10a);
-                    m01a += sv[k] * dp4a_u8s8(wa, __ldg(tm0 + slot), 0);
-                    m10b = dp4a_u8s8(wb, __ldg(tu1 + slot), m10b);
-                    m01b += sv[k] * dp4a_u8s8(wb, __ldg(tm1 + slot), 0);
-                }
-#pragma unroll
-                for (int off2 = 16; off2; off2 >>= 1) {
-                    m10a += __shfl_xor_sync(FULL, m10a, off2);
-                    m01a += __shfl_xor_sync(FULL, m01a, off2);
-                    m10b += __shfl_xor_sync(FULL, m10b, off2);
-                    m01b += __shfl_xor_sync(FULL, m01b, off2);
-                }
-                const float angle0 = fast_atan2_deg((float)m01a, (float)m10a);
-                const float angle1 = fast_atan2_deg((float)m01b, (float)m10b);
-                if (lane == it) my_angle = angle0;
-                if (two && lane == it + 1) my_angle = angle1;
+                    return make_uint2(in ? p0[soff[k]] : 0u, in ? p1[soff[k]] : 0u);
+                };
+                const float2 angles = ori_angles(words, xl0 - xa0, xl1 - xa1, d_ori_tab.u, d_ori_tab.m, sv, lane);
+                if (lane == it) my_angle = angles.x;
+                if (two && lane == it + 1) my_angle = angles.y;
             }
-            // the record and the steering (cos, sin) in double, every lane its own keypoint
+            // the record and the steering, every lane its own keypoint
             float2 cs = make_float2(1.f, 0.f);
             if (valid) {
-                const size_t o = (size_t)image * g.kp_cap + my_i;
-                const int x = my_key & 0xFFFF, y = my_key >> 16;
-                const float th = __fmul_rn(my_angle, (float)(3.14159265358979323846 / 180.0));
-                cs = make_float2((float)cos((double)th), (float)sin((double)th));
-                fe_kpoint k;
-                k.x = (float)x; k.y = (float)y; k.size = kp_size; k.angle = my_angle;
-                k.response = report_score ? (float)kp_score[o] : 0.f;
-                k.octave = 0; k.class_id = -1;
-                kp[o] = k;
-                kx[o] = (float)x; ky[o] = (float)y;
-                kcs[o] = cs;
+                cs = steer(my_angle);
+                store_keypoint((size_t)image * g.kp_cap + my_i, my_key, my_angle, cs, kp_size, kp_score, report_score,
+                               kp, kx, ky, kcs);
             }
             // rBRIEF-256 from the blurred tile (rbrief_kernel)
 #pragma unroll 1
@@ -775,23 +751,7 @@ orb_describe_tile_kernel(const uint8_t *__restrict__ img, const uint8_t *__restr
                 const uint32_t key = __shfl_sync(FULL, my_key, it);
                 const int i = __shfl_sync(FULL, my_i, it);
                 const float a = __shfl_sync(FULL, cs.x, it), b = __shfl_sync(FULL, cs.y, it);
-                const uint32_t pcs = blur_s + (key >> 16) * (uint32_t)DT_BLUR_B + (key & 0xFFFF);
-                auto sample = [&](float fx, float fy) {
-                    const uint32_t bx = __float_as_uint(__fadd_rn(fx, 12582912.f)), by = __float_as_uint(__fadd_rn(fy, 12582912.f));
-                    uint32_t v;
-                    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(pcs + by * (uint32_t)DT_BLUR_B + bx));
-                    return v;
-                };
-                uint32_t word = 0;
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const float4 pt = pat[j];
-                    const float px0 = pt.x, py0 = pt.y, px1 = pt.z, py1 = pt.w;
-                    const uint32_t t0 = sample(__fsub_rn(__fmul_rn(px0, a), __fmul_rn(py0, b)), __fadd_rn(__fmul_rn(px0, b), __fmul_rn(py0, a)));
-                    const uint32_t t1 = sample(__fsub_rn(__fmul_rn(px1, a), __fmul_rn(py1, b)), __fadd_rn(__fmul_rn(px1, b), __fmul_rn(py1, a)));
-                    const uint32_t w = __ballot_sync(FULL, t0 < t1);
-                    if (lane == j) word = w;
-                }
+                const uint32_t word = rbrief_tests<DT_BLUR_B>(pat, a, b, blur_o + (key >> 16) * (uint32_t)DT_BLUR_B + (key & 0xFFFF), lane);
                 if (lane < 8) reinterpret_cast<uint32_t *>(desc + ((size_t)image * g.kp_cap + i) * 32)[lane] = word;
             }
         }
@@ -799,7 +759,13 @@ orb_describe_tile_kernel(const uint8_t *__restrict__ img, const uint8_t *__restr
     }
 }
 
-int launch_describe_tile(const Geom &g, const DetectParams &p, const Buffers &b, float kp_size, cudaStream_t s) {
+// rbrief_kernel stages the blurred image within BR_R px of each keypoint without a border, and orb_describe_tile_kernel stages
+// image tiles the same way: both serve bit_pattern_31_ (WTA_K 2) at keypoints at least BR_R px from the border.
+static bool rbrief_fast(const DetectParams &p) { return p.wta_k == 2 && p.patch_size == ORB_PATCH && p.edge >= BR_R; }
+
+bool describe_tile_fits(const DetectParams &p) { return orient_fast(p) && rbrief_fast(p); }
+
+int launch_describe_tile(const Geom &g, const DetectParams &p, const Buffers &b, cudaStream_t s) {
     static bool smem_set[64] = {false};         // per device: the attribute belongs to the device's context
     int dev = 0;
     cudaGetDevice(&dev);
@@ -809,14 +775,25 @@ int launch_describe_tile(const Geom &g, const DetectParams &p, const Buffers &b,
     }
     dim3 grid(div_up(g.w, DT_COLS), div_up(g.h, DT_ROWS), g.n_images);
     orb_describe_tile_kernel<<<grid, DT_THREADS, DT_SMEM, s>>>(b.img, b.blur, g, b.n_kp, b.kp_key, b.kp_score, p.nonmax ? 1 : 0,
-                                                               kp_size, b.kp, b.kx, b.ky, b.kcs, b.desc);
+                                                               (float)p.patch_size, b.kp, b.kx, b.ky, b.kcs, b.desc);
     return 1;
 }
 
-// rBRIEF-256 with a caller-selected pattern (ORB::setPatchSize != 31 -> makeRandomPattern, bin/detect_node:50-51).
-// No staging: the pattern may reach half_patch * sqrt(2) px.  cv2 samples a bordered copy of the image in which
-// only the image area was blurred: a sample outside the image is the RAW pixel at the BORDER_REFLECT_101 position
-// (pinned against cv2 4.13 with patchSize 70, where 8.7 % of the descriptors touch the border).
+// Sample of cv::ORB's bordered image at the keypoint (cx, cy) plus the steered, rounded pattern point (px, py): the blurred
+// pixel inside the image; outside it the RAW pixel at the BORDER_REFLECT_101 position, because cv2 blurs only the image area
+// of its bordered buffer (pinned against cv2 4.13 with patchSize 70, where 8.7 % of the descriptors touch the border)
+__device__ __forceinline__ int bordered_sample(const uint8_t *bl, const uint8_t *rw, const Geom &g, int cx, int cy, float px,
+                                               float py, float a, float b) {
+    const float2 r = steer_point(px, py, a, b);
+    int x = cx + rint_small(r.x), y = cy + rint_small(r.y);
+    if (x >= 0 && x < g.w && y >= 0 && y < g.h) return bl[(size_t)y * g.pitch + x];
+    x = min(max(reflect101(x, g.w), 0), g.w - 1);
+    y = min(max(reflect101(y, g.h), 0), g.h - 1);
+    return rw[(size_t)y * g.pitch + x];
+}
+
+// rBRIEF-256 with a caller-selected pattern (ORB::setPatchSize != 31 -> makeRandomPattern, bin/detect_node:50-51), or the
+// built-in one at keypoints nearer the border than BR_R.  No staging: the pattern may reach half_patch * sqrt(2) px.
 __global__ void __launch_bounds__(BR_WARPS * 32)
 rbrief_general_kernel(const uint8_t *__restrict__ blur, const uint8_t *__restrict__ raw, Geom g,
                       const uint32_t *__restrict__ counts, const float *__restrict__ kx, const float *__restrict__ ky,
@@ -835,33 +812,17 @@ rbrief_general_kernel(const uint8_t *__restrict__ blur, const uint8_t *__restric
     const size_t o = (size_t)image * g.kp_cap + i;
     const int cx = __float2int_rn(kx[o]), cy = __float2int_rn(ky[o]);
     const float2 cs = kcs[o];
-    const float a = cs.x, b = cs.y;
     const uint8_t *bl = blur + (size_t)image * g.img_stride, *rw = raw + (size_t)image * g.img_stride;
-    auto sample = [&](int x, int y) -> int {
-        if (x >= 0 && x < g.w && y >= 0 && y < g.h) return bl[(size_t)y * g.pitch + x];
-        x = min(max(reflect101(x, g.w), 0), g.w - 1);
-        y = min(max(reflect101(y, g.h), 0), g.h - 1);
-        return rw[(size_t)y * g.pitch + x];
-    };
     uint32_t word = 0;
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
         const float4 pt = s_pat[j * 32 + lane];
-        const int ix0 = rint_small(__fsub_rn(__fmul_rn(pt.x, a), __fmul_rn(pt.y, b)));
-        const int iy0 = rint_small(__fadd_rn(__fmul_rn(pt.x, b), __fmul_rn(pt.y, a)));
-        const int ix1 = rint_small(__fsub_rn(__fmul_rn(pt.z, a), __fmul_rn(pt.w, b)));
-        const int iy1 = rint_small(__fadd_rn(__fmul_rn(pt.z, b), __fmul_rn(pt.w, a)));
-        const int t0 = sample(cx + ix0, cy + iy0), t1 = sample(cx + ix1, cy + iy1);
+        const int t0 = bordered_sample(bl, rw, g, cx, cy, pt.x, pt.y, cs.x, cs.y);
+        const int t1 = bordered_sample(bl, rw, g, cx, cy, pt.z, pt.w, cs.x, cs.y);
         const uint32_t w = __ballot_sync(0xffffffffu, t0 < t1);
         if (lane == j) word = w;
     }
     if (lane < 8) reinterpret_cast<uint32_t *>(desc + o * 32)[lane] = word;
-}
-
-int launch_brief_general(const Geom &g, const Buffers &b, const uint32_t *counts, cudaStream_t s) {
-    dim3 grid(div_up(g.kp_cap, BR_WARPS), g.n_images);
-    rbrief_general_kernel<<<grid, BR_WARPS * 32, 0, s>>>(b.blur, b.img, g, counts, b.kx, b.ky, b.kcs, b.pattern, b.desc);
-    return 1;
 }
 
 // ORB with WTA_K = 3 / 4 (orb.cpp computeOrbDescriptors): 128 tuples of K points, two bits per tuple = index of the
@@ -883,17 +844,8 @@ rbrief_wta_kernel(const uint8_t *__restrict__ blur, const uint8_t *__restrict__ 
     const size_t o = (size_t)image * g.kp_cap + i;
     const int cx = __float2int_rn(kx[o]), cy = __float2int_rn(ky[o]);
     const float2 cs = kcs[o];
-    const float a = cs.x, b = cs.y;
     const uint8_t *bl = blur + (size_t)image * g.img_stride, *rw = raw + (size_t)image * g.img_stride;
-    auto sample = [&](int idx) -> int {
-        const float2 pt = s_pat[idx];
-        int x = cx + rint_small(__fsub_rn(__fmul_rn(pt.x, a), __fmul_rn(pt.y, b)));
-        int y = cy + rint_small(__fadd_rn(__fmul_rn(pt.x, b), __fmul_rn(pt.y, a)));
-        if (x >= 0 && x < g.w && y >= 0 && y < g.h) return bl[(size_t)y * g.pitch + x];
-        x = min(max(reflect101(x, g.w), 0), g.w - 1);
-        y = min(max(reflect101(y, g.h), 0), g.h - 1);
-        return rw[(size_t)y * g.pitch + x];
-    };
+    auto sample = [&](int idx) { return bordered_sample(bl, rw, g, cx, cy, s_pat[idx].x, s_pat[idx].y, cs.x, cs.y); };
     uint32_t val = 0;
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
@@ -915,16 +867,17 @@ rbrief_wta_kernel(const uint8_t *__restrict__ blur, const uint8_t *__restrict__ 
     desc[o * 32 + lane] = (uint8_t)val;
 }
 
-int launch_brief_wta(const Geom &g, const Buffers &b, const uint32_t *counts, int wta_k, cudaStream_t s) {
+int launch_rbrief(const Geom &g, const DetectParams &p, const Buffers &b, const uint32_t *counts, cudaStream_t s) {
+    if (rbrief_fast(p)) {
+        dim3 grid(div_up(g.kp_cap, BR_WARPS * BR_KPW), g.n_images);
+        rbrief_kernel<<<grid, BR_WARPS * 32, 0, s>>>(b.blur, g, counts, b.kx, b.ky, b.kcs, b.desc);
+        return 1;
+    }
+    // b.pattern holds the ctx's pattern (bit_pattern_31_ or makeRandomPattern(patch_size)), as WTA_K-point tuples for WTA_K 3 / 4
     dim3 grid(div_up(g.kp_cap, BR_WARPS), g.n_images);
-    if (wta_k == 3) rbrief_wta_kernel<3><<<grid, BR_WARPS * 32, 0, s>>>(b.blur, b.img, g, counts, b.kx, b.ky, b.kcs, b.pattern, b.desc);
-    else rbrief_wta_kernel<4><<<grid, BR_WARPS * 32, 0, s>>>(b.blur, b.img, g, counts, b.kx, b.ky, b.kcs, b.pattern, b.desc);
-    return 1;
-}
-
-int launch_brief(const Geom &g, const Buffers &b, const uint32_t *counts, cudaStream_t s) {
-    dim3 grid(div_up(g.kp_cap, BR_WARPS * BR_KPW), g.n_images);
-    rbrief_kernel<<<grid, BR_WARPS * 32, 0, s>>>(b.blur, g, counts, b.kx, b.ky, b.kcs, b.desc);
+    if (p.wta_k == 3) rbrief_wta_kernel<3><<<grid, BR_WARPS * 32, 0, s>>>(b.blur, b.img, g, counts, b.kx, b.ky, b.kcs, b.pattern, b.desc);
+    else if (p.wta_k == 4) rbrief_wta_kernel<4><<<grid, BR_WARPS * 32, 0, s>>>(b.blur, b.img, g, counts, b.kx, b.ky, b.kcs, b.pattern, b.desc);
+    else rbrief_general_kernel<<<grid, BR_WARPS * 32, 0, s>>>(b.blur, b.img, g, counts, b.kx, b.ky, b.kcs, b.pattern, b.desc);
     return 1;
 }
 

@@ -50,6 +50,7 @@ struct fe_ctx {
     int batch_desc = FE_DESC_ORB256;  // what the batched pipeline describes with (fe_set_batch_descriptor)
     int wu_frames = 0, wu_prev_n = 0;  // fe_window_update: frames in the window, landmarks of the previous frame
     bool wu_prev_sorted = true;
+    int wu_dim = 0;                    // rows of the frames in the window: 0 = binary, 64 / 128 = SURF floats
     int brief_bytes[3] = {0, 0, 0};   // fe_set_brief_pattern: table present for BRIEF-16 / 32 / 64 (Buffers::brief_tab)
     int brief_orient[3] = {0, 0, 0};
     // fe_set_freak: cv::FREAK's pattern sizes and parameters (the pattern itself is in Buffers::freak_*)
@@ -1379,16 +1380,20 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
     if (!cfg || !n_tracks || n < 0 || (n > 0 && (!l_kps || !l_desc)) || cap < 0 || (cap > 0 && !tracks))
         return fail(c, FE_ERR_BAD_ARG, "fe_window_update: bad argument");
     const bool live = cfg->mode == FE_MATCH_CROSSCHECK;
-    if (desc_kind != FE_DESC_ORB256 && desc_kind != FE_DESC_BRIEF16 && desc_kind != FE_DESC_BRIEF32)
-        return fail(c, FE_ERR_UNSUPPORTED, "fe_window_update: binary descriptors of up to 256 bits");
-    if (cfg->norm != FE_NORM_HAMMING && cfg->norm != FE_NORM_HAMMING2) return fail(c, FE_ERR_UNSUPPORTED, "fe_window_update: Hamming norms");
+    const int dim = desc_dim(desc_kind);      // SURF-64 / SURF-128 float rows; 0 = binary
+    if (dim == 0 && desc_kind != FE_DESC_ORB256 && desc_kind != FE_DESC_BRIEF16 && desc_kind != FE_DESC_BRIEF32)
+        return fail(c, FE_ERR_UNSUPPORTED, "fe_window_update: binary descriptors of up to 256 bits, or SURF-64 / SURF-128");
+    if (dim == 0 && cfg->norm != FE_NORM_HAMMING && cfg->norm != FE_NORM_HAMMING2) return fail(c, FE_ERR_UNSUPPORTED, "fe_window_update: Hamming norms");
+    if (dim > 0 && cfg->norm != FE_NORM_L2) return fail(c, FE_ERR_UNSUPPORTED, "fe_window_update: SURF rows are matched with FE_NORM_L2");
     if (live && !r_desc && n > 0) return fail(c, FE_ERR_BAD_ARG, "fe_window_update: the liveGraph variant needs the right descriptors");
     if (live && cfg->mask != FE_MASK_NONE) return fail(c, FE_ERR_BAD_ARG, "fe_window_update: cross-check takes no mask (BFMatcher asserts)");
+    if (c->wu_frames >= 1 && dim != c->wu_dim)
+        return fail(c, FE_ERR_BAD_ARG, "fe_window_update: the previous frame's rows are of another kind (binary, SURF-64, SURF-128): reset the window first");
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     const size_t C = c->cfg.max_keypoints;
     if (n > (int)C) return fail(c, FE_ERR_CAPACITY, "more landmarks than fe_config.max_keypoints");
     int r;
-    if ((r = ensure(c, GRP_WUPDATE | (live ? GRP_WLIVE : 0u))) != FE_OK) return r;
+    if ((r = ensure(c, GRP_WUPDATE | (dim > 0 ? match_groups(dim, false) | GRP_WUFLOAT : live ? GRP_WLIVE : 0u))) != FE_OK) return r;
     Buffers &b = c->b;
     if (c->g.kp_cap == 0 && (r = set_geom(c, 16, 16, 2)) != FE_OK) return r;
     const int bin_bytes = desc_kind == FE_DESC_BRIEF16 ? 16 : 32;
@@ -1400,12 +1405,23 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
         }
         return FE_OK;
     };
+    // float rows of dim floats -> device rows of 128 floats (fdesc's stride, which the L2 matchers read)
+    auto put_rows = [&](float *dst, const void *src) -> int {
+        FE_CUDA(c, cudaMemcpy2DAsync(dst, sizeof(float) * 128, src, sizeof(float) * dim, sizeof(float) * dim, n, cudaMemcpyHostToDevice,
+                                     c->stream));
+        return FE_OK;
+    };
     {   // slot 0 <- the new frame
         StageTimer t(c, ST_H2D);
         if (n > 0) {
             FE_CUDA(c, cudaMemcpyAsync(b.wu_kp, l_kps, sizeof(fe_kpoint) * n, cudaMemcpyHostToDevice, c->stream));
-            if ((r = put_desc(b.wu_desc, l_desc)) != FE_OK) return r;
-            if (r_desc && (r = put_desc(b.wu_rdesc, r_desc)) != FE_OK) return r;
+            if (dim > 0) {
+                if ((r = put_rows(b.wu_fdesc, l_desc)) != FE_OK) return r;
+                if (r_desc && (r = put_rows(b.wu_frdesc, r_desc)) != FE_OK) return r;
+            } else {
+                if ((r = put_desc(b.wu_desc, l_desc)) != FE_OK) return r;
+                if (r_desc && (r = put_desc(b.wu_rdesc, r_desc)) != FE_OK) return r;
+            }
         }
         c->h_counts[0] = (uint32_t)n; c->h_counts[1] = (uint32_t)c->wu_prev_n;
         FE_CUDA(c, cudaMemcpyAsync(b.wu_n, c->h_counts, 2 * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
@@ -1414,7 +1430,7 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
     Geom gv = c->g;
     gv.n_images = 2;
     Buffers v = b;
-    v.kp = b.wu_kp; v.kx = b.wu_kx; v.ky = b.wu_ky; v.kcs = b.wu_kcs; v.desc = b.wu_desc;
+    v.kp = b.wu_kp; v.kx = b.wu_kx; v.ky = b.wu_ky; v.kcs = b.wu_kcs; v.desc = b.wu_desc; v.fdesc = b.wu_fdesc;
     { StageTimer t(c, ST_ORIENT); t.done(launch_unpack_kps(gv, v, b.wu_n, c->stream)); }   // (re-derives the previous frame's kx / ky too)
     bool sorted = true;        // raster order of the new frame's landmarks: the banded kernel's precondition when it is the train side next time
     for (int i = 1; i < n && sorted; ++i) sorted = !(l_kps[i].y < l_kps[i - 1].y);
@@ -1427,7 +1443,20 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
     else if (frames >= len) frames = std::max(len - 1, 0);
     int found = 0;
     if (c->wu_frames >= 1 && frames > 1) {      // window.size() > 1: match against window[size - 2]
-        if (live) {
+        if (live && dim > 0) {
+            // liveGraph applies no |dy| filter: the exact all-pairs FP32 pass on the left and on the right rows.  The right
+            // side's keys use the ratio-mode key arrays, which cross-check mode leaves free.
+            Buffers vl = v, vr = v;
+            vr.fdesc = b.wu_frdesc; vr.allbest64 = b.best64; vr.colbest64 = b.second64;
+            const MatchParams none = match_params(nullptr);
+            { StageTimer t(c, ST_L2);
+              t.done(launch_l2_match(gv, 1, dim, none, false, true, vl, b.wu_n, c->stream) +
+                     launch_l2_match(gv, 1, dim, none, false, true, vr, b.wu_n, c->stream)); }
+            { StageTimer t(c, ST_FINALIZE);
+              t.done(launch_l2_finalize_cross_both(gv, 1, b.wu_n, b.allbest64, b.colbest64, b.best64, b.second64, b.match_b, b.n_b,
+                                                   c->stream)); }
+            FE_CUDA(c, cudaGetLastError());
+        } else if (live) {
             const bool h2 = cfg->norm == FE_NORM_HAMMING2;
             Buffers vl = v, vr = v;
             vl.allbest = b.allbest; vl.colbest = b.colbest;
@@ -1441,7 +1470,9 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
             fe_match_cfg w = *cfg;
             w.mode = FE_MATCH_RATIO;
             if (w.mask == FE_MASK_WINDOW) { if (w.win_w <= 0) w.win_w = 100; if (w.win_h <= 0) w.win_h = 100; }
-            if ((r = run_match_on(c, gv, v, c->stream, true, 1, &w, nullptr, b.wu_n, c->wu_prev_sorted, false)) != FE_OK) return r;
+            if (dim > 0) r = run_match_l2_on(c, gv, v, c->stream, true, 1, dim, &w, nullptr, b.wu_n, c->wu_prev_sorted);
+            else r = run_match_on(c, gv, v, c->stream, true, 1, &w, nullptr, b.wu_n, c->wu_prev_sorted, false);
+            if (r != FE_OK) return r;
         }
         FE_CUDA(c, cudaMemcpyAsync(c->h_counts, live ? b.n_b : b.n_a, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
         FE_CUDA(c, cudaStreamSynchronize(c->stream));
@@ -1449,13 +1480,21 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
         const int m = std::min(found, cap);
         if (m > 0) FE_CUDA(c, cudaMemcpyAsync(tracks, live ? b.match_b : b.match_a, sizeof(fe_match) * m, cudaMemcpyDeviceToHost, c->stream));
     }
-    // shift: the new frame becomes the previous one (device-to-device, ~70 bytes per landmark)
+    // shift: the new frame becomes the previous one (device-to-device, ~70 bytes per binary landmark, 4 * dim + 28 per SURF one)
     if (n > 0) {
         FE_CUDA(c, cudaMemcpyAsync(b.wu_kp + C, b.wu_kp, sizeof(fe_kpoint) * n, cudaMemcpyDeviceToDevice, c->stream));
-        FE_CUDA(c, cudaMemcpyAsync(b.wu_desc + C * 32, b.wu_desc, (size_t)32 * n, cudaMemcpyDeviceToDevice, c->stream));
-        if (r_desc) FE_CUDA(c, cudaMemcpyAsync(b.wu_rdesc + C * 32, b.wu_rdesc, (size_t)32 * n, cudaMemcpyDeviceToDevice, c->stream));
+        if (dim > 0) {
+            const size_t pitch = sizeof(float) * 128;
+            FE_CUDA(c, cudaMemcpy2DAsync(b.wu_fdesc + C * 128, pitch, b.wu_fdesc, pitch, sizeof(float) * dim, n, cudaMemcpyDeviceToDevice, c->stream));
+            if (r_desc)
+                FE_CUDA(c, cudaMemcpy2DAsync(b.wu_frdesc + C * 128, pitch, b.wu_frdesc, pitch, sizeof(float) * dim, n, cudaMemcpyDeviceToDevice,
+                                             c->stream));
+        } else {
+            FE_CUDA(c, cudaMemcpyAsync(b.wu_desc + C * 32, b.wu_desc, (size_t)32 * n, cudaMemcpyDeviceToDevice, c->stream));
+            if (r_desc) FE_CUDA(c, cudaMemcpyAsync(b.wu_rdesc + C * 32, b.wu_rdesc, (size_t)32 * n, cudaMemcpyDeviceToDevice, c->stream));
+        }
     }
-    c->wu_prev_n = n; c->wu_prev_sorted = sorted; c->wu_frames = frames;
+    c->wu_prev_n = n; c->wu_prev_sorted = sorted; c->wu_frames = frames; c->wu_dim = dim;
     *n_tracks = found;
     if (frames_in_window) *frames_in_window = frames;
     if ((r = sync_and_resolve(c)) != FE_OK) return r;
@@ -1478,13 +1517,46 @@ int32_t fe_batch_upload(fe_ctx *c, int32_t n_pairs, const uint8_t *left, const u
     return FE_OK;
 }
 
+// fe_window_batch on a SURF batch: the landmarks' float rows gathered into virtual pairs (g: the resident batch, gv: its
+// 2 (F - 1) virtual-pair slots) and matched by the L2 kernels.
+static int window_batch_l2(fe_ctx *c, const Geom &g, const Geom &gv, const fe_match_cfg *cfg, bool live, int dim) {
+    const int F = g.n_images / 2, V = F - 1;
+    Buffers &b = c->b;
+    { StageTimer t(c, ST_ORIENT); t.done(launch_gather_landmarks(g, F, b, 0, dim, b.wfdesc, b.wkx, b.wky, b.wcount, c->stream)); }
+    Buffers v = b;
+    v.fdesc = b.wfdesc; v.kx = b.wkx; v.ky = b.wky;
+    v.best64 = b.wbest64; v.second64 = b.wsecond64; v.match_a = b.wmatch; v.n_a = b.wn;
+    if (live) {
+        // liveGraph applies no |dy| filter, so there are no band candidates for the tensor-core cross-check: the exact
+        // all-pairs FP32 pass on the left rows and on the right rows, then the same-landmark intersection
+        { StageTimer t(c, ST_ORIENT); t.done(launch_gather_landmarks(g, F, b, 1, dim, b.wfdesc_r, nullptr, nullptr, b.wcount, c->stream)); }
+        Buffers vl = v, vr = v;
+        vl.allbest64 = b.wbest64; vl.colbest64 = b.wsecond64;
+        vr.fdesc = b.wfdesc_r; vr.allbest64 = b.wbest64_r; vr.colbest64 = b.wcol64_r;
+        const MatchParams none = match_params(nullptr);
+        { StageTimer t(c, ST_L2);
+          t.done(launch_l2_match(gv, V, dim, none, false, true, vl, b.wcount, c->stream) +
+                 launch_l2_match(gv, V, dim, none, false, true, vr, b.wcount, c->stream)); }
+        { StageTimer t(c, ST_FINALIZE);
+          t.done(launch_l2_finalize_cross_both(gv, V, b.wcount, b.wbest64, b.wsecond64, b.wbest64_r, b.wcol64_r, b.wmatch, b.wn,
+                                               c->stream)); }
+        FE_CUDA(c, cudaGetLastError());
+        return FE_OK;
+    }
+    // landmarks inherit the left keypoints' order: raster order only without a pyramid (level-major otherwise)
+    return run_match_l2_on(c, gv, v, c->stream, true, V, dim, cfg, nullptr, b.wcount, c->nlevels == 1);
+}
+
 // WindowMatcher::newStereo matching stage for a whole resident sequence (src/WindowMatcher.cpp:75-231).
 int32_t fe_window_batch(fe_ctx *c, const fe_match_cfg *cfg, const double *Q, int32_t cap, fe_match *tracks,
                         int32_t *n_tracks, double *xyz) {
     if (!c || !cfg || cap < 0 || (cap > 0 && !tracks) || !n_tracks) return fail(c, FE_ERR_BAD_ARG, "fe_window_batch: bad argument");
     if (c->g.n_images < 4) return fail(c, FE_ERR_BAD_ARG, "fe_window_batch: run fe_batch_run on at least two frames first");
-    if ((cfg->norm != FE_NORM_HAMMING && cfg->norm != FE_NORM_HAMMING2) || c->batch_desc != FE_DESC_ORB256)
-        return fail(c, FE_ERR_UNSUPPORTED, "fe_window_batch: ORB-256 / Hamming sequences only");
+    const int dim = desc_dim(c->batch_desc);     // SURF-64 / SURF-128 batches: float rows and FE_NORM_L2
+    const bool hamming = cfg->norm == FE_NORM_HAMMING || cfg->norm == FE_NORM_HAMMING2;
+    if (dim == 0 && (!hamming || c->batch_desc != FE_DESC_ORB256))
+        return fail(c, FE_ERR_UNSUPPORTED, "fe_window_batch: ORB-256 sequences are matched with FE_NORM_HAMMING / FE_NORM_HAMMING2");
+    if (dim > 0 && cfg->norm != FE_NORM_L2) return fail(c, FE_ERR_UNSUPPORTED, "fe_window_batch: SURF sequences are matched with FE_NORM_L2");
     const bool live = cfg->mode == FE_MATCH_CROSSCHECK;       // liveGraph variant (algorithm.py:1160-1190)
     if (!live && (cfg->mode != FE_MATCH_RATIO || cfg->mask != FE_MASK_WINDOW))
         return fail(c, FE_ERR_BAD_ARG, "fe_window_batch: cfg must be ratio mode with the window mask, or cross-check mode (liveGraph)");
@@ -1492,31 +1564,34 @@ int32_t fe_window_batch(fe_ctx *c, const fe_match_cfg *cfg, const double *Q, int
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     const Geom &g = c->g;
     const int F = g.n_images / 2, V = F - 1;
-    int r = ensure(c, GRP_WINDOW | (live ? GRP_WLIVE : 0u));
+    int r = ensure(c, GRP_WINDOW | (dim > 0 ? match_groups(dim, false) | GRP_WFLOAT | (live ? GRP_WFLIVE : 0u) : live ? GRP_WLIVE : 0u));
     if (r != FE_OK) return r;
     Buffers &b = c->b;
-    { StageTimer t(c, ST_ORIENT); t.done(launch_gather_landmarks(g, F, b, 0, b.wdesc, b.wkx, b.wky, b.wcount, c->stream)); }
-    // the stereo matcher's kernels on the virtual pairs: a Buffers view whose inputs / outputs are the w* arrays
-    Buffers v = b;
-    v.desc = b.wdesc; v.kx = b.wkx; v.ky = b.wky;
-    v.best = b.wbest; v.second = b.wsecond; v.match_a = b.wmatch; v.n_a = b.wn;
     Geom gv = g;
     gv.n_images = 2 * V;
-    if (live) {
-        // cur <-> prev cross-check on the LEFT descriptors and on the RIGHT descriptors, then the same-landmark intersection
-        { StageTimer t(c, ST_ORIENT); t.done(launch_gather_landmarks(g, F, b, 1, b.wdesc_r, nullptr, nullptr, b.wcount, c->stream)); }
-        const bool h2 = cfg->norm == FE_NORM_HAMMING2;
-        Buffers vl = b, vr = b;
-        vl.desc = b.wdesc; vl.allbest = b.wbest; vl.colbest = b.wsecond;
-        vr.desc = b.wdesc_r; vr.allbest = b.wbest_r; vr.colbest = b.wcol_r;
-        { StageTimer t(c, ST_MATCH);
-          t.done(launch_hamming_cross(gv, V, h2, vl, b.wcount, c->stream) + launch_hamming_cross(gv, V, h2, vr, b.wcount, c->stream)); }
-        { StageTimer t(c, ST_FINALIZE);
-          t.done(launch_finalize_cross_both(gv, V, b.wcount, b.wbest, b.wsecond, b.wbest_r, b.wcol_r, b.wmatch, b.wn, c->stream)); }
-        FE_CUDA(c, cudaGetLastError());
-    } else {
-        // landmarks inherit the left keypoints' order: raster order only without a pyramid (level-major otherwise)
-        r = run_match_on(c, gv, v, c->stream, true, V, cfg, nullptr, b.wcount, c->nlevels == 1, false);
+    if (dim > 0) r = window_batch_l2(c, g, gv, cfg, live, dim);
+    else {
+        { StageTimer t(c, ST_ORIENT); t.done(launch_gather_landmarks(g, F, b, 0, b.wdesc, b.wkx, b.wky, b.wcount, c->stream)); }
+        // the stereo matcher's kernels on the virtual pairs: a Buffers view whose inputs / outputs are the w* arrays
+        Buffers v = b;
+        v.desc = b.wdesc; v.kx = b.wkx; v.ky = b.wky;
+        v.best = b.wbest; v.second = b.wsecond; v.match_a = b.wmatch; v.n_a = b.wn;
+        if (live) {
+            // cur <-> prev cross-check on the LEFT descriptors and on the RIGHT descriptors, then the same-landmark intersection
+            { StageTimer t(c, ST_ORIENT); t.done(launch_gather_landmarks(g, F, b, 1, b.wdesc_r, nullptr, nullptr, b.wcount, c->stream)); }
+            const bool h2 = cfg->norm == FE_NORM_HAMMING2;
+            Buffers vl = b, vr = b;
+            vl.desc = b.wdesc; vl.allbest = b.wbest; vl.colbest = b.wsecond;
+            vr.desc = b.wdesc_r; vr.allbest = b.wbest_r; vr.colbest = b.wcol_r;
+            { StageTimer t(c, ST_MATCH);
+              t.done(launch_hamming_cross(gv, V, h2, vl, b.wcount, c->stream) + launch_hamming_cross(gv, V, h2, vr, b.wcount, c->stream)); }
+            { StageTimer t(c, ST_FINALIZE);
+              t.done(launch_finalize_cross_both(gv, V, b.wcount, b.wbest, b.wsecond, b.wbest_r, b.wcol_r, b.wmatch, b.wn, c->stream)); }
+            FE_CUDA(c, cudaGetLastError());
+        } else {
+            // landmarks inherit the left keypoints' order: raster order only without a pyramid (level-major otherwise)
+            r = run_match_on(c, gv, v, c->stream, true, V, cfg, nullptr, b.wcount, c->nlevels == 1, false);
+        }
     }
     if (r != FE_OK) return r;
     if (Q && xyz) {
@@ -1651,21 +1726,23 @@ int32_t fe_set_orb_pyramid(fe_ctx *c, int32_t nlevels, float scale_factor) {
 }
 
 // stereoLandmarks of every pair of the resident batch (algorithm_one's packing, src/front_end/algorithm.py:893-913).
-int32_t fe_batch_landmarks(fe_ctx *c, int32_t which, int32_t cap, fe_kpoint *l_kps, uint8_t *l_desc, fe_kpoint *r_kps,
-                           uint8_t *r_desc, fe_match *matches, int32_t *n) {
+int32_t fe_batch_landmarks(fe_ctx *c, int32_t which, int32_t cap, fe_kpoint *l_kps, void *l_desc, fe_kpoint *r_kps,
+                           void *r_desc, fe_match *matches, int32_t *n) {
     if (!c || !n || cap < 0 || (which != 0 && which != 1)) return fail(c, FE_ERR_BAD_ARG, "fe_batch_landmarks: bad argument");
     if (c->g.n_images < 2) return fail(c, FE_ERR_BAD_ARG, "fe_batch_landmarks: run fe_batch_run first");
-    if (c->batch_desc != FE_DESC_ORB256) return fail(c, FE_ERR_UNSUPPORTED, "fe_batch_landmarks: ORB-256 batches only");
+    const int dim = desc_dim(c->batch_desc);     // SURF batches: rows of dim floats
+    if (c->batch_desc != FE_DESC_ORB256 && dim == 0) return fail(c, FE_ERR_UNSUPPORTED, "fe_batch_landmarks: ORB-256 or SURF batches");
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     const Geom &g = c->g;
     const int P = g.n_images / 2;
-    int r = ensure(c, GRP_LANDMARKS);
+    int r = ensure(c, GRP_LANDMARKS | (dim > 0 ? GRP_LMFLOAT : 0u));
     if (r != FE_OK) return r;
     Buffers &b = c->b;
     const uint32_t *cnt = which == 0 ? b.n_a : b.n_b;
+    const fe_match *src = which == 0 ? b.match_a : b.match_b;
     { StageTimer t(c, ST_FINALIZE);
-      t.done(launch_pack_landmarks(g, P, b, cnt, which == 0 ? b.match_a : b.match_b, b.lm_lkp, b.lm_rkp, b.lm_ldesc, b.lm_rdesc,
-                                   b.lm_match, c->stream)); }
+      t.done(dim > 0 ? launch_pack_landmarks(g, P, b, cnt, src, b.lm_lkp, b.lm_rkp, dim, b.lm_lfdesc, b.lm_rfdesc, b.lm_match, c->stream)
+                     : launch_pack_landmarks(g, P, b, cnt, src, b.lm_lkp, b.lm_rkp, b.lm_ldesc, b.lm_rdesc, b.lm_match, c->stream)); }
     FE_CUDA(c, cudaGetLastError());
     FE_CUDA(c, cudaMemcpyAsync(c->h_counts, cnt, sizeof(uint32_t) * P, cudaMemcpyDeviceToHost, c->stream));
     FE_CUDA(c, cudaStreamSynchronize(c->stream));
@@ -1680,8 +1757,10 @@ int32_t fe_batch_landmarks(fe_ctx *c, int32_t which, int32_t cap, fe_kpoint *l_k
     if (mx > 0) {
         if (l_kps) FE_CUDA(c, cudaMemcpy2DAsync(l_kps, sizeof(fe_kpoint) * (size_t)cap, b.lm_lkp, sizeof(fe_kpoint) * C, sizeof(fe_kpoint) * (size_t)mx, P, cudaMemcpyDeviceToHost, c->stream));
         if (r_kps) FE_CUDA(c, cudaMemcpy2DAsync(r_kps, sizeof(fe_kpoint) * (size_t)cap, b.lm_rkp, sizeof(fe_kpoint) * C, sizeof(fe_kpoint) * (size_t)mx, P, cudaMemcpyDeviceToHost, c->stream));
-        if (l_desc) FE_CUDA(c, cudaMemcpy2DAsync(l_desc, (size_t)32 * cap, b.lm_ldesc, 32 * C, (size_t)32 * mx, P, cudaMemcpyDeviceToHost, c->stream));
-        if (r_desc) FE_CUDA(c, cudaMemcpy2DAsync(r_desc, (size_t)32 * cap, b.lm_rdesc, 32 * C, (size_t)32 * mx, P, cudaMemcpyDeviceToHost, c->stream));
+        const size_t row = dim > 0 ? sizeof(float) * dim : 32;     // descriptor bytes per landmark, packed on both sides
+        const void *ld = dim > 0 ? (const void *)b.lm_lfdesc : b.lm_ldesc, *rd = dim > 0 ? (const void *)b.lm_rfdesc : b.lm_rdesc;
+        if (l_desc) FE_CUDA(c, cudaMemcpy2DAsync(l_desc, row * cap, ld, row * C, row * mx, P, cudaMemcpyDeviceToHost, c->stream));
+        if (r_desc) FE_CUDA(c, cudaMemcpy2DAsync(r_desc, row * cap, rd, row * C, row * mx, P, cudaMemcpyDeviceToHost, c->stream));
         if (matches) FE_CUDA(c, cudaMemcpy2DAsync(matches, sizeof(fe_match) * (size_t)cap, b.lm_match, sizeof(fe_match) * C, sizeof(fe_match) * (size_t)mx, P, cudaMemcpyDeviceToHost, c->stream));
     }
     if ((r = sync_and_resolve(c)) != FE_OK) return r;

@@ -140,6 +140,10 @@ enum BufGroup : unsigned {
     GRP_SURFDET = 1u << 12,    // Fast-Hessian scale space
     GRP_LANDMARKS = 1u << 13,  // stereoLandmarks packing
     GRP_PYRAMID = 1u << 14,    // multi-level ORB
+    GRP_WFLOAT = 1u << 15,     // WindowMatcher over a resident SURF sequence: float landmark rows, 64-bit L2 keys
+    GRP_WFLIVE = 1u << 16,     // its liveGraph variant: right float rows and the right side's keys
+    GRP_WUFLOAT = 1u << 17,    // fe_window_update's current / previous float rows (SURF-64 / SURF-128)
+    GRP_LMFLOAT = 1u << 18,    // stereoLandmarks packing of SURF batches
 };
 
 // Every device buffer of a ctx, declared once: X(element type, name, scope, group, elements per unit).  The element count is
@@ -225,6 +229,13 @@ enum BufGroup : unsigned {
     X(uint8_t, wdesc_r, PER_IMAGE, GRP_WLIVE, 32 * g.kp_cap)       /* right descriptors of the landmarks */ \
     X(uint32_t, wbest_r, PER_PAIR, GRP_WLIVE, g.kp_cap)            /* row / column arg-mins of the right-descriptor cross-check */ \
     X(uint32_t, wcol_r, PER_PAIR, GRP_WLIVE, g.kp_cap) \
+    /* the same window over a SURF sequence: float rows at fdesc's 128-float stride, L2 keys (float bits of d^2 << 32 | index) */ \
+    X(float, wfdesc, PER_IMAGE, GRP_WFLOAT, 128 * g.kp_cap) \
+    X(unsigned long long, wbest64, PER_PAIR, GRP_WFLOAT, g.kp_cap)        /* row best (ratio) / row arg-min (cross-check) */ \
+    X(unsigned long long, wsecond64, PER_PAIR, GRP_WFLOAT, g.kp_cap)      /* row second (ratio) / column arg-min (cross-check) */ \
+    X(float, wfdesc_r, PER_IMAGE, GRP_WFLIVE, 128 * g.kp_cap)            /* right float rows of the landmarks */ \
+    X(unsigned long long, wbest64_r, PER_PAIR, GRP_WFLIVE, g.kp_cap)      /* row / column arg-mins of the right-row cross-check */ \
+    X(unsigned long long, wcol64_r, PER_PAIR, GRP_WFLIVE, g.kp_cap) \
     /* fe_window_update: the current (slot 0) and previous (slot 1) frame's landmark lists */ \
     X(fe_kpoint, wu_kp, PER_CTX, GRP_WUPDATE, 2 * g.kp_cap) \
     X(uint8_t, wu_desc, PER_CTX, GRP_WUPDATE, 64 * g.kp_cap) \
@@ -233,6 +244,8 @@ enum BufGroup : unsigned {
     X(float, wu_ky, PER_CTX, GRP_WUPDATE, 2 * g.kp_cap) \
     X(float2, wu_kcs, PER_CTX, GRP_WUPDATE, 2 * g.kp_cap)          /* scratch of the keypoint unpack */ \
     X(uint32_t, wu_n, PER_CTX, GRP_WUPDATE, 2) \
+    X(float, wu_fdesc, PER_CTX, GRP_WUFLOAT, 2 * 128 * g.kp_cap)        /* [2][kp_cap][128] left float rows */ \
+    X(float, wu_frdesc, PER_CTX, GRP_WUFLOAT, 2 * 128 * g.kp_cap)       /* [2][kp_cap][128] right float rows */ \
     /* Fast-Hessian scale space: [image of the pass][all layers back to back] */ \
     X(float, hes_det, PER_CTX, GRP_SURFDET, (size_t)std::min(g.n_images, HESSIAN_CHUNK_IMAGES) * g.w * g.h * 20) \
     X(float, hes_trace, PER_CTX, GRP_SURFDET, (size_t)std::min(g.n_images, HESSIAN_CHUNK_IMAGES) * g.w * g.h * 20) \
@@ -243,6 +256,8 @@ enum BufGroup : unsigned {
     X(uint8_t, lm_ldesc, PER_PAIR, GRP_LANDMARKS, 32 * g.kp_cap) \
     X(uint8_t, lm_rdesc, PER_PAIR, GRP_LANDMARKS, 32 * g.kp_cap) \
     X(fe_match, lm_match, PER_PAIR, GRP_LANDMARKS, g.kp_cap) \
+    X(float, lm_lfdesc, PER_PAIR, GRP_LMFLOAT, 128 * g.kp_cap)          /* rows of dim floats, packed (the host's layout) */ \
+    X(float, lm_rfdesc, PER_PAIR, GRP_LMFLOAT, 128 * g.kp_cap) \
     /* multi-level ORB: two ping-pong level images (level-1 geometry is the largest), coefficient table, accumulated results */ \
     X(uint8_t, pyr_img0, PER_IMAGE, GRP_PYRAMID, g.img_stride) \
     X(uint8_t, pyr_img1, PER_IMAGE, GRP_PYRAMID, g.img_stride) \
@@ -344,9 +359,15 @@ int launch_integral(const Geom &g, const Buffers &b, cudaStream_t s);
 // side 0: left keypoints / descriptors of the landmarks (queryIdx of matches_a); side 1: right descriptors (trainIdx), wkx / wky unused
 int launch_gather_landmarks(const Geom &g, int n_frames, const Buffers &b, int side, uint8_t *wdesc, float *wkx, float *wky,
                             uint32_t *wcount, cudaStream_t s);
+// SURF batches: the first dim (64 / 128) floats of the b.fdesc rows, to rows of 128 floats in wfdesc
+int launch_gather_landmarks(const Geom &g, int n_frames, const Buffers &b, int side, int dim, float *wfdesc, float *wkx,
+                            float *wky, uint32_t *wcount, cudaStream_t s);
 int launch_triangulate(const Geom &g, int n_frames, const Buffers &b, const double *Q, double *xyz, cudaStream_t s);
 int launch_pack_landmarks(const Geom &g, int n_pairs, const Buffers &b, const uint32_t *n_m, const fe_match *matches,
                           fe_kpoint *lkp, fe_kpoint *rkp, uint8_t *ldesc, uint8_t *rdesc, fe_match *out, cudaStream_t s);
+// SURF batches: rows of dim floats, packed (dim floats apart)
+int launch_pack_landmarks(const Geom &g, int n_pairs, const Buffers &b, const uint32_t *n_m, const fe_match *matches,
+                          fe_kpoint *lkp, fe_kpoint *rkp, int dim, float *ldesc, float *rdesc, fe_match *out, cudaStream_t s);
 
 // Row table of raster-ordered keypoint lists (match.cu): rowstart[image][r] = first index whose floor(y), clamped to
 // [0, h], is >= r, for r in [0, h + 1] (rowstart[h + 1] = n); h = Geom::rs_h.  The banded matchers read their candidate range from it instead of searching.
@@ -418,6 +439,10 @@ int launch_l2_verify(const Geom &g, int n_pairs, int dim, const Buffers &b, cons
 size_t l2_verify_list_entries(int kp_cap);
 int launch_l2_finalize_ratio(const Geom &g, int n_pairs, double ratio, const Buffers &b, const uint32_t *counts, cudaStream_t s);
 int launch_l2_finalize_cross(const Geom &g, int n_pairs, float max_dy, const Buffers &b, const uint32_t *counts, cudaStream_t s);
+// liveGraph on float rows: the 64-bit-key twin of launch_finalize_cross_both
+int launch_l2_finalize_cross_both(const Geom &g, int n_pairs, const uint32_t *counts, const unsigned long long *abL,
+                                  const unsigned long long *cbL, const unsigned long long *abR, const unsigned long long *cbR,
+                                  fe_match *out, uint32_t *n_out, cudaStream_t s);
 int launch_finalize_ratio(const Geom &g, int n_pairs, double ratio, const Buffers &b,
                           const uint32_t *counts, cudaStream_t s);
 int launch_finalize_cross(const Geom &g, int n_pairs, float max_dy, const Buffers &b,

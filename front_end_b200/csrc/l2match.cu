@@ -416,6 +416,42 @@ l2_finalize_cross_kernel(Geom g, float max_dy, const uint32_t *__restrict__ coun
     if (threadIdx.x == 0) n_out[pair] = offset;
 }
 
+// liveGraph's tracker on float rows (/root/reference src/front_end/algorithm.py:1160-1190), the 64-bit-key twin of match.cu's
+// finalize_cross_both_kernel: landmark i of the current frame continues landmark t of the previous one iff the row arg-mins
+// of the left and of the right rows both name t and both column arg-mins name i.  Left distance; ordered by i.
+__global__ void __launch_bounds__(LFIN)
+l2_finalize_cross_both_kernel(Geom g, const uint32_t *__restrict__ counts, const unsigned long long *__restrict__ abL,
+                              const unsigned long long *__restrict__ cbL, const unsigned long long *__restrict__ abR,
+                              const unsigned long long *__restrict__ cbR, fe_match *__restrict__ out, uint32_t *__restrict__ n_out) {
+    __shared__ uint32_t s_warp[33];
+    const int pair = blockIdx.x;
+    const int nq = min((int)counts[2 * pair], g.kp_cap), nt = min((int)counts[2 * pair + 1], g.kp_cap);
+    const size_t o0 = (size_t)pair * g.kp_cap;
+    fe_match *o = out + o0;
+    uint32_t offset = 0;
+    for (int base = 0; base < nq; base += LFIN) {
+        const int i = base + threadIdx.x;
+        bool good = false;
+        unsigned long long kl = KEY64_NONE;
+        if (i < nq && nt > 0) {
+            kl = abL[o0 + i];
+            const unsigned long long kr = abR[o0 + i];
+            const uint32_t tl = (uint32_t)(kl & 0xFFFFFFFFu), tr = (uint32_t)(kr & 0xFFFFFFFFu);
+            good = kl != KEY64_NONE && kr != KEY64_NONE && tl == tr && tl < (uint32_t)nt &&
+                   (uint32_t)(cbL[o0 + tl] & 0xFFFFFFFFu) == (uint32_t)i && (uint32_t)(cbR[o0 + tr] & 0xFFFFFFFFu) == (uint32_t)i;
+        }
+        uint32_t total;
+        const uint32_t pos = offset + block_excl_scan_1024b(good ? 1u : 0u, s_warp, total);
+        if (good) {
+            fe_match m;
+            m.queryIdx = (uint32_t)i; m.trainIdx = (uint32_t)(kl & 0xFFFFFFFFu); m.imgIdx = 0; m.distance = key_dist(kl);
+            o[pos] = m;
+        }
+        offset += total;
+    }
+    if (threadIdx.x == 0) n_out[pair] = offset;
+}
+
 template <int D>
 static void launch_l2_d(const Geom &g, int n_pairs, const MatchParams &mp, bool masked, bool all, const Buffers &b,
                         const uint32_t *counts, cudaStream_t s) {
@@ -451,6 +487,13 @@ int launch_l2_finalize_ratio(const Geom &g, int n_pairs, double ratio, const Buf
 
 int launch_l2_finalize_cross(const Geom &g, int n_pairs, float max_dy, const Buffers &b, const uint32_t *counts, cudaStream_t s) {
     l2_finalize_cross_kernel<<<n_pairs, LFIN, 0, s>>>(g, max_dy, counts, b.allbest64, b.colbest64, b.ky, b.match_b, b.n_b);
+    return 1;
+}
+
+int launch_l2_finalize_cross_both(const Geom &g, int n_pairs, const uint32_t *counts, const unsigned long long *abL,
+                                  const unsigned long long *cbL, const unsigned long long *abR, const unsigned long long *cbR,
+                                  fe_match *out, uint32_t *n_out, cudaStream_t s) {
+    l2_finalize_cross_both_kernel<<<n_pairs, LFIN, 0, s>>>(g, counts, abL, cbL, abR, cbR, out, n_out);
     return 1;
 }
 

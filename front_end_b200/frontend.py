@@ -13,6 +13,7 @@ import numpy as np
 from . import lib as L
 
 _lib = None
+_SURF_DIM = {L.DESC_SURF64: 64, L.DESC_SURF128: 128}       # float row width of the SURF descriptor kinds
 
 
 def get_lib():
@@ -196,16 +197,23 @@ class FrontEnd:
     # -- srv/windowMatching.srv: the stateful window (WindowMatcher.cpp:92-102 / the Python window service) ----------
     def window_update(self, l_kps=None, l_desc=None, r_desc=None, cfg=None, reset=False, length=0, variant=0, kind=L.DESC_ORB256):
         """Returns (tracks, frames_in_window).  cfg: ratio + MASK_WINDOW (WindowMatcher) or cross-check + MASK_NONE
-        (liveGraph: needs r_desc).  reset=True clears the window."""
+        (liveGraph: needs r_desc); its norm defaults to NORM_L2 for DESC_SURF64 / DESC_SURF128 rows ((n, 64) / (n, 128)
+        float32), Hamming otherwise.  Switching between binary, SURF-64 and SURF-128 rows needs a reset first.
+        reset=True clears the window."""
         nt, fr = C.c_int32(), C.c_int32()
         wc = L.WindowCfg(length, variant)
         if reset:
             self._check(self.lib.fe_window_update(self.h, 1, None, None, None, 0, kind, None, C.byref(wc), None, 0, C.byref(nt), C.byref(fr)))
             return np.zeros(0, L.MATCH), 0
-        cfg = cfg or L.match_cfg(mask=L.MASK_WINDOW)
+        dim = _SURF_DIM.get(kind, 0)
+        cfg = cfg or L.match_cfg(mask=L.MASK_WINDOW, norm=L.NORM_L2 if dim else L.NORM_HAMMING)
         l_kps = np.ascontiguousarray(l_kps, dtype=L.KPOINT)
         l_desc = np.ascontiguousarray(l_desc)
         r_desc = np.ascontiguousarray(r_desc) if r_desc is not None else None
+        if dim:
+            for d in (l_desc, r_desc):
+                if d is not None and (d.dtype != np.float32 or d.shape != (len(l_kps), dim)):
+                    raise ValueError("SURF-%d rows: expected a (%d, %d) float32 array" % (dim, len(l_kps), dim))
         cap = max(len(l_kps), 1)
         out = np.zeros(cap, L.MATCH)
         self._check(self.lib.fe_window_update(self.h, 0, _ptr(l_kps), _ptr(l_desc), _ptr(r_desc), len(l_kps), kind, C.byref(cfg),
@@ -230,8 +238,10 @@ class FrontEnd:
 
     def window_batch(self, cfg=None, Q=None, cap=None, out=None):
         """WindowMatcher over the resident sequence (call after batch_run / pipeline_batch with a ratio cfg_a on
-        consecutive frames).  Returns (tracks [F-1][cap], n_tracks [F-1], xyz [F][cap][3] or None)."""
-        cfg = cfg or L.match_cfg(mask=L.MASK_WINDOW)
+        consecutive frames; the default cfg matches SURF batches with NORM_L2).  Returns (tracks [F-1][cap],
+        n_tracks [F-1], xyz [F][cap][3] or None)."""
+        surf = getattr(self, "_batch_kind", L.DESC_ORB256) in _SURF_DIM
+        cfg = cfg or L.match_cfg(mask=L.MASK_WINDOW, norm=L.NORM_L2 if surf else L.NORM_HAMMING)
         cap = cap or self.max_keypoints
         F = self._n_pairs
         if out is not None:                       # caller-owned (e.g. pinned) result buffers: (tracks [>= F-1][cap], n [>= F-1])
@@ -278,11 +288,14 @@ class FrontEnd:
         self._check(self.lib.fe_set_orb_patch_size(self.h, patch_size))
 
     def batch_landmarks(self, which=0, cap=None):
-        """stereoLandmarks of every resident pair (algorithm.py:893-913): dict(l_kps, l_desc, r_kps, r_desc, matches, n)."""
+        """stereoLandmarks of every resident pair (algorithm.py:893-913): dict(l_kps, l_desc, r_kps, r_desc, matches, n).
+        Descriptor rows: (P, cap, 32) uint8 for ORB-256 batches, (P, cap, 64 / 128) float32 for SURF-64 / SURF-128."""
         cap = cap or self.max_keypoints
         P = self._n_pairs
+        dim = _SURF_DIM.get(getattr(self, "_batch_kind", L.DESC_ORB256), 0)
+        dw, dt = (dim, np.float32) if dim else (32, np.uint8)
         out = dict(l_kps=np.zeros((P, cap), L.KPOINT), r_kps=np.zeros((P, cap), L.KPOINT),
-                   l_desc=np.zeros((P, cap, 32), np.uint8), r_desc=np.zeros((P, cap, 32), np.uint8),
+                   l_desc=np.zeros((P, cap, dw), dt), r_desc=np.zeros((P, cap, dw), dt),
                    matches=np.zeros((P, cap), L.MATCH), n=np.zeros(P, np.int32))
         self._check(self.lib.fe_batch_landmarks(self.h, which, cap, _ptr(out["l_kps"]), _ptr(out["l_desc"]), _ptr(out["r_kps"]),
                                                 _ptr(out["r_desc"]), _ptr(out["matches"]), _ptr(out["n"])))

@@ -26,7 +26,8 @@
 extern "C" {
 #endif
 
-#define FE_ABI_VERSION 6   /* 6: fe_set_freak, FE_DESC_FREAK, 64-byte rows through the matchers (additive) */
+#define FE_ABI_VERSION 6   /* 6: fe_set_freak, FE_DESC_FREAK, 64-byte rows through the matchers; SURF rows in fe_window_batch,
+                              fe_window_update and fe_batch_landmarks, whose l_desc / r_desc became void * (all additive) */
 
 /* ---- wire-compatible PODs ------------------------------------------------------------------ */
 
@@ -214,7 +215,11 @@ int32_t fe_describe(fe_ctx *ctx, const uint8_t *img, int32_t width, int32_t heig
  * wc (optional): window length and erase rule -- variant 0: C++ node, length = nWindow (`if size >= nWindow erase`:
  * nWindow - 1 frames stay; default 3 = `WindowMatcher slidingWindow(3)`, src/front_end_window_node.cpp:6), variant 1:
  * Python service (`if len >= length + 1: del [0]`, default length 2).  frames_in_window: window size after this update.  Tracks:
- * queryIdx = landmark of the new frame, trainIdx = landmark of the previous frame, ordered by queryIdx. */
+ * queryIdx = landmark of the new frame, trainIdx = landmark of the previous frame, ordered by queryIdx.
+ * desc_kind FE_DESC_ORB256 / BRIEF16 / BRIEF32 (n x 32 / 16 u8 rows) with FE_NORM_HAMMING / HAMMING2, or FE_DESC_SURF64 /
+ * SURF128 (n x 64 / 128 f32 rows) with FE_NORM_L2 (WindowMatcher.cpp:150-153's knnMatch, "Hamming-256 or L2-128"); every
+ * frame of a window has rows of one kind: an update whose rows differ in kind (binary, SURF-64, SURF-128) from the previous
+ * frame's fails with FE_ERR_BAD_ARG and leaves the window unchanged -- reset first. */
 typedef struct fe_window_cfg {
     int32_t length;     /* nWindow (variant 0, <= 0 -> 3) / length (variant 1, <= 0 -> 2) */
     int32_t variant;    /* 0 = WindowMatcher.cpp, 1 = Python window service */
@@ -305,9 +310,11 @@ int32_t fe_set_batch_descriptor(fe_ctx *ctx, int32_t desc_kind);
  * f = 1 .. F-1, landmarks(f) are matched against landmarks(f-1): search-box mask on the LEFT keypoint coordinates
  * (:104-128), left descriptors (:134-148), kNN-2 (:150-153), Lowe ratio with singleton acceptance (:161-224).
  * tracks[(f-1)*cap + i] (queryIdx = landmark index in frame f, trainIdx = landmark index in frame f-1, :227-231),
- * n_tracks[f-1].  cfg: mode FE_MATCH_RATIO, mask FE_MASK_WINDOW, norm FE_NORM_HAMMING -- or mode FE_MATCH_CROSSCHECK with
- * FE_MASK_NONE for liveGraph's tracker (src/front_end/algorithm.py:1160-1190: cross-check of the left AND of the right
- * descriptors of consecutive frames, intersected on the same previous landmark).
+ * n_tracks[f-1].  cfg: mode FE_MATCH_RATIO, mask FE_MASK_WINDOW -- or mode FE_MATCH_CROSSCHECK with FE_MASK_NONE for
+ * liveGraph's tracker (src/front_end/algorithm.py:1160-1190: cross-check of the left AND of the right descriptors of
+ * consecutive frames, intersected on the same previous landmark, no |dy| filter).  norm: FE_NORM_HAMMING / HAMMING2 on an
+ * ORB-256 batch, FE_NORM_L2 on a SURF-64 / SURF-128 batch (fe_set_batch_descriptor; exact FP32 distances, the liveGraph
+ * mode by two all-pairs passes); a norm that does not fit the batch's descriptor is FE_ERR_UNSUPPORTED.
  * Optional triangulation (:36-51): Q = 4x4 row-major reprojection matrix, xyz[(f*cap + i)*3 .. +3] =
  * (Q [xl, yl, xl - xr, 1]^T)_{0..2} / (1000 * (.)_3) for landmark i of frame f; pass NULL, NULL to skip. */
 int32_t fe_window_batch(fe_ctx *ctx, const fe_match_cfg *cfg, const double *Q, int32_t cap, fe_match *tracks,
@@ -342,9 +349,10 @@ int32_t fe_set_orb_patch_size(fe_ctx *ctx, int32_t patch_size);
 /* srv/stereoMatching.srv's reply for every pair of the resident batch: msg/stereoLandmarks.msg as algorithm_one packs it
  * (src/front_end/algorithm.py:893-913) -- row i of the left / right keypoint and descriptor arrays are the two ends of
  * match i, and matches[i] = {i, i, 0, distance}.  which: 0 = the ratio matches (cfg_a), 1 = the cross-check matches.
- * Slabs of `cap` rows per pair; n[p] = landmarks of pair p.  Any output pointer may be NULL.  ORB-256 batches. */
-int32_t fe_batch_landmarks(fe_ctx *ctx, int32_t which, int32_t cap, fe_kpoint *l_kps, uint8_t *l_desc, fe_kpoint *r_kps,
-                           uint8_t *r_desc, fe_match *matches, int32_t *n);
+ * Slabs of `cap` rows per pair; n[p] = landmarks of pair p.  Any output pointer may be NULL.  Descriptor rows per batch
+ * descriptor: 32 u8 (ORB-256), 64 f32 (SURF-64), 128 f32 (SURF-128), packed (row p * cap + i). */
+int32_t fe_batch_landmarks(fe_ctx *ctx, int32_t which, int32_t cap, fe_kpoint *l_kps, void *l_desc, fe_kpoint *r_kps,
+                           void *r_desc, fe_match *matches, int32_t *n);
 
 /* Pairs per chunk of fe_pipeline_batch's overlapped path (0 = the default, 48; batches of fewer than 2 chunks run
  * on the single-stream path).  A tuning knob: results do not depend on it. */

@@ -48,6 +48,8 @@ struct fe_ctx {
     int patch_size = 31;              // ORB patchSize (fe_set_orb_patch_size); != 31 selects the generated pattern
     int chunk_pairs = 0;              // pairs per chunk of the overlapped pipeline (fe_set_chunk_pairs); 0 = default
     int batch_desc = FE_DESC_ORB256;  // what the batched pipeline describes with (fe_set_batch_descriptor)
+    bool hessian = false;             // the batched pipeline detects with SURF's Fast-Hessian detector (fe_set_batch_detector)
+    fe_surf_params surf{};            // its parameters
     int wu_frames = 0, wu_prev_n = 0;  // fe_window_update: frames in the window, landmarks of the previous frame
     bool wu_prev_sorted = true;
     int wu_dim = 0;                    // rows of the frames in the window: 0 = binary, 64 / 128 = SURF floats
@@ -391,6 +393,15 @@ int desc_dim(int kind) { return kind == FE_DESC_SURF64 ? 64 : kind == FE_DESC_SU
 int brief_width(int kind) { return kind == FE_DESC_BRIEF16 ? 16 : kind == FE_DESC_BRIEF32 ? 32 : kind == FE_DESC_BRIEF64 ? 64 : 0; }
 int brief_slot(int kind) { return kind - FE_DESC_BRIEF16; }
 
+// What rows the batch holds: SURF-64 / SURF-128 per fe_surf_params.extended when it detects with the Fast-Hessian detector,
+// else what fe_set_batch_descriptor selected.
+int batch_rows(const fe_ctx *c) { return c->hessian ? (c->surf.extended ? FE_DESC_SURF128 : FE_DESC_SURF64) : c->batch_desc; }
+// Whether the SURF rows of the batch are upright (no orientation, no integral image for it)
+bool batch_upright(const fe_ctx *c) { return c->hessian ? c->surf.upright != 0 : c->cfg.surf_upright != 0; }
+// Whether every image's keypoints are in raster order: always with the Fast-Hessian detector, else without a pyramid (the
+// pyramid's keypoints are level-major)
+bool batch_raster(const fe_ctx *c) { return c->hessian || c->nlevels == 1; }
+
 // (g, b, st): the batch -- or the chunk view of it -- to match; timed = false on the auxiliary streams of the chunked pipeline.
 // Needs the groups of match_groups(dim, cfg_b != nullptr).
 int run_match_l2_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bool timed, int n_pairs, int dim,
@@ -495,10 +506,92 @@ int run_match_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bo
 // Checks the match configs against the batch descriptor and allocates what run_batch_on reads beyond the core buffers.  Runs
 // before any view of the buffers is taken, and its zero-fills are on the ctx stream.
 int prepare_batch(fe_ctx *c, const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b) {
-    const int dim = desc_dim(c->batch_desc);
+    const int dim = desc_dim(batch_rows(c));
     if (dim > 0 && ((cfg_a && cfg_a->norm != FE_NORM_L2) || (cfg_b && cfg_b->norm != FE_NORM_L2)))
         return fail(c, FE_ERR_UNSUPPORTED, "SURF descriptors are matched with FE_NORM_L2");
-    return ensure(c, match_groups(dim, cfg_b != nullptr) | (dim > 0 && !c->cfg.surf_upright ? GRP_INTEGRAL : 0u));
+    const unsigned hessian = c->hessian ? GRP_INTEGRAL | GRP_SURFDET : 0u;      // the scale space reads the integral image
+    return ensure(c, match_groups(dim, cfg_b != nullptr) | (dim > 0 && !batch_upright(c) ? GRP_INTEGRAL : 0u) | hessian);
+}
+
+// cv::SURF's Fast-Hessian detector (src/surf.cpp:462-512) on the images of (g, b) in b.img: integral image, scale-space layers
+// and maxima, HESSIAN_CHUNK_IMAGES images per pass through the one scale space of the ctx.  Leaves the unsorted maxima in
+// b.hes_kp and their counts (which may exceed kp_cap) in b.hes_count.  max_win (optional): the largest descriptor window
+// (int)(21 * size * 1.2 / 9) a keypoint of this layer schedule can have -- an interpolated maximum of a middle layer is no
+// larger than the layer above it -- so that a caller can pick the descriptor variant without reading anything back.
+// Needs GRP_INTEGRAL and GRP_SURFDET.  Used by fe_surf_detect_* and by the batched pipeline (fe_set_batch_detector).
+int hessian_detect(fe_ctx *c, const Geom &g, const Buffers &b, const fe_surf_params *sp, cudaStream_t st, bool timed, int *max_win) {
+    const int nOct = sp->n_octaves > 0 ? sp->n_octaves : 4, nLay = sp->n_octave_layers > 0 ? sp->n_octave_layers : 2;
+    const int R = g.h, C = g.w, stride_i = g.w + 1;        // the integral image is (h + 1) x (w + 1)
+    const int n_images = g.n_images;
+    const size_t MI = c->cfg.max_images;
+    // layer schedule
+    const int nTotal = (nLay + 2) * nOct;
+    std::vector<int> sizes(nTotal), steps(nTotal);
+    std::vector<size_t> offs(nTotal + 1, 0);
+    for (int o = 0, idx = 0, step = 1; o < nOct; ++o, step *= 2)
+        for (int l = 0; l < nLay + 2; ++l, ++idx) {
+            sizes[idx] = (9 + 6 * l) << o;
+            steps[idx] = step;
+            offs[idx + 1] = offs[idx] + (size_t)(R / step) * (size_t)(C / step);
+        }
+    const size_t per_image = (size_t)c->cfg.max_width * c->cfg.max_height * 10 * 2;     // floats of scale space per image (capacity)
+    const int IC = std::min(c->cfg.max_images, HESSIAN_CHUNK_IMAGES);                       // images per scale-space chunk
+    if (offs[nTotal] > per_image)
+        return fail(c, FE_ERR_CAPACITY, "fe_surf_detect: too many octave layers for the scale-space buffer");
+    { StageTimer t(c, ST_SURF, st, timed); t.done(launch_integral(g, b, st)); }
+    FE_CUDA(c, cudaMemsetAsync(b.hes_count, 0, sizeof(uint32_t) * 2 * MI, st));
+    static const int DX[3][5] = {{0, 2, 3, 7, 1}, {3, 2, 6, 7, -2}, {6, 2, 9, 7, 1}};
+    static const int DY[3][5] = {{2, 0, 7, 3, 1}, {2, 3, 7, 6, -2}, {2, 6, 7, 9, 1}};
+    static const int DXY[4][5] = {{1, 1, 4, 4, 1}, {5, 1, 8, 4, -1}, {1, 5, 4, 8, -1}, {5, 5, 8, 8, 1}};
+    auto resize_box = [](const int *src, int size) {      // resizeHaarPattern, src/surf.cpp:136-152
+        const float ratio = (float)size / 9;
+        HaarBoxI o;
+        o.dx1 = cv_round_f(ratio * src[0]); o.dy1 = cv_round_f(ratio * src[1]);
+        o.dx2 = cv_round_f(ratio * src[2]); o.dy2 = cv_round_f(ratio * src[3]);
+        o.w = src[4] / ((float)(o.dx2 - o.dx1) * (o.dy2 - o.dy1));
+        return o;
+    };
+    const size_t s_img = (size_t)(g.h + 1) * (g.w + 1);
+    int win = 1;
+    for (int c0 = 0; c0 < n_images; c0 += IC) {
+        const int ic = std::min(IC, n_images - c0);
+        {
+            StageTimer t(c, ST_FAST, st, timed);
+            int nl = 0;
+            for (int i = 0; i < nTotal; ++i) {
+                HessianLayer hl{};
+                hl.size = sizes[i]; hl.step = steps[i];
+                hl.valid = !(sizes[i] > R || sizes[i] > C);
+                hl.samples_i = hl.valid ? 1 + (R - sizes[i]) / steps[i] : 0;
+                hl.samples_j = hl.valid ? 1 + (C - sizes[i]) / steps[i] : 0;
+                hl.margin = (sizes[i] / 2) / steps[i];
+                for (int k = 0; k < 3; ++k) { hl.box[k] = resize_box(DX[k], sizes[i]); hl.box[3 + k] = resize_box(DY[k], sizes[i]); }
+                for (int k = 0; k < 4; ++k) hl.box[6 + k] = resize_box(DXY[k], sizes[i]);
+                nl += launch_hessian_layer(b.integral + (size_t)c0 * s_img, s_img, stride_i, R, C, hl, b.hes_det + offs[i], b.hes_trace + offs[i],
+                                           per_image, ic, st);
+            }
+            t.done(nl);
+        }
+        {
+            StageTimer t(c, ST_SELECT, st, timed);
+            int nl = 0;
+            for (int o = 0; o < nOct; ++o)
+                for (int l = 1; l <= nLay; ++l) {
+                    const int idx = o * (nLay + 2) + l, step = steps[idx];
+                    const int rows = R / step, cols = C / step;
+                    const int margin = (sizes[idx + 1] / 2) / step + 1;
+                    const int n = launch_hessian_maxima(b.hes_det + offs[idx - 1], b.hes_det + offs[idx], b.hes_det + offs[idx + 1],
+                                                        b.hes_trace + offs[idx], per_image, rows, cols, margin, sizes[idx], sizes[idx - 1],
+                                                        step, o, sp->hessian_threshold, b.hes_kp + (size_t)c0 * g.kp_cap, g.kp_cap,
+                                                        b.hes_count + c0, ic, st);
+                    if (n) win = std::max(win, (int)(21.f * ((float)sizes[idx + 1] * 1.2f / 9.0f)));
+                    nl += n;
+                }
+            t.done(nl);
+        }
+    }
+    if (max_win) *max_win = win;
+    return FE_OK;
 }
 
 // Detect, describe and match the batch (g, b) on st: the resident batch, or a chunk view of it.  ORB-256 with Hamming
@@ -506,13 +599,22 @@ int prepare_batch(fe_ctx *c, const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_
 // pending detection changes and calls prepare_batch; the pyramid (nlevels > 1) runs on the whole resident batch only.
 int run_batch_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bool timed, int n_pairs,
                  const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b) {
-    const int dim = desc_dim(c->batch_desc);
-    const bool sorted = c->nlevels == 1;          // the pyramid's keypoints are level-major, not in raster order
-    int r = sorted ? run_detect_on(c, g, b, st, dim == 0, timed) : run_detect_pyramid(c, dim == 0);
-    if (r != FE_OK) return r;
-    if (dim > 0) {
-        StageTimer t(c, ST_SURF, st, timed);
-        t.done(launch_surf(g, b, b.n_kp, dim == 128, c->cfg.surf_upright != 0, detected_surf_win(c), st));
+    const int dim = desc_dim(batch_rows(c));
+    const bool sorted = batch_raster(c);
+    if (c->hessian) {
+        // Fast-Hessian maxima -> the survivors in raster order -> descriptors; nothing returns to the host
+        int max_win = 0;
+        int r = hessian_detect(c, g, b, &c->surf, st, timed, &max_win);
+        if (r != FE_OK) return r;
+        { StageTimer t(c, ST_SELECT, st, timed); t.done(launch_surf_raster(g, b.hes_kp, b.hes_count, batch_upright(c), b, st)); }
+        { StageTimer t(c, ST_SURF, st, timed); t.done(launch_surf(g, b, b.n_kp, dim == 128, batch_upright(c), max_win, st)); }
+    } else {
+        int r = sorted ? run_detect_on(c, g, b, st, dim == 0, timed) : run_detect_pyramid(c, dim == 0);
+        if (r != FE_OK) return r;
+        if (dim > 0) {
+            StageTimer t(c, ST_SURF, st, timed);
+            t.done(launch_surf(g, b, b.n_kp, dim == 128, batch_upright(c), detected_surf_win(c), st));
+        }
     }
     if (!cfg_a && !cfg_b) return FE_OK;
     if (dim > 0) return run_match_l2_on(c, g, b, st, timed, n_pairs, dim, cfg_a, cfg_b, b.n_kp, sorted);
@@ -561,7 +663,7 @@ int download_pairs(fe_ctx *c, int p0, int np, cudaStream_t st, const HostBatch &
         if (o.n_a) o.n_a[p] = (int32_t)hc[NI + p];
         if (o.n_b) o.n_b[p] = (int32_t)hc[NI + NP + p];
     }
-    const int dim = desc_dim(c->batch_desc);
+    const int dim = desc_dim(batch_rows(c));
     const size_t drow = dim > 0 ? sizeof(float) * dim : 32;       // descriptor bytes per keypoint on the host
     c->d2h_bytes += (int64_t)sizeof(uint32_t) * 2 * ni + (o.kps ? (int64_t)sizeof(fe_kpoint) * max_kp * ni : 0) +
                     (o.desc ? (int64_t)drow * max_kp * ni : 0) + (o.ma ? (int64_t)sizeof(fe_match) * max_a * np : 0) +
@@ -953,72 +1055,9 @@ static int surf_detect_impl(fe_ctx *c, int n_images, const uint8_t *imgs, int w,
     if ((r = ensure(c, GRP_FLOAT | GRP_INTEGRAL | GRP_SURFDET)) != FE_OK) return r;
     const Geom &g = c->g;
     Buffers &b = c->b;
-    const int R = h, C = w, stride_i = w + 1;              // the integral image is (h + 1) x (w + 1)
     const size_t MI = c->cfg.max_images;
-    // layer schedule
-    const int nTotal = (nLay + 2) * nOct;
-    std::vector<int> sizes(nTotal), steps(nTotal);
-    std::vector<size_t> offs(nTotal + 1, 0);
-    for (int o = 0, idx = 0, step = 1; o < nOct; ++o, step *= 2)
-        for (int l = 0; l < nLay + 2; ++l, ++idx) {
-            sizes[idx] = (9 + 6 * l) << o;
-            steps[idx] = step;
-            offs[idx + 1] = offs[idx] + (size_t)(R / step) * (size_t)(C / step);
-        }
-    const size_t per_image = (size_t)c->cfg.max_width * c->cfg.max_height * 10 * 2;     // floats of scale space per image (capacity)
-    const int IC = std::min(c->cfg.max_images, HESSIAN_CHUNK_IMAGES);                       // images per scale-space chunk
-    if (offs[nTotal] > per_image)
-        return fail(c, FE_ERR_CAPACITY, "fe_surf_detect: too many octave layers for the scale-space buffer");
     { StageTimer t(c, ST_H2D); if ((r = upload_images(c, imgs, n_images, stride, 0, 1)) != FE_OK) return r; t.done(0); }
-    { StageTimer t(c, ST_SURF); t.done(launch_integral(g, b, c->stream)); }
-    FE_CUDA(c, cudaMemsetAsync(b.hes_count, 0, sizeof(uint32_t) * 2 * MI, c->stream));
-    static const int DX[3][5] = {{0, 2, 3, 7, 1}, {3, 2, 6, 7, -2}, {6, 2, 9, 7, 1}};
-    static const int DY[3][5] = {{2, 0, 7, 3, 1}, {2, 3, 7, 6, -2}, {2, 6, 7, 9, 1}};
-    static const int DXY[4][5] = {{1, 1, 4, 4, 1}, {5, 1, 8, 4, -1}, {1, 5, 4, 8, -1}, {5, 5, 8, 8, 1}};
-    auto resize_box = [](const int *src, int size) {      // resizeHaarPattern, src/surf.cpp:136-152
-        const float ratio = (float)size / 9;
-        HaarBoxI o;
-        o.dx1 = cv_round_f(ratio * src[0]); o.dy1 = cv_round_f(ratio * src[1]);
-        o.dx2 = cv_round_f(ratio * src[2]); o.dy2 = cv_round_f(ratio * src[3]);
-        o.w = src[4] / ((float)(o.dx2 - o.dx1) * (o.dy2 - o.dy1));
-        return o;
-    };
-    const size_t s_img = (size_t)(g.h + 1) * (g.w + 1);
-    for (int c0 = 0; c0 < n_images; c0 += IC) {
-        const int ic = std::min(IC, n_images - c0);
-        {
-            StageTimer t(c, ST_FAST);
-            int nl = 0;
-            for (int i = 0; i < nTotal; ++i) {
-                HessianLayer hl{};
-                hl.size = sizes[i]; hl.step = steps[i];
-                hl.valid = !(sizes[i] > R || sizes[i] > C);
-                hl.samples_i = hl.valid ? 1 + (R - sizes[i]) / steps[i] : 0;
-                hl.samples_j = hl.valid ? 1 + (C - sizes[i]) / steps[i] : 0;
-                hl.margin = (sizes[i] / 2) / steps[i];
-                for (int k = 0; k < 3; ++k) { hl.box[k] = resize_box(DX[k], sizes[i]); hl.box[3 + k] = resize_box(DY[k], sizes[i]); }
-                for (int k = 0; k < 4; ++k) hl.box[6 + k] = resize_box(DXY[k], sizes[i]);
-                nl += launch_hessian_layer(b.integral + (size_t)c0 * s_img, s_img, stride_i, R, C, hl, b.hes_det + offs[i], b.hes_trace + offs[i],
-                                           per_image, ic, c->stream);
-            }
-            t.done(nl);
-        }
-        {
-            StageTimer t(c, ST_SELECT);
-            int nl = 0;
-            for (int o = 0; o < nOct; ++o)
-                for (int l = 1; l <= nLay; ++l) {
-                    const int idx = o * (nLay + 2) + l, st = steps[idx];
-                    const int rows = R / st, cols = C / st;
-                    const int margin = (sizes[idx + 1] / 2) / st + 1;
-                    nl += launch_hessian_maxima(b.hes_det + offs[idx - 1], b.hes_det + offs[idx], b.hes_det + offs[idx + 1],
-                                                b.hes_trace + offs[idx], per_image, rows, cols, margin, sizes[idx], sizes[idx - 1], st, o,
-                                                sp->hessian_threshold, b.hes_kp + (size_t)c0 * g.kp_cap, g.kp_cap, b.hes_count + c0, ic,
-                                                c->stream);
-                }
-            t.done(nl);
-        }
-    }
+    if ((r = hessian_detect(c, g, b, sp, c->stream, true, nullptr)) != FE_OK) return r;
     // std::sort(keypoints, KeypointGreater()) -- src/surf.cpp:445-460,511 -- as a rank sort on the device
     { StageTimer t(c, ST_SELECT); t.done(launch_surf_rank_sort(b.hes_kp, b.kp, b.hes_count, g.kp_cap, b.hes_count + MI, n_images, c->stream)); }
     FE_CUDA(c, cudaGetLastError());
@@ -1543,8 +1582,8 @@ static int window_batch_l2(fe_ctx *c, const Geom &g, const Geom &gv, const fe_ma
         FE_CUDA(c, cudaGetLastError());
         return FE_OK;
     }
-    // landmarks inherit the left keypoints' order: raster order only without a pyramid (level-major otherwise)
-    return run_match_l2_on(c, gv, v, c->stream, true, V, dim, cfg, nullptr, b.wcount, c->nlevels == 1);
+    // landmarks inherit the left keypoints' order
+    return run_match_l2_on(c, gv, v, c->stream, true, V, dim, cfg, nullptr, b.wcount, batch_raster(c));
 }
 
 // WindowMatcher::newStereo matching stage for a whole resident sequence (src/WindowMatcher.cpp:75-231).
@@ -1552,9 +1591,9 @@ int32_t fe_window_batch(fe_ctx *c, const fe_match_cfg *cfg, const double *Q, int
                         int32_t *n_tracks, double *xyz) {
     if (!c || !cfg || cap < 0 || (cap > 0 && !tracks) || !n_tracks) return fail(c, FE_ERR_BAD_ARG, "fe_window_batch: bad argument");
     if (c->g.n_images < 4) return fail(c, FE_ERR_BAD_ARG, "fe_window_batch: run fe_batch_run on at least two frames first");
-    const int dim = desc_dim(c->batch_desc);     // SURF-64 / SURF-128 batches: float rows and FE_NORM_L2
+    const int rows = batch_rows(c), dim = desc_dim(rows);     // SURF-64 / SURF-128 batches: float rows and FE_NORM_L2
     const bool hamming = cfg->norm == FE_NORM_HAMMING || cfg->norm == FE_NORM_HAMMING2;
-    if (dim == 0 && (!hamming || c->batch_desc != FE_DESC_ORB256))
+    if (dim == 0 && (!hamming || rows != FE_DESC_ORB256))
         return fail(c, FE_ERR_UNSUPPORTED, "fe_window_batch: ORB-256 sequences are matched with FE_NORM_HAMMING / FE_NORM_HAMMING2");
     if (dim > 0 && cfg->norm != FE_NORM_L2) return fail(c, FE_ERR_UNSUPPORTED, "fe_window_batch: SURF sequences are matched with FE_NORM_L2");
     const bool live = cfg->mode == FE_MATCH_CROSSCHECK;       // liveGraph variant (algorithm.py:1160-1190)
@@ -1589,8 +1628,8 @@ int32_t fe_window_batch(fe_ctx *c, const fe_match_cfg *cfg, const double *Q, int
               t.done(launch_finalize_cross_both(gv, V, b.wcount, b.wbest, b.wsecond, b.wbest_r, b.wcol_r, b.wmatch, b.wn, c->stream)); }
             FE_CUDA(c, cudaGetLastError());
         } else {
-            // landmarks inherit the left keypoints' order: raster order only without a pyramid (level-major otherwise)
-            r = run_match_on(c, gv, v, c->stream, true, V, cfg, nullptr, b.wcount, c->nlevels == 1, false);
+            // landmarks inherit the left keypoints' order
+            r = run_match_on(c, gv, v, c->stream, true, V, cfg, nullptr, b.wcount, batch_raster(c), false);
         }
     }
     if (r != FE_OK) return r;
@@ -1730,8 +1769,8 @@ int32_t fe_batch_landmarks(fe_ctx *c, int32_t which, int32_t cap, fe_kpoint *l_k
                            void *r_desc, fe_match *matches, int32_t *n) {
     if (!c || !n || cap < 0 || (which != 0 && which != 1)) return fail(c, FE_ERR_BAD_ARG, "fe_batch_landmarks: bad argument");
     if (c->g.n_images < 2) return fail(c, FE_ERR_BAD_ARG, "fe_batch_landmarks: run fe_batch_run first");
-    const int dim = desc_dim(c->batch_desc);     // SURF batches: rows of dim floats
-    if (c->batch_desc != FE_DESC_ORB256 && dim == 0) return fail(c, FE_ERR_UNSUPPORTED, "fe_batch_landmarks: ORB-256 or SURF batches");
+    const int rows = batch_rows(c), dim = desc_dim(rows);     // SURF batches: rows of dim floats
+    if (rows != FE_DESC_ORB256 && dim == 0) return fail(c, FE_ERR_UNSUPPORTED, "fe_batch_landmarks: ORB-256 or SURF batches");
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     const Geom &g = c->g;
     const int P = g.n_images / 2;
@@ -1867,10 +1906,29 @@ int32_t fe_set_chunk_pairs(fe_ctx *c, int32_t pairs) {
 
 int32_t fe_set_batch_descriptor(fe_ctx *c, int32_t desc_kind) {
     if (!c) return FE_ERR_BAD_ARG;
+    if (c->hessian)
+        return fail(c, FE_ERR_UNSUPPORTED, "fe_set_batch_descriptor: the Fast-Hessian batch describes with SURF (fe_set_batch_detector(ctx, NULL) first)");
     if (desc_kind != FE_DESC_ORB256 && desc_dim(desc_kind) == 0) return fail(c, FE_ERR_BAD_ARG, "unknown descriptor kind");
     if (desc_dim(desc_kind) > 0 && detected_surf_win(c) > SURF_DIRECT_MAX_WIN)
         return fail(c, FE_ERR_UNSUPPORTED, "SURF keypoint size not supported");
     c->batch_desc = desc_kind;
+    return FE_OK;
+}
+
+int32_t fe_set_batch_detector(fe_ctx *c, const fe_surf_params *surf) {
+    if (!c) return FE_ERR_BAD_ARG;
+    if (!surf) {      // back to FAST / ORB: fe_config, the fe_set_orb_* settings and the batch descriptor were never changed
+        c->hessian = false;
+        return FE_OK;
+    }
+    const int nOct = surf->n_octaves > 0 ? surf->n_octaves : 4, nLay = surf->n_octave_layers > 0 ? surf->n_octave_layers : 2;
+    if (nOct > 8 || nLay > 8) return fail(c, FE_ERR_BAD_ARG, "fe_set_batch_detector: at most 8 octaves / 8 layers");
+    int smem_max = 0;
+    FE_CUDA(c, cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->cfg.device));
+    if (surf_raster_smem(c->cfg.max_keypoints, c->cfg.max_height) > (size_t)smem_max - 1024)
+        return fail(c, FE_ERR_UNSUPPORTED, "fe_set_batch_detector: max_keypoints and max_height exceed the raster selection's shared memory");
+    c->surf = *surf;
+    c->hessian = true;
     return FE_OK;
 }
 
@@ -1881,7 +1939,14 @@ int32_t fe_batch_run(fe_ctx *c, const fe_match_cfg *cfg_a, const fe_match_cfg *c
     int r = prepare_batch(c, cfg_a, cfg_b);
     if (r == FE_OK) r = run_batch_on(c, c->g, c->b, c->stream, true, c->g.n_images / 2, cfg_a, cfg_b);
     if (r != FE_OK || !sync) return r;
-    return sync_and_resolve(c);
+    if ((r = sync_and_resolve(c)) != FE_OK || !c->hessian) return r;
+    // FAST keeps at most kp_cap keypoints, the Fast-Hessian detector may find more maxima than that
+    const int NI = c->g.n_images;
+    FE_CUDA(c, cudaMemcpyAsync(c->h_counts, c->b.n_kp, sizeof(uint32_t) * NI, cudaMemcpyDeviceToHost, c->stream));
+    FE_CUDA(c, cudaStreamSynchronize(c->stream));
+    for (int i = 0; i < NI; ++i)
+        if ((int)c->h_counts[i] > c->g.kp_cap) return fail(c, FE_ERR_CAPACITY, "fe_batch_run: more Fast-Hessian maxima than fe_config.max_keypoints");
+    return FE_OK;
 }
 
 int32_t fe_batch_download(fe_ctx *c, int32_t kp_cap, fe_kpoint *kps, uint8_t *desc, int32_t *n_kps,
@@ -1982,8 +2047,10 @@ static int pipeline_chunked(fe_ctx *c, int32_t n_pairs, const uint8_t *left, con
 int32_t fe_pipeline_batch(fe_ctx *c, int32_t n_pairs, const uint8_t *left, const uint8_t *right, int32_t w, int32_t h,
                           const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b, int32_t kp_cap, fe_kpoint *kps,
                           uint8_t *desc, int32_t *n_kps, fe_match *ma, int32_t *n_a, fe_match *mb, int32_t *n_b) {
-    if (c && left && right && n_pairs >= 2 * chunk_pairs_of(c) && kp_cap >= 1 && c->nlevels == 1 &&
-        (c->batch_desc == FE_DESC_ORB256 || desc_dim(c->batch_desc) > 0)) {
+    // (the pyramid runs on the whole resident batch; the Fast-Hessian scale space is one per ctx, which two compute lanes
+    // would overwrite)
+    if (c && left && right && n_pairs >= 2 * chunk_pairs_of(c) && kp_cap >= 1 && c->nlevels == 1 && !c->hessian &&
+        (batch_rows(c) == FE_DESC_ORB256 || desc_dim(batch_rows(c)) > 0)) {
         // overlapped path: H2D of chunk k+1, kernels of chunk k and D2H of chunk k-1 run concurrently
         FE_CUDA(c, cudaSetDevice(c->cfg.device));
         return pipeline_chunked(c, n_pairs, left, right, w, h, cfg_a, cfg_b, {kp_cap, kps, desc, n_kps, ma, n_a, mb, n_b});

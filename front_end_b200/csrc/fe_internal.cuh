@@ -330,6 +330,43 @@ int launch_surf(const Geom &g, const Buffers &b, const uint32_t *counts, bool ex
                 cudaStream_t s);
 constexpr int SURF_DIRECT_MAX_WIN = 1024;   // windows above SURF_MAX_WIN are produced on the fly (never staged), up to this size
 constexpr int SURF_MAX_WIN = 88;   // largest supported (int)(21 * size * 1.2 / 9): keypoint size <= 31.4 (ORB: 31 -> 86)
+constexpr int SURF_ORI_RADIUS = 6;  // orientation samples: the (i, j) with i^2 + j^2 <= 36
+
+// Scale of a SURF keypoint (src/surf.cpp:609-611): s = size * 1.2 / 9, the Haar wavelet size and the descriptor window.
+struct SurfScale { float s; int grad_wav_size, win_size; };
+__device__ __forceinline__ SurfScale surf_scale(float size) {
+    SurfScale r;
+    r.s = __fdiv_rn(__fmul_rn(size, 1.2f), 9.0f);
+    r.grad_wav_size = 2 * __float2int_rn(__fmul_rn(2.f, r.s));
+    r.win_size = (int)__fmul_rn(21.f, r.s);
+    return r;
+}
+
+// Orientation sample (i, j) of a keypoint at (cx, cy): its Haar wavelet's top-left corner (x, y) on the integral image and
+// whether the wavelet lies inside the w x h image (src/surf.cpp:630-636).  half = (grad_wav_size - 1) / 2.
+__device__ __forceinline__ bool surf_ori_sample(float cx, float cy, const SurfScale &sc, float half, int i, int j, int w, int h,
+                                                int &x, int &y) {
+    x = __float2int_rn(__fsub_rn(__fadd_rn(cx, __fmul_rn((float)i, sc.s)), half));
+    y = __float2int_rn(__fsub_rn(__fadd_rn(cy, __fmul_rn((float)j, sc.s)), half));
+    return !(y < 0 || y >= (h + 1) - sc.grad_wav_size || x < 0 || x >= (w + 1) - sc.grad_wav_size);
+}
+
+// SURFInvoker's drop rule (src/surf.cpp:953-978): the keypoints whose descriptor the reference does not compute and which it
+// removes.  Geometric only: the wavelet larger than the image, a window outside [1, max_win], or -- oriented -- no orientation
+// sample inside the image.  The descriptor kernel and the batch's raster selection of Fast-Hessian maxima both decide with it,
+// so a batch never holds a keypoint the descriptor pass drops.
+__device__ __forceinline__ bool surf_drops(float cx, float cy, float size, int w, int h, bool upright, int max_win) {
+    const SurfScale sc = surf_scale(size);
+    if (h + 1 < sc.grad_wav_size || w + 1 < sc.grad_wav_size || sc.win_size < 1 || sc.win_size > max_win) return true;
+    if (upright) return false;
+    const float half = __fdiv_rn((float)(sc.grad_wav_size - 1), 2.f);
+    for (int i = -SURF_ORI_RADIUS; i <= SURF_ORI_RADIUS; ++i)
+        for (int j = -SURF_ORI_RADIUS; j <= SURF_ORI_RADIUS; ++j) {
+            int x, y;
+            if (i * i + j * j <= SURF_ORI_RADIUS * SURF_ORI_RADIUS && surf_ori_sample(cx, cy, sc, half, i, j, w, h, x, y)) return false;
+        }
+    return true;
+}
 
 // multi-level ORB (pyramid.cu)
 int launch_resize_linear_exact(const uint8_t *src, int sw, int sh, int spitch, size_t sstride, uint8_t *dst, int dw, int dh,
@@ -354,6 +391,11 @@ int launch_hessian_maxima(const float *d0, const float *d1, const float *d2, con
 int launch_surf_rank_sort(const fe_kpoint *in, fe_kpoint *out, const uint32_t *count, int cap, uint32_t *max_size_bits, int n_images,
                           cudaStream_t s);
 int launch_integral(const Geom &g, const Buffers &b, cudaStream_t s);
+// Batched pipeline (fe_set_batch_detector): of the count[i] maxima in in + i * kp_cap, those SURFInvoker keeps
+// (surf_drops), in raster order (y, x, then KeypointGreater) -> b.kp, b.kx, b.ky; b.n_kp = survivors, or the maxima count when
+// it exceeds kp_cap.  One CTA per image of g, surf_raster_smem(kp_cap, h) bytes of dynamic shared memory.
+size_t surf_raster_smem(int kp_cap, int h);
+int launch_surf_raster(const Geom &g, const fe_kpoint *in, const uint32_t *count, bool upright, const Buffers &b, cudaStream_t s);
 
 // WindowMatcher over a resident sequence (window.cu)
 // side 0: left keypoints / descriptors of the landmarks (queryIdx of matches_a); side 1: right descriptors (trainIdx), wkx / wky unused

@@ -23,7 +23,7 @@ namespace fe {
 constexpr int S_WARPS_SMALL = 8, S_WARPS_LARGE = 4;      // warps per CTA for the 32-px / 88-px window variants
 constexpr int PATCH = 20;           // PATCH_SZ
 constexpr int PW = PATCH + 1;       // 21
-constexpr int ORI_RADIUS = 6, N_ORI = 113;
+constexpr int ORI_RADIUS = SURF_ORI_RADIUS, N_ORI = 113;
 
 __device__ float d_aptw[N_ORI];     // Gaussian weights of the orientation samples (sigma 2.5)
 __device__ int8_t d_apt[N_ORI][2];  // sample offsets (x, y)
@@ -205,14 +205,18 @@ surf_describe_kernel(const uint8_t *__restrict__ img, const int32_t *__restrict_
     const fe_kpoint key = kp[o];
     const uint8_t *src = img + (size_t)image * g.img_stride;
     const float cx = key.x, cy = key.y;
-    const float s = __fdiv_rn(__fmul_rn(key.size, 1.2f), 9.0f);
-    const int grad_wav_size = 2 * __float2int_rn(__fmul_rn(2.f, s));
-    const int win_size = (int)__fmul_rn((float)PW, s);
-    bool drop = (g.h + 1 < grad_wav_size || g.w + 1 < grad_wav_size) || win_size < 1 || win_size > (MAXWIN > 0 ? MAXWIN : SURF_DIRECT_MAX_WIN);
+    const SurfScale sc = surf_scale(key.size);
+    const int grad_wav_size = sc.grad_wav_size, win_size = sc.win_size;
+    // (warp-uniform) a keypoint that is not dropped has at least one orientation sample inside the image
+    const bool drop = surf_drops(cx, cy, key.size, g.w, g.h, upright != 0, MAXWIN > 0 ? MAXWIN : SURF_DIRECT_MAX_WIN);
+    if (drop) {
+        if (lane == 0) { kp[o].size = -1.f; }
+        return;
+    }
     float dir = 270.f;
 
     // ---- orientation (src/surf.cpp:617-670) ---------------------------------------------------------------
-    if (!upright && !drop) {
+    if (!upright) {
         const int stride = g.w + 1;
         const int32_t *S = integ + (size_t)image * (g.h + 1) * stride;
         const HaarBox dx0 = haar_box(0, 0, 2, 4, -1, grad_wav_size), dx1 = haar_box(2, 0, 4, 4, 1, grad_wav_size);
@@ -224,9 +228,8 @@ surf_describe_kernel(const uint8_t *__restrict__ img, const int32_t *__restrict_
             bool ok = false;
             float X = 0.f, Y = 0.f;
             if (kk < N_ORI) {
-                const int x = __float2int_rn(__fsub_rn(__fadd_rn(cx, __fmul_rn((float)d_apt[kk][0], s)), half));
-                const int y = __float2int_rn(__fsub_rn(__fadd_rn(cy, __fmul_rn((float)d_apt[kk][1], s)), half));
-                ok = !(y < 0 || y >= (g.h + 1) - grad_wav_size || x < 0 || x >= (g.w + 1) - grad_wav_size);
+                int x, y;
+                ok = surf_ori_sample(cx, cy, sc, half, d_apt[kk][0], d_apt[kk][1], g.w, g.h, x, y);
                 if (ok) {
                     const int32_t *ptr = S + (size_t)y * stride + x;
                     const float vx = haar2(ptr, stride, dx0, dx1), vy = haar2(ptr, stride, dy0, dy1);
@@ -244,9 +247,7 @@ surf_describe_kernel(const uint8_t *__restrict__ img, const int32_t *__restrict_
             nangle += __popc(m);
         }
         __syncwarp();
-        if (nangle == 0) {
-            drop = true;
-        } else {
+        {
             // 72 windows of 60 degrees, 5 degrees apart; lane handles windows lane, lane+32, lane+64
             float best_mod = 0.f, bestx = 0.f, besty = 0.f;
             int best_i = 1 << 30;
@@ -274,10 +275,6 @@ surf_describe_kernel(const uint8_t *__restrict__ img, const int32_t *__restrict_
             }
             dir = fast_atan2_deg(-besty, bestx);
         }
-    }
-    if (drop) {
-        if (lane == 0) { kp[o].size = -1.f; }
-        return;
     }
     if (lane == 0) kp[o].angle = dir;
 

@@ -14,7 +14,9 @@
 //   surf_rank_sort_kernel  std::sort(keypoints, KeypointGreater()) (src/surf.cpp:445-460,511) on the device: the comparator is
 //                          a strict total order (response, size, octave, y, x), so the rank of a record -- the number of
 //                          records that precede it -- is its final position; deterministic although the append order is not.
-// All three kernels take a batch of images (blockIdx.z); nothing returns to the host between detection and description.
+//   surf_raster_kernel     the batched pipeline's replacement of the sort: the maxima SURFInvoker keeps, in raster order
+//                          (y, x, then KeypointGreater), bucketed by floor(y) -- what the banded matchers read.
+// All of them take a batch of images; nothing returns to the host between detection and description.
 #include "fe_internal.cuh"
 
 namespace fe {
@@ -180,6 +182,115 @@ int launch_surf_rank_sort(const fe_kpoint *in, fe_kpoint *out, const uint32_t *c
     cudaMemsetAsync(max_size_bits, 0, sizeof(uint32_t) * n_images, s);
     dim3 grid(div_up(cap, 256), n_images);
     surf_rank_sort_kernel<<<grid, 256, 0, s>>>(in, out, count, cap, max_size_bits);
+    return 1;
+}
+
+// ---- batched pipeline: the maxima that survive SURFInvoker, in raster order ---------------------------------------------
+// The banded matchers need keypoints whose floor(y) never decreases; the maxima arrive in atomic-append order.  One CTA per
+// image, everything in shared memory: survivor bits and a histogram of floor(y) (pass 1), an exclusive scan of the histogram,
+// a scatter of survivor indices into their rows (pass 2), and a rank inside each row (pass 3, ~16 keypoints per row at
+// 1280x720) under the strict total order (y, x, KeypointGreater) -- deterministic although the append order is not.
+constexpr int RASTER_THREADS = 1024;
+
+__device__ __forceinline__ int raster_row(float y, int h) { return min(max((int)floorf(y), 0), h - 1); }
+
+// a precedes q in the batch's order; the input index breaks ties of identical records (whose bytes are then the same anyway)
+__device__ __forceinline__ bool raster_before(const fe_kpoint &a, int ia, const fe_kpoint &q, int iq) {
+    if (a.y != q.y) return a.y < q.y;
+    if (a.x != q.x) return a.x < q.x;
+    if (kp_greater(a, q)) return true;
+    if (kp_greater(q, a)) return false;
+    return ia < iq;
+}
+
+size_t surf_raster_smem(int kp_cap, int h) {
+    return sizeof(uint32_t) * div_up(kp_cap, 32) + sizeof(int) * (size_t)(h + 1) + sizeof(uint16_t) * (size_t)kp_cap;
+}
+
+__global__ void __launch_bounds__(RASTER_THREADS)
+surf_raster_kernel(const fe_kpoint *__restrict__ in, const uint32_t *__restrict__ count, Geom g, int upright,
+                   fe_kpoint *__restrict__ out, float *__restrict__ kx, float *__restrict__ ky, uint32_t *__restrict__ n_out) {
+    extern __shared__ __align__(16) uint32_t s_raster[];
+    const int image = blockIdx.x, cap = g.kp_cap, H = g.h, tid = threadIdx.x;
+    const int words = div_up(cap, 32);
+    uint32_t *keep = s_raster;                                        // [words] survivor bits
+    int *rows = reinterpret_cast<int *>(keep + words);                // [H + 1] counts -> starts -> ends of the rows
+    uint16_t *order = reinterpret_cast<uint16_t *>(rows + H + 1);     // [cap] input index of the survivors, row by row
+    const uint32_t found = count[image];
+    const int n = min((int)found, cap);
+    const fe_kpoint *src = in + (size_t)image * cap;
+    for (int i = tid; i < words; i += RASTER_THREADS) keep[i] = 0u;
+    for (int r = tid; r <= H; r += RASTER_THREADS) rows[r] = 0;
+    __syncthreads();
+    for (int i = tid; i < n; i += RASTER_THREADS) {
+        const fe_kpoint k = src[i];
+        if (!surf_drops(k.x, k.y, k.size, g.w, g.h, upright != 0, SURF_DIRECT_MAX_WIN)) {
+            atomicOr(&keep[i >> 5], 1u << (i & 31));
+            atomicAdd(&rows[raster_row(k.y, H)], 1);
+        }
+    }
+    __syncthreads();
+    {   // exclusive scan of rows[0 .. H]: every thread owns a contiguous run of `per` rows
+        __shared__ int s_warp[RASTER_THREADS / 32];
+        const int per = div_up(H + 1, RASTER_THREADS), r0 = min(tid * per, H + 1), r1 = min(r0 + per, H + 1);
+        int local = 0;
+        for (int r = r0; r < r1; ++r) local += rows[r];
+        const int lane = tid & 31, warp = tid >> 5;
+        int incl = local;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int v = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += v;
+        }
+        if (lane == 31) s_warp[warp] = incl;
+        __syncthreads();
+        if (warp == 0) {
+            int w = s_warp[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int v = __shfl_up_sync(0xffffffffu, w, o);
+                if (lane >= o) w += v;
+            }
+            s_warp[lane] = w;
+        }
+        __syncthreads();
+        int run = (warp > 0 ? s_warp[warp - 1] : 0) + incl - local;
+        for (int r = r0; r < r1; ++r) { const int c = rows[r]; rows[r] = run; run += c; }
+    }
+    __syncthreads();
+    const int m = rows[H];                   // survivors (row H is empty: its start is the total)
+    for (int i = tid; i < n; i += RASTER_THREADS)
+        if (keep[i >> 5] & (1u << (i & 31))) order[atomicAdd(&rows[raster_row(src[i].y, H)], 1)] = (uint16_t)i;
+    __syncthreads();                         // rows[r] is now the end of row r, the start of row r + 1
+    fe_kpoint *dst = out + (size_t)image * cap;
+    float *dx = kx + (size_t)image * cap, *dy = ky + (size_t)image * cap;
+    for (int p = tid; p < m; p += RASTER_THREADS) {
+        const int i = order[p];
+        const fe_kpoint k = src[i];
+        const int r = raster_row(k.y, H), lo = r > 0 ? rows[r - 1] : 0, hi = rows[r];
+        int rank = 0;
+        for (int q = lo; q < hi; ++q) {
+            const int j = order[q];
+            if (j != i && raster_before(src[j], j, k, i)) ++rank;
+        }
+        dst[lo + rank] = k;
+        dx[lo + rank] = k.x;
+        dy[lo + rank] = k.y;
+    }
+    if (found > (uint32_t)cap) {
+        // more maxima than capacity (the caller reports FE_ERR_CAPACITY): the consumers read all cap records, so the tail
+        // holds empty records below the last row -- still raster-ordered, dropped by the descriptor pass
+        fe_kpoint e{};
+        e.y = (float)H; e.angle = -1.f;
+        for (int p = m + tid; p < cap; p += RASTER_THREADS) { dst[p] = e; dx[p] = 0.f; dy[p] = e.y; }
+    }
+    if (tid == 0) n_out[image] = found > (uint32_t)cap ? found : (uint32_t)m;
+}
+
+int launch_surf_raster(const Geom &g, const fe_kpoint *in, const uint32_t *count, bool upright, const Buffers &b, cudaStream_t s) {
+    const size_t smem = surf_raster_smem(g.kp_cap, g.h);
+    if (smem > 48 * 1024) cudaFuncSetAttribute(surf_raster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    surf_raster_kernel<<<g.n_images, RASTER_THREADS, smem, s>>>(in, count, g, upright ? 1 : 0, b.kp, b.kx, b.ky, b.n_kp);
     return 1;
 }
 

@@ -308,7 +308,25 @@ class FrontEnd:
     def set_batch_descriptor(self, kind):
         """Descriptor of the batched pipeline: DESC_ORB256 (default) or DESC_SURF64 / DESC_SURF128."""
         self._check(self.lib.fe_set_batch_descriptor(self.h, kind))
-        self._batch_kind = kind
+        self._desc_kind = self._batch_kind = kind
+
+    def set_batch_detector(self, surf=None):
+        """Detector of the batched pipeline (fe_set_batch_detector).  surf=None: FAST / ORB (the default), described with
+        set_batch_descriptor's choice.  Otherwise cv::SURF's Fast-Hessian detector: a dict of surf_detect_batch's keywords
+        (hessian_threshold=100.0, n_octaves=4, n_octave_layers=2, extended=False, upright=False; {} = all defaults).  Its
+        batches hold the surviving keypoints in raster order with SURF-64 / SURF-128 float rows, matched with NORM_L2."""
+        if surf is None:
+            self._check(self.lib.fe_set_batch_detector(self.h, None))
+            self._batch_kind = getattr(self, "_desc_kind", L.DESC_ORB256)
+            return
+        p = dict(hessian_threshold=100.0, n_octaves=4, n_octave_layers=2, extended=False, upright=False)
+        unknown = set(surf) - set(p)
+        if unknown:
+            raise ValueError("unknown SURF parameters: %s" % sorted(unknown))
+        p.update(surf)
+        sp = L.SurfParams(p["hessian_threshold"], p["n_octaves"], p["n_octave_layers"], int(p["extended"]), int(p["upright"]))
+        self._check(self.lib.fe_set_batch_detector(self.h, C.byref(sp)))
+        self._batch_kind = L.DESC_SURF128 if p["extended"] else L.DESC_SURF64
 
     # -- batched pipeline -----------------------------------------------------------------------------------
     @staticmethod

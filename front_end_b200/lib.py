@@ -113,6 +113,7 @@ EXPORTS = {
                                        C.c_void_p, C.c_void_p]),
     "fe_set_chunk_pairs": (C.c_int32, [C.c_void_p, C.c_int32]),
     "fe_set_batch_descriptor": (C.c_int32, [C.c_void_p, C.c_int32]),
+    "fe_set_batch_detector": (C.c_int32, [C.c_void_p, C.POINTER(SurfParams)]),
     "fe_batch_upload": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
     "fe_batch_run": (C.c_int32, [C.c_void_p, C.POINTER(MatchCfg), C.POINTER(MatchCfg), C.c_int32]),
     "fe_batch_download": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

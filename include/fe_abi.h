@@ -27,7 +27,8 @@ extern "C" {
 #endif
 
 #define FE_ABI_VERSION 6   /* 6: fe_set_freak, FE_DESC_FREAK, 64-byte rows through the matchers; SURF rows in fe_window_batch,
-                              fe_window_update and fe_batch_landmarks, whose l_desc / r_desc became void * (all additive) */
+                              fe_window_update and fe_batch_landmarks, whose l_desc / r_desc became void *; fe_set_batch_detector
+                              (all additive: no struct changed size, every earlier call behaves as before) */
 
 /* ---- wire-compatible PODs ------------------------------------------------------------------ */
 
@@ -304,6 +305,30 @@ int32_t fe_pipeline_batch(fe_ctx *ctx, int32_t n_pairs, const uint8_t *left, con
  * SURF stage would drop (src/surf.cpp:953-978; cannot happen with edge_threshold >= 16) stay in place
  * with size = -1 in batch mode. */
 int32_t fe_set_batch_descriptor(fe_ctx *ctx, int32_t desc_kind);
+/* Selects the detector of the batched pipeline (fe_batch_run, fe_pipeline_batch, and through them fe_batch_landmarks /
+ * fe_window_batch).  surf == NULL: FAST / ORB per fe_config and the fe_set_orb_* calls (the default, unchanged).
+ * surf != NULL: cv::SURF's Fast-Hessian detector with these parameters (src/surf.cpp:462-512), described with SURF-64 /
+ * SURF-128 per surf->extended, oriented or upright per surf->upright, matched with FE_NORM_L2.  The service chain
+ * getStereoFeatures(SURF, SURF) -> stereoMatching -> windowMatching (features.py:149-156, bin/feature_node:24-80) then runs
+ * on the device from the images to the matches.
+ *  - Keypoints: the maxima SURFInvoker keeps (src/surf.cpp:953-978; the batch never holds a size = -1 record), in RASTER
+ *    order (y ascending, then x ascending, then KeypointGreater) -- not the KeypointGreater order of fe_surf_detect_batch,
+ *    whose keypoints and rows they equal bit for bit as a set.  Sort by response on the host for the reference's order.
+ *    Raster order lets mode A take the banded L2 kernel and mode B the exact tensor-core cross-check.
+ *  - Rows: SURF-64 / SURF-128 floats in fe_batch_download, fe_pipeline_batch and fe_batch_landmarks;
+ *    fe_set_batch_descriptor returns FE_ERR_UNSUPPORTED until the ctx is switched back with NULL, and a Hamming norm
+ *    with such a batch is FE_ERR_UNSUPPORTED.
+ *  - fe_set_orb_*, fe_set_detection and fe_config's FAST fields do not apply while the detector is selected; switching
+ *    back with NULL restores them exactly (they are not changed).
+ *  - fe_pipeline_batch runs upload -> run -> download for these batches (as for nlevels > 1): the scale space is one per
+ *    ctx, so the two compute lanes of the overlapped path would overwrite each other's.
+ *  - The scale space (Buffers group GRP_SURFDET) is allocated on first use; a FAST / ORB ctx allocates nothing for it.
+ *  - An image can have more maxima than fe_config.max_keypoints: the call that synchronises (fe_batch_run with sync,
+ *    fe_batch_download, fe_pipeline_batch) returns FE_ERR_CAPACITY, n_kps reports the number of maxima found, and that
+ *    pair's outputs are unspecified (but in bounds).
+ * Returns FE_ERR_BAD_ARG for more than 8 octaves / layers, FE_ERR_UNSUPPORTED if max_keypoints and max_height exceed the
+ * raster selection's shared memory (one CTA per image: 2.1 B per keypoint + 4 B per row). */
+int32_t fe_set_batch_detector(fe_ctx *ctx, const fe_surf_params *surf);
 /* WindowMatcher::newStereo's data-parallel stage for a whole resident sequence (src/WindowMatcher.cpp:75-231;
  * BASELINE config 4).  Call after fe_batch_run(cfg_a = ratio mode, ...) on F consecutive stereo frames (pair f =
  * frame f).  The landmarks of frame f are its matches_a rows (every stereo match becomes a landmark, :79-85); for

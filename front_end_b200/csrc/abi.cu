@@ -392,6 +392,9 @@ int desc_dim(int kind) { return kind == FE_DESC_SURF64 ? 64 : kind == FE_DESC_SU
 // cv::BriefDescriptorExtractor rows: bytes per descriptor (0 for the other kinds)
 int brief_width(int kind) { return kind == FE_DESC_BRIEF16 ? 16 : kind == FE_DESC_BRIEF32 ? 32 : kind == FE_DESC_BRIEF64 ? 64 : 0; }
 int brief_slot(int kind) { return kind - FE_DESC_BRIEF16; }
+// Bytes of a binary row on the host, packed as fe_describe writes it: 16 for BRIEF-16, 32 for ORB-256 and BRIEF-32.  The
+// matchers' device rows are 32 bytes; BRIEF-16 rows ride in them zero-padded, which leaves every Hamming distance unchanged.
+int binary_bytes(int kind) { return kind == FE_DESC_BRIEF16 ? 16 : 32; }
 
 // What rows the batch holds: SURF-64 / SURF-128 per fe_surf_params.extended when it detects with the Fast-Hessian detector,
 // else what fe_set_batch_descriptor selected.
@@ -456,11 +459,11 @@ int run_match_l2_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st,
 }
 
 // train_sorted: the train keypoints of every pair are in raster order (y non-decreasing), which
-// makes the mask-allowed trains of a query one contiguous index range (banded kernel).  Needs the groups of
-// match_groups(0, cfg_b != nullptr).
+// makes the mask-allowed trains of a query one contiguous index range (banded kernel).  row_bytes: binary_bytes of the rows.
+// Needs the groups of match_groups(0, cfg_b != nullptr).
 int run_match_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bool timed, int n_pairs,
                  const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b, const uint32_t *counts, bool train_sorted,
-                 bool both_sorted) {
+                 bool both_sorted, int row_bytes) {
     auto binary = [](const fe_match_cfg *m) { return !m || m->norm == FE_NORM_HAMMING || m->norm == FE_NORM_HAMMING2; };
     if (!binary(cfg_a) || !binary(cfg_b))
         return fail(c, FE_ERR_UNSUPPORTED, "binary descriptors are matched with FE_NORM_HAMMING or FE_NORM_HAMMING2");
@@ -487,7 +490,7 @@ int run_match_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bo
                 FE_CUDA(c, cudaEventCreateWithFlags(&c->ev_join[lane], cudaEventDisableTiming));
             }
             const bool side = overlap && lane >= 0;
-            t.done(launch_hamming_cross_pruned(g, n_pairs, cfg_b->max_dy, fuse_band, c->cross_mih, b, counts, cfg_a ? std::max(cfg_a->ratio, 0.0) : -1.0, st,
+            t.done(launch_hamming_cross_pruned(g, n_pairs, cfg_b->max_dy, fuse_band, c->cross_mih, row_bytes, b, counts, cfg_a ? std::max(cfg_a->ratio, 0.0) : -1.0, st,
                                                side ? c->s_aux[lane] : nullptr, side ? c->ev_fork[lane] : nullptr, side ? c->ev_join[lane] : nullptr));
         }
         else t.done(launch_hamming_cross(g, n_pairs, cfg_b->norm == FE_NORM_HAMMING2, b, counts, st));
@@ -510,7 +513,8 @@ int prepare_batch(fe_ctx *c, const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_
     if (dim > 0 && ((cfg_a && cfg_a->norm != FE_NORM_L2) || (cfg_b && cfg_b->norm != FE_NORM_L2)))
         return fail(c, FE_ERR_UNSUPPORTED, "SURF descriptors are matched with FE_NORM_L2");
     const unsigned hessian = c->hessian ? GRP_INTEGRAL | GRP_SURFDET : 0u;      // the scale space reads the integral image
-    return ensure(c, match_groups(dim, cfg_b != nullptr) | (dim > 0 && !batch_upright(c) ? GRP_INTEGRAL : 0u) | hessian);
+    const unsigned brief = brief_width(batch_rows(c)) > 0 && !batch_raster(c) ? GRP_INTEGRAL : 0u;   // brief_kernel's input
+    return ensure(c, match_groups(dim, cfg_b != nullptr) | (dim > 0 && !batch_upright(c) ? GRP_INTEGRAL : 0u) | hessian | brief);
 }
 
 // cv::SURF's Fast-Hessian detector (src/surf.cpp:462-512) on the images of (g, b) in b.img: integral image, scale-space layers
@@ -594,13 +598,34 @@ int hessian_detect(fe_ctx *c, const Geom &g, const Buffers &b, const fe_surf_par
     return FE_OK;
 }
 
-// Detect, describe and match the batch (g, b) on st: the resident batch, or a chunk view of it.  ORB-256 with Hamming
-// matching, or FAST / ORB-mode keypoints with SURF descriptors (bin/detect_node:33-41) and L2 matching.  The caller applies
+// cv::BriefDescriptorExtractor::compute (kind BRIEF-16 / 32 / 64) of the keypoints the detector left in (g, b), with the table
+// and use_orientation set for that width now: runByImageBorder(28) on the device, then the rows, row_bytes apart, into out.
+// Raster-ordered keypoints take the tile kernel, the pyramid's level-major ones brief_kernel over the integral images
+// (GRP_INTEGRAL).  The caller checked that the table exists.
+int run_brief_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bool timed, int kind, bool raster, uint8_t *out,
+                 int row_bytes) {
+    const int slot = brief_slot(kind), bw = brief_width(kind);
+    const int8_t *tab = b.brief_tab + (size_t)slot * 512 * 4;
+    // (timed as description: the border is compute()'s runByImageBorder, and fe_stereo_features reports it with the rows)
+    { StageTimer t(c, ST_BRIEF, st, timed); t.done(launch_brief_border(g, b, st)); }
+    if (raster) {
+        StageTimer t(c, ST_BRIEF, st, timed);
+        t.done(launch_brief_tile(g, b, tab, bw, c->brief_orient[slot], out, row_bytes, st));
+    } else {
+        { StageTimer t(c, ST_BLUR, st, timed); t.done(launch_integral(g, b, st)); }
+        { StageTimer t(c, ST_BRIEF, st, timed); t.done(launch_brief_ext(g, b, b.n_kp, tab, bw, c->brief_orient[slot], out, row_bytes, st)); }
+    }
+    FE_CUDA(c, cudaGetLastError());
+    return FE_OK;
+}
+
+// Detect, describe and match the batch (g, b) on st: the resident batch, or a chunk view of it.  ORB-256 or BRIEF-16 / 32 with
+// Hamming matching, or FAST / ORB-mode keypoints with SURF descriptors (bin/detect_node:33-41) and L2 matching.  The caller applies
 // pending detection changes and calls prepare_batch; the pyramid (nlevels > 1) runs on the whole resident batch only.
 int run_batch_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bool timed, int n_pairs,
                  const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b) {
-    const int dim = desc_dim(batch_rows(c));
-    const bool sorted = batch_raster(c);
+    const int rows = batch_rows(c), dim = desc_dim(rows);
+    const bool sorted = batch_raster(c), brief = brief_width(rows) > 0;
     if (c->hessian) {
         // Fast-Hessian maxima -> the survivors in raster order -> descriptors; nothing returns to the host
         int max_win = 0;
@@ -609,16 +634,18 @@ int run_batch_on(fe_ctx *c, const Geom &g, const Buffers &b, cudaStream_t st, bo
         { StageTimer t(c, ST_SELECT, st, timed); t.done(launch_surf_raster(g, b.hes_kp, b.hes_count, batch_upright(c), b, st)); }
         { StageTimer t(c, ST_SURF, st, timed); t.done(launch_surf(g, b, b.n_kp, dim == 128, batch_upright(c), max_win, st)); }
     } else {
-        int r = sorted ? run_detect_on(c, g, b, st, dim == 0, timed) : run_detect_pyramid(c, dim == 0);
+        const bool orb = dim == 0 && !brief;
+        int r = sorted ? run_detect_on(c, g, b, st, orb, timed) : run_detect_pyramid(c, orb);
         if (r != FE_OK) return r;
         if (dim > 0) {
             StageTimer t(c, ST_SURF, st, timed);
             t.done(launch_surf(g, b, b.n_kp, dim == 128, batch_upright(c), detected_surf_win(c), st));
         }
+        if (brief && (r = run_brief_on(c, g, b, st, timed, rows, sorted, b.desc, 32)) != FE_OK) return r;
     }
     if (!cfg_a && !cfg_b) return FE_OK;
     if (dim > 0) return run_match_l2_on(c, g, b, st, timed, n_pairs, dim, cfg_a, cfg_b, b.n_kp, sorted);
-    return run_match_on(c, g, b, st, timed, n_pairs, cfg_a, cfg_b, b.n_kp, sorted, sorted);
+    return run_match_on(c, g, b, st, timed, n_pairs, cfg_a, cfg_b, b.n_kp, sorted, sorted, binary_bytes(rows));
 }
 
 // Counts of pairs [p0, p0 + np) into h_counts: keypoints of image i at [i], n_a of pair p at [NI + p], n_b at [NI + NP + p]
@@ -663,8 +690,9 @@ int download_pairs(fe_ctx *c, int p0, int np, cudaStream_t st, const HostBatch &
         if (o.n_a) o.n_a[p] = (int32_t)hc[NI + p];
         if (o.n_b) o.n_b[p] = (int32_t)hc[NI + NP + p];
     }
-    const int dim = desc_dim(batch_rows(c));
-    const size_t drow = dim > 0 ? sizeof(float) * dim : 32;       // descriptor bytes per keypoint on the host
+    const int rows = batch_rows(c), dim = desc_dim(rows);
+    const size_t drow = dim > 0 ? sizeof(float) * dim : binary_bytes(rows);      // descriptor bytes per keypoint on the host
+    const size_t dev_row = dim > 0 ? sizeof(float) * 128 : 32;                    // and on the device
     c->d2h_bytes += (int64_t)sizeof(uint32_t) * 2 * ni + (o.kps ? (int64_t)sizeof(fe_kpoint) * max_kp * ni : 0) +
                     (o.desc ? (int64_t)drow * max_kp * ni : 0) + (o.ma ? (int64_t)sizeof(fe_match) * max_a * np : 0) +
                     (o.mb ? (int64_t)sizeof(fe_match) * max_b * np : 0);
@@ -673,12 +701,12 @@ int download_pairs(fe_ctx *c, int p0, int np, cudaStream_t st, const HostBatch &
     if (o.kps && max_kp > 0)
         FE_CUDA(c, cudaMemcpy2DAsync(o.kps + i0 * K, sizeof(fe_kpoint) * K, v.kp, sizeof(fe_kpoint) * C, sizeof(fe_kpoint) * max_kp,
                                      ni, cudaMemcpyDeviceToHost, st));
-    if (o.desc && max_kp > 0 && dim != 64)       // host rows as on the device (32 bytes or 128 floats): one strided copy
-        FE_CUDA(c, cudaMemcpy2DAsync(o.desc + i0 * K * drow, drow * K, dim ? (const void *)v.fdesc : v.desc, drow * C,
-                                     drow * max_kp, ni, cudaMemcpyDeviceToHost, st));
-    if (o.desc && max_kp > 0 && dim == 64)       // 64-d: pack the first 64 floats of every 128-float device row
+    const uint8_t *dsrc = dim ? reinterpret_cast<const uint8_t *>(v.fdesc) : v.desc;
+    if (o.desc && max_kp > 0 && drow == dev_row)     // host rows as on the device (32 bytes or 128 floats): one strided copy
+        FE_CUDA(c, cudaMemcpy2DAsync(o.desc + i0 * K * drow, drow * K, dsrc, drow * C, drow * max_kp, ni, cudaMemcpyDeviceToHost, st));
+    if (o.desc && max_kp > 0 && drow < dev_row)      // SURF-64, BRIEF-16: pack the leading drow bytes of every device row
         for (int i = 0; i < ni; ++i)
-            FE_CUDA(c, cudaMemcpy2DAsync(o.desc + (i0 + i) * K * 256, 256, v.fdesc + i * C * 128, 512, 256,
+            FE_CUDA(c, cudaMemcpy2DAsync(o.desc + (i0 + i) * K * drow, drow, dsrc + i * C * dev_row, dev_row, drow,
                                          std::min((int)hc[i0 + i], max_kp), cudaMemcpyDeviceToHost, st));
     if (o.ma && max_a > 0)
         FE_CUDA(c, cudaMemcpy2DAsync(o.ma + p0 * K, sizeof(fe_match) * K, v.match_a, sizeof(fe_match) * C, sizeof(fe_match) * max_a,
@@ -1214,7 +1242,7 @@ int32_t fe_describe(fe_ctx *c, const uint8_t *img, int32_t w, int32_t h, int32_t
           t.done(0); }
         { StageTimer t(c, ST_BLUR); t.done(launch_integral(c->g, bb, c->stream)); }
         { StageTimer t(c, ST_BRIEF);
-          t.done(launch_brief_ext(c->g, bb, bb.n_override, bb.brief_tab + (size_t)slot * 512 * 4, bw, c->brief_orient[slot], bb.brief_desc, c->stream)); }
+          t.done(launch_brief_ext(c->g, bb, bb.n_override, bb.brief_tab + (size_t)slot * 512 * 4, bw, c->brief_orient[slot], bb.brief_desc, 64, c->stream)); }
         FE_CUDA(c, cudaGetLastError());
         FE_CUDA(c, cudaMemcpy2DAsync(desc, (size_t)bw, bb.brief_desc, 64, (size_t)bw, m, cudaMemcpyDeviceToHost, c->stream));
         return sync_and_resolve(c);
@@ -1290,7 +1318,7 @@ static int match_host_inputs(fe_ctx *c, const fe_kpoint *qk, const void *qd, int
         return fail(c, FE_ERR_UNSUPPORTED, "match: ORB256 / BRIEF go with FE_NORM_HAMMING / FE_NORM_HAMMING2, SURF64/128 with FE_NORM_L2");
     const bool wide = desc_kind == FE_DESC_BRIEF64 || desc_kind == FE_DESC_FREAK;      // 512-bit rows (match512.cu)
     if (wide && cfg->norm != FE_NORM_HAMMING) return fail(c, FE_ERR_UNSUPPORTED, "match: BRIEF-64 / FREAK rows go with FE_NORM_HAMMING");
-    const int bin_bytes = desc_kind == FE_DESC_BRIEF16 ? 16 : 32;
+    const int bin_bytes = binary_bytes(desc_kind);
     const bool cross = cfg->mode == FE_MATCH_CROSSCHECK;
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     { int r0 = ensure(c, wide ? GRP_BRIEF : match_groups(dim, cross)); if (r0 != FE_OK) return r0; }
@@ -1327,7 +1355,8 @@ static int match_host_inputs(fe_ctx *c, const fe_kpoint *qk, const void *qd, int
     if (dim > 0) return run_match_l2_on(c, c->g, c->b, c->stream, true, 1, dim, cross ? nullptr : cfg, cross ? cfg : nullptr, c->b.n_override, sorted);
     bool qsorted = sorted;
     for (int i = 1; i < nq && qsorted; ++i) qsorted = !(qk[i].y < qk[i - 1].y);
-    return run_match_on(c, c->g, c->b, c->stream, true, 1, cross ? nullptr : cfg, cross ? cfg : nullptr, c->b.n_override, sorted, qsorted);
+    return run_match_on(c, c->g, c->b, c->stream, true, 1, cross ? nullptr : cfg, cross ? cfg : nullptr, c->b.n_override, sorted, qsorted,
+                        bin_bytes);
 }
 
 int32_t fe_knn2(fe_ctx *c, const fe_kpoint *qk, const void *qd, int32_t nq, const fe_kpoint *tk, const void *td,
@@ -1435,7 +1464,7 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
     if ((r = ensure(c, GRP_WUPDATE | (dim > 0 ? match_groups(dim, false) | GRP_WUFLOAT : live ? GRP_WLIVE : 0u))) != FE_OK) return r;
     Buffers &b = c->b;
     if (c->g.kp_cap == 0 && (r = set_geom(c, 16, 16, 2)) != FE_OK) return r;
-    const int bin_bytes = desc_kind == FE_DESC_BRIEF16 ? 16 : 32;
+    const int bin_bytes = binary_bytes(desc_kind);
     auto put_desc = [&](uint8_t *dst, const void *src) -> int {
         if (bin_bytes == 32) { FE_CUDA(c, cudaMemcpyAsync(dst, src, (size_t)32 * n, cudaMemcpyHostToDevice, c->stream)); }
         else {
@@ -1510,7 +1539,7 @@ int32_t fe_window_update(fe_ctx *c, int32_t reset, const fe_kpoint *l_kps, const
             w.mode = FE_MATCH_RATIO;
             if (w.mask == FE_MASK_WINDOW) { if (w.win_w <= 0) w.win_w = 100; if (w.win_h <= 0) w.win_h = 100; }
             if (dim > 0) r = run_match_l2_on(c, gv, v, c->stream, true, 1, dim, &w, nullptr, b.wu_n, c->wu_prev_sorted);
-            else r = run_match_on(c, gv, v, c->stream, true, 1, &w, nullptr, b.wu_n, c->wu_prev_sorted, false);
+            else r = run_match_on(c, gv, v, c->stream, true, 1, &w, nullptr, b.wu_n, c->wu_prev_sorted, false, bin_bytes);
             if (r != FE_OK) return r;
         }
         FE_CUDA(c, cudaMemcpyAsync(c->h_counts, live ? b.n_b : b.n_a, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
@@ -1593,8 +1622,8 @@ int32_t fe_window_batch(fe_ctx *c, const fe_match_cfg *cfg, const double *Q, int
     if (c->g.n_images < 4) return fail(c, FE_ERR_BAD_ARG, "fe_window_batch: run fe_batch_run on at least two frames first");
     const int rows = batch_rows(c), dim = desc_dim(rows);     // SURF-64 / SURF-128 batches: float rows and FE_NORM_L2
     const bool hamming = cfg->norm == FE_NORM_HAMMING || cfg->norm == FE_NORM_HAMMING2;
-    if (dim == 0 && (!hamming || rows != FE_DESC_ORB256))
-        return fail(c, FE_ERR_UNSUPPORTED, "fe_window_batch: ORB-256 sequences are matched with FE_NORM_HAMMING / FE_NORM_HAMMING2");
+    if (dim == 0 && !hamming)
+        return fail(c, FE_ERR_UNSUPPORTED, "fe_window_batch: ORB-256 / BRIEF sequences are matched with FE_NORM_HAMMING / FE_NORM_HAMMING2");
     if (dim > 0 && cfg->norm != FE_NORM_L2) return fail(c, FE_ERR_UNSUPPORTED, "fe_window_batch: SURF sequences are matched with FE_NORM_L2");
     const bool live = cfg->mode == FE_MATCH_CROSSCHECK;       // liveGraph variant (algorithm.py:1160-1190)
     if (!live && (cfg->mode != FE_MATCH_RATIO || cfg->mask != FE_MASK_WINDOW))
@@ -1629,7 +1658,7 @@ int32_t fe_window_batch(fe_ctx *c, const fe_match_cfg *cfg, const double *Q, int
             FE_CUDA(c, cudaGetLastError());
         } else {
             // landmarks inherit the left keypoints' order
-            r = run_match_on(c, gv, v, c->stream, true, V, cfg, nullptr, b.wcount, batch_raster(c), false);
+            r = run_match_on(c, gv, v, c->stream, true, V, cfg, nullptr, b.wcount, batch_raster(c), false, binary_bytes(rows));
         }
     }
     if (r != FE_OK) return r;
@@ -1769,8 +1798,7 @@ int32_t fe_batch_landmarks(fe_ctx *c, int32_t which, int32_t cap, fe_kpoint *l_k
                            void *r_desc, fe_match *matches, int32_t *n) {
     if (!c || !n || cap < 0 || (which != 0 && which != 1)) return fail(c, FE_ERR_BAD_ARG, "fe_batch_landmarks: bad argument");
     if (c->g.n_images < 2) return fail(c, FE_ERR_BAD_ARG, "fe_batch_landmarks: run fe_batch_run first");
-    const int rows = batch_rows(c), dim = desc_dim(rows);     // SURF batches: rows of dim floats
-    if (rows != FE_DESC_ORB256 && dim == 0) return fail(c, FE_ERR_UNSUPPORTED, "fe_batch_landmarks: ORB-256 or SURF batches");
+    const int rows = batch_rows(c), dim = desc_dim(rows);     // SURF batches: rows of dim floats; binary ones: binary_bytes(rows)
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     const Geom &g = c->g;
     const int P = g.n_images / 2;
@@ -1796,10 +1824,21 @@ int32_t fe_batch_landmarks(fe_ctx *c, int32_t which, int32_t cap, fe_kpoint *l_k
     if (mx > 0) {
         if (l_kps) FE_CUDA(c, cudaMemcpy2DAsync(l_kps, sizeof(fe_kpoint) * (size_t)cap, b.lm_lkp, sizeof(fe_kpoint) * C, sizeof(fe_kpoint) * (size_t)mx, P, cudaMemcpyDeviceToHost, c->stream));
         if (r_kps) FE_CUDA(c, cudaMemcpy2DAsync(r_kps, sizeof(fe_kpoint) * (size_t)cap, b.lm_rkp, sizeof(fe_kpoint) * C, sizeof(fe_kpoint) * (size_t)mx, P, cudaMemcpyDeviceToHost, c->stream));
-        const size_t row = dim > 0 ? sizeof(float) * dim : 32;     // descriptor bytes per landmark, packed on both sides
-        const void *ld = dim > 0 ? (const void *)b.lm_lfdesc : b.lm_ldesc, *rd = dim > 0 ? (const void *)b.lm_rfdesc : b.lm_rdesc;
-        if (l_desc) FE_CUDA(c, cudaMemcpy2DAsync(l_desc, row * cap, ld, row * C, row * mx, P, cudaMemcpyDeviceToHost, c->stream));
-        if (r_desc) FE_CUDA(c, cudaMemcpy2DAsync(r_desc, row * cap, rd, row * C, row * mx, P, cudaMemcpyDeviceToHost, c->stream));
+        const size_t row = dim > 0 ? sizeof(float) * dim : binary_bytes(rows);     // descriptor bytes per landmark on the host
+        const size_t dev_row = dim > 0 ? row : 32;                                 // and on the device (the float rows are packed)
+        const uint8_t *ld = dim > 0 ? reinterpret_cast<const uint8_t *>(b.lm_lfdesc) : b.lm_ldesc;
+        const uint8_t *rd = dim > 0 ? reinterpret_cast<const uint8_t *>(b.lm_rfdesc) : b.lm_rdesc;
+        for (int s = 0; s < 2; ++s) {
+            uint8_t *dst = static_cast<uint8_t *>(s ? r_desc : l_desc);
+            const uint8_t *src = s ? rd : ld;
+            if (!dst) continue;
+            if (row == dev_row) FE_CUDA(c, cudaMemcpy2DAsync(dst, row * cap, src, row * C, row * mx, P, cudaMemcpyDeviceToHost, c->stream));
+            else        // BRIEF-16: the leading 16 bytes of every 32-byte device row, pair by pair
+                for (int p = 0; p < P; ++p)
+                    if (std::min(n[p], mx) > 0)
+                        FE_CUDA(c, cudaMemcpy2DAsync(dst + p * row * cap, row, src + p * dev_row * C, dev_row, row, std::min(n[p], mx),
+                                                     cudaMemcpyDeviceToHost, c->stream));
+        }
         if (matches) FE_CUDA(c, cudaMemcpy2DAsync(matches, sizeof(fe_match) * (size_t)cap, b.lm_match, sizeof(fe_match) * C, sizeof(fe_match) * (size_t)mx, P, cudaMemcpyDeviceToHost, c->stream));
     }
     if ((r = sync_and_resolve(c)) != FE_OK) return r;
@@ -1908,7 +1947,12 @@ int32_t fe_set_batch_descriptor(fe_ctx *c, int32_t desc_kind) {
     if (!c) return FE_ERR_BAD_ARG;
     if (c->hessian)
         return fail(c, FE_ERR_UNSUPPORTED, "fe_set_batch_descriptor: the Fast-Hessian batch describes with SURF (fe_set_batch_detector(ctx, NULL) first)");
-    if (desc_kind != FE_DESC_ORB256 && desc_dim(desc_kind) == 0) return fail(c, FE_ERR_BAD_ARG, "unknown descriptor kind");
+    if (desc_kind == FE_DESC_BRIEF64 || desc_kind == FE_DESC_FREAK)
+        return fail(c, FE_ERR_UNSUPPORTED, "fe_set_batch_descriptor: the batch matches rows of at most 256 bits (BRIEF-64 / FREAK rows are 512)");
+    if (desc_kind == FE_DESC_BRIEF16 || desc_kind == FE_DESC_BRIEF32) {
+        if (!c->brief_bytes[brief_slot(desc_kind)])
+            return fail(c, FE_ERR_UNSUPPORTED, "fe_set_batch_descriptor: no BRIEF test table of this width (fe_set_brief_pattern)");
+    } else if (desc_kind != FE_DESC_ORB256 && desc_dim(desc_kind) == 0) return fail(c, FE_ERR_BAD_ARG, "unknown descriptor kind");
     if (desc_dim(desc_kind) > 0 && detected_surf_win(c) > SURF_DIRECT_MAX_WIN)
         return fail(c, FE_ERR_UNSUPPORTED, "SURF keypoint size not supported");
     c->batch_desc = desc_kind;
@@ -2048,9 +2092,8 @@ int32_t fe_pipeline_batch(fe_ctx *c, int32_t n_pairs, const uint8_t *left, const
                           const fe_match_cfg *cfg_a, const fe_match_cfg *cfg_b, int32_t kp_cap, fe_kpoint *kps,
                           uint8_t *desc, int32_t *n_kps, fe_match *ma, int32_t *n_a, fe_match *mb, int32_t *n_b) {
     // (the pyramid runs on the whole resident batch; the Fast-Hessian scale space is one per ctx, which two compute lanes
-    // would overwrite)
-    if (c && left && right && n_pairs >= 2 * chunk_pairs_of(c) && kp_cap >= 1 && c->nlevels == 1 && !c->hessian &&
-        (batch_rows(c) == FE_DESC_ORB256 || desc_dim(batch_rows(c)) > 0)) {
+    // would overwrite; every descriptor of the FAST / ORB batch -- ORB-256, BRIEF-16 / 32, SURF -- runs per chunk)
+    if (c && left && right && n_pairs >= 2 * chunk_pairs_of(c) && kp_cap >= 1 && c->nlevels == 1 && !c->hessian) {
         // overlapped path: H2D of chunk k+1, kernels of chunk k and D2H of chunk k-1 run concurrently
         FE_CUDA(c, cudaSetDevice(c->cfg.device));
         return pipeline_chunked(c, n_pairs, left, right, w, h, cfg_a, cfg_b, {kp_cap, kps, desc, n_kps, ma, n_a, mb, n_b});
@@ -2066,8 +2109,10 @@ int32_t fe_stereo_features(fe_ctx *c, const uint8_t *left, const uint8_t *right,
                            int32_t cap, double *proc_seconds) {
     if (!c || !left || !right || !lk || !ld || !nl || !rk || !rd || !nr || cap < 1 || stride < w)
         return fail(c, FE_ERR_BAD_ARG, "fe_stereo_features: bad argument");
-    const int dim = desc_dim(desc_kind);
-    if (desc_kind != FE_DESC_ORB256 && dim == 0) return fail(c, FE_ERR_UNSUPPORTED, "fe_stereo_features: unknown descriptor kind");
+    const int dim = desc_dim(desc_kind), bw = brief_width(desc_kind);
+    if (desc_kind != FE_DESC_ORB256 && dim == 0 && bw == 0) return fail(c, FE_ERR_UNSUPPORTED, "fe_stereo_features: unknown descriptor kind");
+    if (bw > 0 && !c->brief_bytes[brief_slot(desc_kind)])
+        return fail(c, FE_ERR_UNSUPPORTED, "fe_stereo_features: no BRIEF test table for this width (fe_set_brief_pattern)");
     FE_CUDA(c, cudaSetDevice(c->cfg.device));
     int r = set_geom(c, w, h, 2);
     if (r != FE_OK) return r;
@@ -2077,17 +2122,22 @@ int32_t fe_stereo_features(fe_ctx *c, const uint8_t *left, const uint8_t *right,
             return fail(c, FE_ERR_UNSUPPORTED, "fe_stereo_features: SURF keypoint size not supported");
         if ((r = ensure(c, GRP_FLOAT | (upright ? 0u : GRP_INTEGRAL))) != FE_OK) return r;
     }
+    // BRIEF rows: BRIEF-16 / 32 in the 32-byte desc rows, BRIEF-64 in the 64-byte brief_desc rows
+    const int brow = bw == 64 ? 64 : 32;
+    if (bw > 0 && (r = ensure(c, (bw == 64 ? GRP_BRIEF : 0u) | (c->nlevels > 1 ? GRP_INTEGRAL : 0u))) != FE_OK) return r;
     const bool was = c->profiling;
     c->profiling = true;     // the service reports per-stage ProcTime (bin/feature_node:27-34,72-75)
     { StageTimer t(c, ST_H2D);
       if ((r = upload_images(c, left, 1, stride, 0, 1)) != FE_OK) return r;
       if ((r = upload_images(c, right, 1, stride, 1, 1)) != FE_OK) return r;
       t.done(0); }
-    if ((r = run_detect(c, dim == 0)) != FE_OK) { c->profiling = was; return r; }
+    if ((r = run_detect(c, dim == 0 && bw == 0)) != FE_OK) { c->profiling = was; return r; }
     if (dim > 0) {
         StageTimer t(c, ST_SURF);
         t.done(launch_surf(c->g, c->b, c->b.n_kp, dim == 128, upright, detected_surf_win(c), c->stream));
     }
+    if (bw > 0 && (r = run_brief_on(c, c->g, c->b, c->stream, true, desc_kind, c->nlevels == 1, bw == 64 ? c->b.brief_desc : c->b.desc,
+                                    brow)) != FE_OK) { c->profiling = was; return r; }
     FE_CUDA(c, cudaMemcpyAsync(c->h_counts, c->b.n_kp, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
     FE_CUDA(c, cudaStreamSynchronize(c->stream));
     const size_t C = c->g.kp_cap;
@@ -2102,7 +2152,10 @@ int32_t fe_stereo_features(fe_ctx *c, const uint8_t *left, const uint8_t *right,
         kept[e] = m;
         if (m > 0) {
             FE_CUDA(c, cudaMemcpyAsync(ok[e], c->b.kp + e * C, sizeof(fe_kpoint) * m, cudaMemcpyDeviceToHost, c->stream));
-            if (dim == 0)
+            if (bw > 0)
+                FE_CUDA(c, cudaMemcpy2DAsync(od[e], (size_t)bw, (bw == 64 ? c->b.brief_desc : c->b.desc) + e * C * brow, (size_t)brow,
+                                             (size_t)bw, m, cudaMemcpyDeviceToHost, c->stream));
+            else if (dim == 0)
                 FE_CUDA(c, cudaMemcpyAsync(od[e], c->b.desc + e * C * 32, (size_t)32 * m, cudaMemcpyDeviceToHost, c->stream));
             else
                 FE_CUDA(c, cudaMemcpy2DAsync(od[e], sizeof(float) * dim, c->b.fdesc + e * C * 128, sizeof(float) * 128,

@@ -91,6 +91,74 @@ __host__ __device__ inline float fast_atan2_deg(float y, float x) {
     return a;
 }
 
+// Exclusive prefix sum of v over a 1024-thread block; total = the block's sum.  s_warp: 33 words of shared memory.
+__device__ __forceinline__ uint32_t block_excl_scan_1024(uint32_t v, uint32_t *s_warp, uint32_t &total) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    uint32_t incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        uint32_t n = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += n;
+    }
+    if (lane == 31) s_warp[wid] = incl;
+    __syncthreads();
+    if (wid == 0) {
+        uint32_t w = s_warp[lane], wi = w;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            uint32_t n = __shfl_up_sync(0xffffffffu, wi, o);
+            if (lane >= o) wi += n;
+        }
+        s_warp[lane] = wi - w;            // exclusive warp bases
+        if (lane == 31) s_warp[32] = wi;  // grand total
+    }
+    __syncthreads();
+    const uint32_t r = s_warp[wid] + incl - v;
+    total = s_warp[32];
+    __syncthreads();
+    return r;
+}
+
+// ---- keypoints of an image tile (raster-ordered lists: kp_key = y << 16 | x ascending) --------------------------------
+// The per-tile kernels (orb_describe_tile_kernel, brief_tile_kernel) find the keypoints of their rows by binary search and
+// keep those of their columns by ballot compaction.
+
+// first index in [0, n) whose key is >= target (n if none): 32-way search, one key per lane per round
+__device__ __forceinline__ int warp_lower_bound(const uint32_t *__restrict__ keys, int n, uint32_t target, int lane) {
+    int lo = 0, hi = n;
+    while (lo < hi) {
+        const int step = (hi - lo + 31) >> 5, i = lo + lane * step;
+        const uint32_t m = __ballot_sync(0xffffffffu, i >= hi || keys[i] >= target);
+        const int f = m ? __ffs(m) - 1 : 32;          // keys[lo + (f - 1) step] < target <= keys[lo + f step]
+        if (f == 0) break;
+        hi = min(lo + f * step, hi);
+        lo += (f - 1) * step + 1;
+    }
+    return lo;
+}
+
+// Appends the indices and keys of the entries [base, min(base + CHUNK, hi)) whose x lies in [x0, x0 + cols) to s_idx / s_key
+// at *s_cnt, in any order (every result of the caller goes to its keypoint's own index).  All THREADS threads call it.
+template <int THREADS, int CHUNK>
+__device__ __forceinline__ void tile_collect(const uint32_t *keys, int base, int hi, int x0, int cols, uint32_t *s_idx,
+                                             uint32_t *s_key, int *s_cnt, int lane) {
+#pragma unroll
+    for (int q = 0; q < CHUNK / THREADS; ++q) {
+        const int i = base + q * THREADS + (int)threadIdx.x;
+        uint32_t key = 0;
+        bool in = false;
+        if (i < hi) {
+            key = keys[i];
+            in = (int)(key & 0xFFFF) >= x0 && (int)(key & 0xFFFF) < x0 + cols;
+        }
+        const uint32_t m = __ballot_sync(0xffffffffu, in);
+        int pos = 0;
+        if (lane == 0 && m) pos = atomicAdd(s_cnt, __popc(m));
+        pos = __shfl_sync(0xffffffffu, pos, 0) + __popc(m & ((1u << lane) - 1u));
+        if (in) { s_idx[pos] = (uint32_t)i; s_key[pos] = key; }
+    }
+}
+
 // Warp-cooperative exact FP32 squared L2 distance between a query held in registers (lane l owns dims
 // [D/32 * l, D/32 * (l + 1))) and a descriptor row in global memory: coalesced row load, per-lane FMA chain,
 // xor-butterfly sum -- a fixed, deterministic summation order; every lane returns the same value.
@@ -314,9 +382,16 @@ int launch_subpix(const Geom &g, const Buffers &b, const uint32_t *counts, const
 int launch_rbrief(const Geom &g, const DetectParams &p, const Buffers &b, const uint32_t *counts, cudaStream_t s);
 int launch_unpack_kps(const Geom &g, const Buffers &b, const uint32_t *counts, cudaStream_t s);
 // cv::BriefDescriptorExtractor(bytes) at the keypoints in b.kp with the caller's test table (brief.cu); needs b.integral.
-// out rows are 64 bytes apart (bytes used)
+// out rows are row_bytes apart (>= bytes; the rest of a row is zeroed)
 int launch_brief_ext(const Geom &g, const Buffers &b, const uint32_t *counts, const int8_t *pattern, int bytes, int use_orientation,
-                     uint8_t *out, cudaStream_t s);
+                     uint8_t *out, int row_bytes, cudaStream_t s);
+// The same rows from b.img per image tile, for the raster-ordered keypoints of one level (b.kp_key, b.n_kp) that all lie 28 px
+// inside the image (launch_brief_border first)
+int launch_brief_tile(const Geom &g, const Buffers &b, const int8_t *pattern, int bytes, int use_orientation, uint8_t *out,
+                      int row_bytes, cudaStream_t s);
+// BriefDescriptorExtractor::compute's runByImageBorder(28) on the detected keypoints: keeps them in order and compacts b.kp,
+// b.kp_key, b.kx, b.ky; b.n_kp becomes the kept count
+int launch_brief_border(const Geom &g, const Buffers &b, cudaStream_t s);
 
 // cv::FREAK at the keypoints in b.kp (freak.cu); needs b.integral and b.img.  table: [64][256][43] (x, y, sigma); opairs: [45]
 // (i, j, weight_dx, weight_dy); dpairs: [512] (i, j); scale_idx: [n_images][kp_cap].  Writes kp.angle and 64-byte rows.
@@ -453,9 +528,10 @@ struct MatchParams {
 double launch_popc_peak(int sms, int iters, uint32_t *sink, cudaStream_t s);
 int launch_hamming_cross(const Geom &g, int n_pairs, bool h2, const Buffers &b, const uint32_t *counts, cudaStream_t s);
 // cross-check + |dy| <= max_dy by band candidates + pruned verification (raster-ordered keypoints on both sides);
-// writes match_b / n_b itself (no separate finalize)
+// writes match_b / n_b itself (no separate finalize).  row_bytes: 32, or 16 for 128-bit rows zero-padded in the 256-bit rows
+// (the multi-index join then reads only their 8 data halves)
 // fused_ratio >= 0: mode A's Lowe-ratio finalize (b.best / b.second -> match_a / n_a) rides in the same finalize launch
-int launch_hamming_cross_pruned(const Geom &g, int n_pairs, float max_dy, bool have_band, bool use_join, const Buffers &b,
+int launch_hamming_cross_pruned(const Geom &g, int n_pairs, float max_dy, bool have_band, bool use_join, int row_bytes, const Buffers &b,
                                 const uint32_t *counts, double fused_ratio, cudaStream_t s, cudaStream_t aux = nullptr,
                                 cudaEvent_t ev_fork = nullptr, cudaEvent_t ev_join = nullptr);      // aux: side stream for the join
 // masked kNN-2; train_sorted = train keypoints are in raster order (enables the banded kernel)

@@ -532,32 +532,6 @@ int launch_hamming_knn2(const Geom &g, int n_pairs, const MatchParams &mp, bool 
 // ---- finalisation: Lowe ratio (mode A) and mutual check + |dy| filter (mode B) ----------------
 constexpr int FIN_THREADS = 1024;
 
-__device__ __forceinline__ uint32_t block_excl_scan_1024(uint32_t v, uint32_t *s_warp, uint32_t &total) {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    uint32_t incl = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        uint32_t n = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += n;
-    }
-    if (lane == 31) s_warp[wid] = incl;
-    __syncthreads();
-    if (wid == 0) {
-        uint32_t w = s_warp[lane], wi = w;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            uint32_t n = __shfl_up_sync(0xffffffffu, wi, o);
-            if (lane >= o) wi += n;
-        }
-        s_warp[lane] = wi - w;            // exclusive warp bases
-        if (lane == 31) s_warp[32] = wi;  // grand total
-    }
-    __syncthreads();
-    const uint32_t r = s_warp[wid] + incl - v;
-    total = s_warp[32];
-    __syncthreads();
-    return r;
-}
 
 // Mode A: accept a row with one candidate, or with d0 < ratio*d1 (double arithmetic, strict) --
 // StereoCamera.cpp:206-264, algorithm.py:838-846.  The C++ query-unique de-dup loop is a no-op
@@ -699,20 +673,22 @@ int launch_finalize_cross_both(const Geom &g, int n_pairs, const uint32_t *count
 // Results are identical to hamming_cross_kernel + finalize_cross_kernel (tests compare against cv2 and the oracle).
 //
 // Multi-index join (exact) for the bulk of the work.  Fifteen or fewer differing bits spread over the sixteen 16-bit halves
-// of a descriptor leave at least one half IDENTICAL (pigeonhole).  So an entry whose threshold is <= CX_T1 = 15 (class A,
-// ~92 %) can only be disturbed by a partner that shares a half with it:
+// of a descriptor leave at least one half IDENTICAL (pigeonhole).  So an entry whose threshold is <= 15 (class A, ~92 %) can
+// only be disturbed by a partner that shares a half with it:
 //   mih_transpose_kernel   halves of every entry in permutation order ([image][half position][k], coalesced for the join) and
 //                          the index of its own mutual candidate (already seeded, never re-measured);
 //   mih_join_kernel<0>     one CTA per (pair, half position): the class-A trains' halves go into a shared-memory hash table,
 //                          every class-A query looks up its own half and measures the few trains it finds -- chance
 //                          collisions, ~0.1 per probe, which leave after the distance.  (R = 1 also probes the 16 one-bit
 //                          neighbours -- valid up to 31 differing bits; measured slower than the LB scan for class B.)
-// The LB scan then only serves class B (CX_T1 < d* <= CX_T, ~5 %) against A + B, and class C (d* > CX_T, ~3 %) is evaluated
+// The LB scan then only serves class B (15 < d* <= CX_T, ~5 %) against A + B, and class C (d* > CX_T, ~3 %) is evaluated
 // in full against everything.  Without the join (per-image capacity above MIH_MAX) class A is empty and the LB scan serves
 // B x B as before.
+// 128-bit rows (BRIEF-16) ride zero-padded in the 256-bit rows: their halves 8 .. 15 are 0 for every entry, so a join at those
+// positions would put every class-A train into one probe run and measure every pair.  The join then covers the 8 data halves
+// only, and class A ends at 7 differing bits -- the pigeonhole of 8 halves.  The LB4 / LB8 scans stay valid on the zero words.
 constexpr int CX_T = 24;             // B / C split of the LB scan (the LB4 filter stops paying above it)
 constexpr int CX_T2 = 48;            // C / D split: the two-POPC LB8 filter serves thresholds up to here, class D is evaluated in full
-constexpr int CX_T1 = 15;            // A / B split: 16 halves, at most 15 differing bits -> one half is identical
 
 __global__ void __launch_bounds__(1024)
 cross_classify_kernel(Geom g, int t1, int t2, int t3, const uint32_t *__restrict__ counts, const uint32_t *__restrict__ bestL,
@@ -1057,7 +1033,7 @@ finalize_cand_and_ratio_kernel(Geom g, const uint32_t *__restrict__ counts, cons
 }
 
 // cross-check + |dy| <= max_dy for raster-ordered keypoints on both sides; writes match_b / n_b
-int launch_hamming_cross_pruned(const Geom &g, int n_pairs, float max_dy, bool have_band, bool use_join, const Buffers &b,
+int launch_hamming_cross_pruned(const Geom &g, int n_pairs, float max_dy, bool have_band, bool use_join, int row_bytes, const Buffers &b,
                                 const uint32_t *counts, double fused_ratio, cudaStream_t s, cudaStream_t aux, cudaEvent_t ev_fork,
                                 cudaEvent_t ev_join) {
     MatchParams mp{};
@@ -1070,12 +1046,14 @@ int launch_hamming_cross_pruned(const Geom &g, int n_pairs, float max_dy, bool h
             b.cx_bestL, b.cx_bestR, b.rowstart);
     }
     const bool mih = use_join && g.kp_cap <= MIH_MAX && b.cx_half;
+    // A / B split: the join's positions are the rows' 16-bit halves, and at most halves - 1 differing bits leave one identical
+    const int halves = row_bytes / 2, join_t1 = halves - 1;
     // without the join class A is empty (t1 = -2: even "no candidate" entries, d* = -1, fall into class B)
     static const int cx_t = getenv("FE_CX_T") ? atoi(getenv("FE_CX_T")) : CX_T;      // B / C split (tuning knob; any value is exact)
     static const int cx_t2 = std::max(cx_t, getenv("FE_CX_T2") ? atoi(getenv("FE_CX_T2")) : CX_T2);   // C / D split (likewise)
     static const bool wide_kill = !(getenv("FE_CX_WIDE") && atoi(getenv("FE_CX_WIDE")) == 0);        // A/B testing
     // the splits must not decrease: a B / C split below the A / B split would put an entry into class A and class D at once
-    const int t1 = mih ? CX_T1 : -2, t2 = std::max(cx_t, t1), t3 = std::max(cx_t2, t2);
+    const int t1 = mih ? join_t1 : -2, t2 = std::max(cx_t, t1), t3 = std::max(cx_t2, t2);
     cross_classify_kernel<<<dim3(n_pairs, 2), 1024, 0, s>>>(g, t1, t2, t3, counts, b.cx_bestL, b.cx_bestR,
                                                    have_band && wide_kill ? b.best : nullptr, b.allbest,
                                                    b.colbest, b.cx_thrq, b.cx_thrt, b.cx_qperm, b.cx_tperm, b.cx_n);
@@ -1095,7 +1073,7 @@ int launch_hamming_cross_pruned(const Geom &g, int n_pairs, float max_dy, bool h
             cudaFuncSetAttribute(mih_join_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         }
 #define FE_JOIN_ARGS b.cx_n, b.desc, b.cx_qperm, b.cx_tperm, b.cx_half, b.cx_star, b.allbest, b.colbest
-        mih_join_kernel<0><<<dim3(16, n_pairs), 1024, smem, js>>>(g, S, FE_JOIN_SPEC(1, 0, 1, 0, 1), CX_T1, FE_JOIN_ARGS);   // A trains | A queries
+        mih_join_kernel<0><<<dim3(halves, n_pairs), 1024, smem, js>>>(g, S, FE_JOIN_SPEC(1, 0, 1, 0, 1), join_t1, FE_JOIN_ARGS);   // A trains | A queries
         if (js != s) cudaEventRecord(ev_join, js);
 #undef FE_JOIN_ARGS
         n_launch += 3;

@@ -622,20 +622,6 @@ static_assert(DT_VECS * 16 <= DT_BLUR_B && DT_VECS * 4 <= DT_RAW_W && DT_BLUR_B 
 static_assert(DT_COLS + 2 * DT_XL - DT_XL >= DT_COLS + 21, "right halo reaches x + 20");
 static_assert(DT_RAW_W % 32 == 9 && (DT_BLUR_B / 4) % 32 == 20, "bank spread of the tile rows");
 
-// first index in [0, n) whose key is >= target (n if none): 32-way search, one key per lane per round
-__device__ __forceinline__ int warp_lower_bound(const uint32_t *__restrict__ keys, int n, uint32_t target, int lane) {
-    int lo = 0, hi = n;
-    while (lo < hi) {
-        const int step = (hi - lo + 31) >> 5, i = lo + lane * step;
-        const uint32_t m = __ballot_sync(0xffffffffu, i >= hi || keys[i] >= target);
-        const int f = m ? __ffs(m) - 1 : 32;          // keys[lo + (f - 1) step] < target <= keys[lo + f step]
-        if (f == 0) break;
-        hi = min(lo + f * step, hi);
-        lo += (f - 1) * step + 1;
-    }
-    return lo;
-}
-
 __global__ void __launch_bounds__(DT_THREADS, 2)
 orb_describe_tile_kernel(const uint8_t *__restrict__ img, const uint8_t *__restrict__ blur, Geom g,
                          const uint32_t *__restrict__ n_kp, const uint32_t *__restrict__ kp_key,
@@ -692,7 +678,9 @@ orb_describe_tile_kernel(const uint8_t *__restrict__ img, const uint8_t *__restr
     // shared-memory address of image pixel (0, 0) in the blurred tile's coordinates
     const uint32_t blur_o = (uint32_t)__cvta_generic_to_shared(s_blur) - (uint32_t)(ty0 * DT_BLUR_B + sx);
     for (int base = lo; base < hi; base += DT_CHUNK) {
-        // the band's keypoints whose x lies in the tile (any order: every result goes to its keypoint's own index)
+        // the band's keypoints whose x lies in the tile (any order: every result goes to its keypoint's own index).  This is
+        // tile_collect (fe_internal.cuh, which brief_tile_kernel calls) written out: through the helper this kernel compiles
+        // to 1960 instead of 1880 instructions, and c2 ran 41.40 k against 41.69 k pairs/s (profiles/r7_ab_brief.log)
 #pragma unroll
         for (int q = 0; q < DT_CHUNK / DT_THREADS; ++q) {
             const int i = base + q * DT_THREADS + (int)threadIdx.x;

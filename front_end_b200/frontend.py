@@ -14,6 +14,9 @@ from . import lib as L
 
 _lib = None
 _SURF_DIM = {L.DESC_SURF64: 64, L.DESC_SURF128: 128}       # float row width of the SURF descriptor kinds
+# (width, dtype) of one descriptor row on the host, per descriptor kind
+_ROW = {L.DESC_ORB256: (32, np.uint8), L.DESC_SURF64: (64, np.float32), L.DESC_SURF128: (128, np.float32),
+        L.DESC_BRIEF16: (16, np.uint8), L.DESC_BRIEF32: (32, np.uint8), L.DESC_BRIEF64: (64, np.uint8), L.DESC_FREAK: (64, np.uint8)}
 
 
 def get_lib():
@@ -155,9 +158,7 @@ class FrontEnd:
         img = _u8img(img)
         kps = np.ascontiguousarray(kps, dtype=L.KPOINT).copy()
         n = C.c_int32(len(kps))
-        width = {L.DESC_ORB256: (32, np.uint8), L.DESC_SURF64: (64, np.float32), L.DESC_SURF128: (128, np.float32),
-                 L.DESC_BRIEF16: (16, np.uint8), L.DESC_BRIEF32: (32, np.uint8), L.DESC_BRIEF64: (64, np.uint8),
-                 L.DESC_FREAK: (64, np.uint8)}[kind]
+        width = _ROW[kind]
         desc = np.zeros((max(len(kps), 1), width[0]), width[1])
         self._check(self.lib.fe_describe(self.h, _ptr(img), img.shape[1], img.shape[0], img.strides[0],
                                          _ptr(kps), C.byref(n), _ptr(desc), kind))
@@ -222,12 +223,14 @@ class FrontEnd:
 
     # -- getStereoFeatures --------------------------------------------------------------------------------
     def stereo_features(self, left, right, kind=L.DESC_ORB256, cap=None):
+        """getStereoFeatures: detect on both eyes and describe with kind (DESC_ORB256, DESC_SURF64 / 128, or DESC_BRIEF16 / 32 /
+        64 with the table of set_brief_pattern, after BRIEF's 28-px border).  Returns (l_kps, l_desc, r_kps, r_desc, proc)."""
         left, right = _u8img(left), _u8img(right)
         if left.shape != right.shape or left.strides != right.strides:
             raise ValueError("left/right geometry differs")
         cap = cap or self.max_keypoints
         lk, rk = np.zeros(cap, L.KPOINT), np.zeros(cap, L.KPOINT)
-        dw, dt = {L.DESC_ORB256: (32, np.uint8), L.DESC_SURF64: (64, np.float32), L.DESC_SURF128: (128, np.float32)}[kind]
+        dw, dt = _ROW[kind]
         ld, rd = np.zeros((cap, dw), dt), np.zeros((cap, dw), dt)
         nl, nr = C.c_int32(), C.c_int32()
         proc = (C.c_double * 4)()
@@ -289,11 +292,11 @@ class FrontEnd:
 
     def batch_landmarks(self, which=0, cap=None):
         """stereoLandmarks of every resident pair (algorithm.py:893-913): dict(l_kps, l_desc, r_kps, r_desc, matches, n).
-        Descriptor rows: (P, cap, 32) uint8 for ORB-256 batches, (P, cap, 64 / 128) float32 for SURF-64 / SURF-128."""
+        Descriptor rows: (P, cap, 32) uint8 for ORB-256 and BRIEF-32 batches, (P, cap, 16) uint8 for BRIEF-16, (P, cap, 64 / 128)
+        float32 for SURF-64 / SURF-128."""
         cap = cap or self.max_keypoints
         P = self._n_pairs
-        dim = _SURF_DIM.get(getattr(self, "_batch_kind", L.DESC_ORB256), 0)
-        dw, dt = (dim, np.float32) if dim else (32, np.uint8)
+        dw, dt = _ROW[getattr(self, "_batch_kind", L.DESC_ORB256)]
         out = dict(l_kps=np.zeros((P, cap), L.KPOINT), r_kps=np.zeros((P, cap), L.KPOINT),
                    l_desc=np.zeros((P, cap, dw), dt), r_desc=np.zeros((P, cap, dw), dt),
                    matches=np.zeros((P, cap), L.MATCH), n=np.zeros(P, np.int32))
@@ -306,7 +309,9 @@ class FrontEnd:
         self._check(self.lib.fe_set_chunk_pairs(self.h, pairs))
 
     def set_batch_descriptor(self, kind):
-        """Descriptor of the batched pipeline: DESC_ORB256 (default) or DESC_SURF64 / DESC_SURF128."""
+        """Descriptor of the batched pipeline: DESC_ORB256 (default), DESC_SURF64 / DESC_SURF128 (matched with NORM_L2), or
+        DESC_BRIEF16 / DESC_BRIEF32 (set_brief_pattern of that width first; the table and use_orientation current at batch_run /
+        pipeline_batch apply; keypoints nearer than 28 px to the border are removed after detection; NORM_HAMMING)."""
         self._check(self.lib.fe_set_batch_descriptor(self.h, kind))
         self._desc_kind = self._batch_kind = kind
 
@@ -363,8 +368,7 @@ class FrontEnd:
     def alloc_batch_outputs(self, n_pairs, pinned=False):
         cap = self.max_keypoints
         mk = self.pinned if pinned else (lambda shape, dt: np.zeros(shape, dt))
-        dw, dt = {L.DESC_ORB256: (32, np.uint8), L.DESC_SURF64: (64, np.float32),
-                  L.DESC_SURF128: (128, np.float32)}[getattr(self, "_batch_kind", L.DESC_ORB256)]
+        dw, dt = _ROW[getattr(self, "_batch_kind", L.DESC_ORB256)]
         return dict(kps=mk((2 * n_pairs, cap), L.KPOINT), desc=mk((2 * n_pairs, cap, dw), dt),
                     n_kps=mk((2 * n_pairs,), np.int32), matches_a=mk((n_pairs, cap), L.MATCH),
                     n_a=mk((n_pairs,), np.int32), matches_b=mk((n_pairs, cap), L.MATCH), n_b=mk((n_pairs,), np.int32))

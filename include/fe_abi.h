@@ -274,7 +274,12 @@ int32_t fe_window_match(fe_ctx *ctx, const fe_kpoint *cur_kps, const void *cur_d
 
 /* srv/getStereoFeatures.srv:1-6 (bin/feature_node:24-80): detect + describe left and right.
  * Outputs per eye: kps (cap records), desc (cap rows), count.  proc_seconds[4] = lkp, ld, rkp, rd
- * stage times (bin/feature_node:27-34,72-75), measured with CUDA events. */
+ * stage times (bin/feature_node:27-34,72-75), measured with CUDA events.
+ * desc_kind: FE_DESC_ORB256, FE_DESC_SURF64 / 128, or FE_DESC_BRIEF16 / 32 / 64 (the service's descriptor table,
+ * features.py:455-461): detector.detect, then BriefDescriptorExtractor::compute with the table of fe_set_brief_pattern --
+ * keypoints nearer than 28 px to the border (28 <= x < w - 28, 28 <= y < h - 28 kept, as floats) are removed after the
+ * detector's top-N / Harris cut, in order; records are the detector's; rows of 16 / 32 / 64 bytes, packed.
+ * FE_ERR_UNSUPPORTED without a table of that width, and for FE_DESC_FREAK. */
 int32_t fe_stereo_features(fe_ctx *ctx, const uint8_t *left, const uint8_t *right, int32_t width,
                            int32_t height, int32_t stride, int32_t desc_kind,
                            fe_kpoint *l_kps, void *l_desc, int32_t *nl,
@@ -283,9 +288,10 @@ int32_t fe_stereo_features(fe_ctx *ctx, const uint8_t *left, const uint8_t *righ
 
 /* ---- batched pipeline (frame-sharded hot path; SURVEY.md section 8e) ----------------------- */
 
-/* One call = detect + describe (ORB-256) + match for n_pairs independent rectified pairs.
+/* One call = detect + describe (the batch descriptor: ORB-256 by default) + match for n_pairs independent rectified pairs.
  * left/right: n_pairs contiguous images each (stride = width).  Outputs are fixed-capacity slabs:
- * kps[(2*p+eye)*kp_cap + i], desc[((2*p+eye)*kp_cap + i)*32], n_kps[2*p+eye];
+ * kps[(2*p+eye)*kp_cap + i], desc[((2*p+eye)*kp_cap + i)*row], n_kps[2*p+eye], row = the descriptor's bytes (32 for
+ * ORB-256 and BRIEF-32, 16 for BRIEF-16, 4 * 64 / 4 * 128 for SURF-64 / 128), rows packed like fe_describe's;
  * matches_a (mode A per cfg_a) / matches_b (mode B per cfg_b): [p*kp_cap + i], counts n_a[p], n_b[p].
  * Any output pointer may be NULL to skip its download (the work is still done on the device).
  * Host buffers should be pinned (fe_host_alloc) for full-speed async copies.  Batches of 96 pairs or
@@ -300,10 +306,20 @@ int32_t fe_pipeline_batch(fe_ctx *ctx, int32_t n_pairs, const uint8_t *left, con
 /* The same pipeline split in three so that a caller (bench.py) can keep inputs resident in HBM:
  * upload (H2D, async + sync), run (kernels only, asynchronous on the ctx stream unless sync != 0),
  * download (D2H + sync). */
-/* Selects the descriptor the batched pipeline computes: FE_DESC_ORB256 (default; Hamming matching) or
- * FE_DESC_SURF64 / FE_DESC_SURF128 (bin/detect_node:33-41; L2 matching, `desc` rows are floats).  Keypoints the
+/* Selects the descriptor the batched pipeline computes: FE_DESC_ORB256 (default; Hamming matching),
+ * FE_DESC_SURF64 / FE_DESC_SURF128 (bin/detect_node:33-41; L2 matching, `desc` rows are floats; keypoints the
  * SURF stage would drop (src/surf.cpp:953-978; cannot happen with edge_threshold >= 16) stay in place
- * with size = -1 in batch mode. */
+ * with size = -1 in batch mode), or FE_DESC_BRIEF16 / FE_DESC_BRIEF32 (cv::BriefDescriptorExtractor, the service's other
+ * descriptor; src/live_stereo.cpp:238,359-360 uses BRIEF-16):
+ *  - the run uses the test table and use_orientation that fe_set_brief_pattern holds for that width when fe_batch_run /
+ *    fe_pipeline_batch is called; FE_ERR_UNSUPPORTED here if no table of that width has been set;
+ *  - detection is the ORB-256 batch's (FAST or ORB mode, top-N, HARRIS_SCORE, pyramid); then, as compute() after detect(),
+ *    the keypoints nearer than 28 px to the border are removed, in order (n_kps = kept); records are the detector's;
+ *  - matched with FE_NORM_HAMMING / FE_NORM_HAMMING2 (FE_NORM_L2 is FE_ERR_UNSUPPORTED); every batched entry point takes
+ *    them (fe_batch_download, fe_pipeline_batch including its overlapped path, fe_batch_landmarks, fe_window_batch).
+ * FE_DESC_BRIEF64 and FE_DESC_FREAK return FE_ERR_UNSUPPORTED: their 512-bit rows are matched by the host entry points
+ * only (the batch's band and cross-check kernels read rows of at most 256 bits).  A ctx with the Fast-Hessian detector
+ * (fe_set_batch_detector) returns FE_ERR_UNSUPPORTED for every kind: it describes with SURF. */
 int32_t fe_set_batch_descriptor(fe_ctx *ctx, int32_t desc_kind);
 /* Selects the detector of the batched pipeline (fe_batch_run, fe_pipeline_batch, and through them fe_batch_landmarks /
  * fe_window_batch).  surf == NULL: FAST / ORB per fe_config and the fe_set_orb_* calls (the default, unchanged).
@@ -338,7 +354,7 @@ int32_t fe_set_batch_detector(fe_ctx *ctx, const fe_surf_params *surf);
  * n_tracks[f-1].  cfg: mode FE_MATCH_RATIO, mask FE_MASK_WINDOW -- or mode FE_MATCH_CROSSCHECK with FE_MASK_NONE for
  * liveGraph's tracker (src/front_end/algorithm.py:1160-1190: cross-check of the left AND of the right descriptors of
  * consecutive frames, intersected on the same previous landmark, no |dy| filter).  norm: FE_NORM_HAMMING / HAMMING2 on an
- * ORB-256 batch, FE_NORM_L2 on a SURF-64 / SURF-128 batch (fe_set_batch_descriptor; exact FP32 distances, the liveGraph
+ * ORB-256 or BRIEF-16 / 32 batch, FE_NORM_L2 on a SURF-64 / SURF-128 batch (fe_set_batch_descriptor; exact FP32 distances, the liveGraph
  * mode by two all-pairs passes); a norm that does not fit the batch's descriptor is FE_ERR_UNSUPPORTED.
  * Optional triangulation (:36-51): Q = 4x4 row-major reprojection matrix, xyz[(f*cap + i)*3 .. +3] =
  * (Q [xl, yl, xl - xr, 1]^T)_{0..2} / (1000 * (.)_3) for landmark i of frame f; pass NULL, NULL to skip. */
@@ -375,7 +391,7 @@ int32_t fe_set_orb_patch_size(fe_ctx *ctx, int32_t patch_size);
  * (src/front_end/algorithm.py:893-913) -- row i of the left / right keypoint and descriptor arrays are the two ends of
  * match i, and matches[i] = {i, i, 0, distance}.  which: 0 = the ratio matches (cfg_a), 1 = the cross-check matches.
  * Slabs of `cap` rows per pair; n[p] = landmarks of pair p.  Any output pointer may be NULL.  Descriptor rows per batch
- * descriptor: 32 u8 (ORB-256), 64 f32 (SURF-64), 128 f32 (SURF-128), packed (row p * cap + i). */
+ * descriptor: 32 u8 (ORB-256, BRIEF-32), 16 u8 (BRIEF-16), 64 f32 (SURF-64), 128 f32 (SURF-128), packed (row p * cap + i). */
 int32_t fe_batch_landmarks(fe_ctx *ctx, int32_t which, int32_t cap, fe_kpoint *l_kps, void *l_desc, fe_kpoint *r_kps,
                            void *r_desc, fe_match *matches, int32_t *n);
 
